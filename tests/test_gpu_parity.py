@@ -11,7 +11,7 @@ import pytest
 import sea_ice_drift_b200 as sid
 from sea_ice_drift_b200 import _lib, synthetic as syn, sharding
 from oracle import c_oracle as co
-from tests.helpers import variant_inputs, classify, make_exact_lookup, assert_parity
+from tests.helpers import variant_inputs, classify, make_exact_lookup, assert_parity, assert_equals_exact_oracle
 
 pytestmark = pytest.mark.gpu
 
@@ -21,17 +21,6 @@ VARIANTS = ["default", "one_angle", "rot_order1", "hes_smth", "raw_hes_mcc_norm"
 
 def flags(opts):
     return _lib.flags_from_kwargs(opts["hes_norm"], opts["hes_smth"], opts["mcc_norm"])
-
-
-def assert_equals_exact_oracle(got, ref, st_got=None, st_ref=None):
-    """GPU vs the exact CPU oracle: integers and r bit-exact, h to float32 rounding."""
-    assert np.array_equal(np.isnan(got), np.isnan(ref))
-    ok = ~np.isnan(ref[:, 0])
-    assert np.array_equal(got[ok, :3], ref[ok, :3]), "position / angle differ from the exact oracle"
-    assert np.array_equal(got[ok, 3], ref[ok, 3]), "r differs from the exact oracle"
-    assert np.all(np.abs(got[ok, 4] - ref[ok, 4]) <= 4e-6 * (1 + np.abs(ref[ok, 4])))
-    if st_got is not None:
-        assert np.array_equal(st_got, st_ref)
 
 
 @pytest.mark.parametrize("name", VARIANTS)
