@@ -245,6 +245,13 @@ size_t tail_split_limit() {
     return (size_t)52 * 1024;
 }
 
+// Words per work item of the tail hand-off regions of a two-class host call: the large class hands over float maps (when its
+// tail is split off), the small class is the one of pm_ws_kernel (three integer arrays per item)
+size_t tail_region_words(int rr_big, int rr_small, bool smth) {
+    const size_t big = pm_tail_smem_bytes(rr_big, smth) <= tail_split_limit() ? tail_item_words((rr_big + 3) & ~3, 0) : 0;
+    return std::max(big, tail_item_words((rr_small + 3) & ~3, 1));
+}
+
 int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1, const double *d_c2fg,
               const double *d_r2fg, const double *d_border, const int *d_order, int max_border, int typ_border,
               int img_size, int n_angles, const double *d_angles, const double *d_tab, int rot_order,
@@ -311,8 +318,9 @@ int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1,
         a.split_tail = 1;
         const size_t cap_n = (size_t)std::max<long long>(n + tail_off, ctx->tail_hint_n);
         a.tail_stride = (a.max_rr + 3) & ~3;
-        // regions of concurrently running launches (bands, border classes) are laid out with ONE stride per host call
-        const size_t region_stride = std::max(ctx->tail_region_stride, (size_t)a.tail_stride);
+        // regions of concurrently running launches (bands, border classes) are laid out with ONE stride per host call;
+        // a work item of this kernel hands over three integer arrays (PmTailRec::mode 1)
+        const size_t region_stride = std::max(ctx->tail_region_stride, tail_item_words(a.tail_stride, 1));
         if ((rc = reserve(ctx, ctx->tail_maps, cap_n * region_stride * sizeof(float)))) return rc;
         if ((rc = reserve(ctx, ctx->tail_recs, cap_n * sizeof(PmTailRec)))) return rc;
         a.tail_maps = (float *)ctx->tail_maps.p + (size_t)tail_off * region_stride;
@@ -1056,7 +1064,7 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
         auto rr_of = [&](int b) { const int R = 2 * (img_size / 2) + 2 * b + 1 - img_size + 1; return R * R; };
         const bool smth = (flags & SID_HES_SMTH) != 0;
         const int rr_big = rr_of(max_border), rr_small = rr_of(small_max);
-        ctx->tail_region_stride = (size_t)(((pm_tail_smem_bytes(rr_big, smth) <= tail_split_limit() ? rr_big : rr_small) + 3) & ~3);
+        ctx->tail_region_stride = tail_region_words(rr_big, rr_small, smth);
     }
     const bool two_streams = pair && nbands > 1;
     if (two_streams) {
@@ -1167,7 +1175,7 @@ int sid_run_device(sid_ctx *ctx, int64_t n, const double *d_c1, const double *d_
         if (n_small >= 256 && n_big > 0) {
             auto rr_of = [&](int b) { const int R = 2 * (img_size / 2) + 2 * b + 1 - img_size + 1; return R * R; };
             const bool smth = (flags & SID_HES_SMTH) != 0;
-            ctx->tail_region_stride = (size_t)(((pm_tail_smem_bytes(rr_of(max_border), smth) <= tail_split_limit() ? rr_of(max_border) : rr_of(limit)) + 3) & ~3);
+            ctx->tail_region_stride = tail_region_words(rr_of(max_border), rr_of(limit), smth);
             ctx->tail_hint_n = n;
             rc = launch_pm(ctx, n_big, d_c1, d_r1, d_c2fg, d_r2fg, d_border, d_big, max_border, max_border, img_size,
                            n_angles, d_angles, d_tab, rot_order, flags, d_out, d_status, nullptr, 0, 0);

@@ -299,6 +299,24 @@ __device__ __forceinline__ void ncc_finish4(const double (&num)[4], const double
         for (int c = 0; c < 4; ++c) v[c] = __double2float_rn(ncc_finish(num[c], t[c]));
     }
 }
+// four positions of one angle from their exact integers: numerator, window sum, window sum of squares (non-flat template)
+__device__ __forceinline__ void ncc_ints4(const int32_t (&corr)[4], const uint32_t (&wsum)[4], const uint32_t (&wsq)[4],
+                                          const TemplStats &st, double inv_area, float (&v)[4]) {
+    double num[4], tt[4];
+#pragma unroll
+    for (int c = 0; c < 4; ++c) {
+        num[c] = __dsub_rn((double)corr[c], __dmul_rn((double)wsum[c], st.mean));
+        tt[c] = __dmul_rn(window_den(wsum[c], wsq[c], inv_area), st.norm);
+    }
+    ncc_finish4(num, tt, v);
+}
+__device__ __forceinline__ float4 ncc_vec4(int4 c, uint4 ws, uint4 wq, const TemplStats &st, double inv_area) {
+    const int32_t cc[4] = {c.x, c.y, c.z, c.w};
+    const uint32_t s4[4] = {ws.x, ws.y, ws.z, ws.w}, q4[4] = {wq.x, wq.y, wq.z, wq.w};
+    float v[4];
+    ncc_ints4(cc, s4, q4, st, inv_area, v);
+    return make_float4(v[0], v[1], v[2], v[3]);
+}
 
 __device__ __noinline__ Ncc3 ncc_value_call3(int c0, int c1, int c2, uint32_t wsum, double wden,
                                              double m0, double n0, double m1, double n1, double m2, double n2) {

@@ -44,7 +44,12 @@ struct PmTailRec {
     int best_idx;      // flat index of the peak
     int best_a;        // index of the winning angle
     float best_r;      // peak value
+    int mode;          // 0: the work item's hand-off region holds the float map; 1 (pm_ws_kernel): the exact integers it is made
+                       //    of -- numerators of the winning angle | window sums | window sums of squares (tail_stride words each)
+    uint32_t tsum, tsq;   // mode 1: template sum / sum of squares of the winning angle
 };
+// words per work item of the hand-off region
+__host__ __device__ inline size_t tail_item_words(int tail_stride, int mode) { return (size_t)tail_stride * (mode ? 3 : 1); }
 
 struct PmArgs {
     const uint8_t *img1; int rows1, cols1; long long pitch1;
@@ -705,6 +710,7 @@ pm_points_kernel(const PmArgs a, const __grid_constant__ CUtensorMap tmap2) {
                 PmTailRec rec;
                 rec.pt = (int)pt; rec.RH = RH; rec.RW = RW; rec.H = H; rec.W = W;
                 rec.best_idx = best_idx; rec.best_a = S.best_a; rec.best_r = S.best_r;
+                rec.mode = 0; rec.tsum = 0u; rec.tsq = 0u;
                 a.tail_recs[pi] = rec;
             }
             continue;
@@ -746,9 +752,26 @@ __global__ void __launch_bounds__(PM_TAIL_MAX_THREADS) pm_tail_kernel(const PmAr
     float *hes = map + a.tail_stride;
     float *tmp_a = hes + a.tail_stride;                                // only with hes_smth
     float *tmp_b = tmp_a + a.tail_stride;
-    const float4 *src = reinterpret_cast<const float4 *>(a.tail_maps + (size_t)blockIdx.x * a.tail_stride);
-    // the producer wrote RR floats; the up to 3 floats behind them in the last vector are never used
-    for (int k = tid; k < (RR + 3) >> 2; k += nt) reinterpret_cast<float4 *>(map)[k] = src[k];
+    const float *item = a.tail_maps + (size_t)blockIdx.x * tail_item_words(a.tail_stride, rec.mode);
+    // the producer wrote RR values per array; the up to 3 values behind them in the last vector are never used
+    if (rec.mode == 0) {
+        const float4 *src = reinterpret_cast<const float4 *>(item);
+        for (int k = tid; k < (RR + 3) >> 2; k += nt) reinterpret_cast<float4 *>(map)[k] = src[k];
+    } else {
+        // the winning map from its exact integers, with the normalisation of every other path (pm_ws_kernel evaluated only
+        // the positions that could hold the peak)
+        const int4 *srcC = reinterpret_cast<const int4 *>(item);
+        const uint4 *srcS = reinterpret_cast<const uint4 *>(item + a.tail_stride);
+        const uint4 *srcQ = reinterpret_cast<const uint4 *>(item + 2 * a.tail_stride);
+        const TemplStats st = templ_stats(rec.tsum, rec.tsq, a.inv_area, a.sqrt_inv_area);
+        for (int k = tid; k < (RR + 3) >> 2; k += nt) {
+            const int4 c = srcC[k];
+            const uint4 ws = srcS[k], wq = srcQ[k];
+            float4 v = make_float4(1.0f, 1.0f, 1.0f, 1.0f);
+            if (!st.flat) v = ncc_vec4(c, ws, wq, st, a.inv_area);
+            reinterpret_cast<float4 *>(map)[k] = v;
+        }
+    }
     __syncthreads();
     // hes_norm-only maps take peak_statistics' three-sweep fast path (sid_common.cuh) on the 2048-word histogram
     const PeakStats ps = peak_statistics(map, rec.RH, rec.RW, rec.best_idx, rec.best_r, a.flags, a.gw, tmp_a, tmp_b, hes, bs, wide_hist);

@@ -788,6 +788,7 @@ pm_tc_kernel(const PmArgs a, const PmTcCfg g, const __grid_constant__ CUtensorMa
                 PmTailRec rec;
                 rec.pt = (int)pt; rec.RH = RH; rec.RW = RW; rec.H = H; rec.W = W;
                 rec.best_idx = best_idx; rec.best_a = S.best_a; rec.best_r = S.best_r;
+                rec.mode = 0; rec.tsum = 0u; rec.tsq = 0u;
                 a.tail_recs[pi] = rec;
             }
             continue;

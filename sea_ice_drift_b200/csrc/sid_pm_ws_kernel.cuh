@@ -9,10 +9,11 @@
 //                      then the Toeplitz EXPANSION of every pair of template rows into a ring of A-operand slots
 //   mma     (4 warps)  one issuing thread each (one x block of 16 result columns each): tcgen05.mma kind::i8,
 //                      A and B both from shared memory, accumulators in tensor memory (2 sets of 256 columns)
-//   stats   (4 warps)  window sums / sums of squares (sliding, exact integers), FP64 denominators
-//   epilogue(2 x 4 warps, alternate points)  tcgen05.ld, combine the two row parities, approximate float screening
-//                      of the angles, OpenCV's exact FP64 normalisation of the winning angle only, argmax, hand-off of
-//                      the winning map to pm_tail_kernel
+//   stats   (7 warps)  window sums / sums of squares (sliding, exact integers), also written to the tail hand-off
+//   epilogue(2 x 4 warps, alternate points)  tcgen05.ld, combine the two row parities, FP32 screening of the angles
+//                      from the exact integers, OpenCV's exact FP64 normalisation of the positions that can still hold
+//                      the peak, argmax, hand-off of the winning angle's numerators to pm_tail_kernel (which rebuilds
+//                      the float map from them)
 //
 // Formulation.  With x' = x + (x0 & 15) = 16 xq + dx (the window is staged from a 16-byte aligned column):
 //
@@ -27,10 +28,11 @@
 // 2 loads, 3 byte permutes, 16 word stores), instead of one Toeplitz row per result column.  Per point and angle
 // batch this is ~1.5 k warp instructions against ~16 k for the row loop of pm_tc_kernel.
 //
-// The exact FP64 normalisation (the most expensive per-output step) runs for the winning angle only: every angle is
-// first screened with a float approximation whose error (< 5e-7) is far below the margin (4e-6) used to decide which
-// angles can still win; angles inside the margin are all evaluated exactly, so the result is the same bit pattern the
-// other kernels produce (strict '>' over angles, np.argmax inside a map).
+// The exact FP64 normalisation (the most expensive per-output step) runs only where the peak can be: every position of
+// every angle is first screened with an FP32 estimate whose error (< 1e-6, bound at WS_MARGIN) is far below the margin
+// (4e-6); the positions whose estimate is within the margin of the best lower bound, and those the estimate cannot
+// judge, are evaluated exactly, so the result is the same bit pattern the other kernels produce (strict '>' over angles,
+// np.argmax inside a map).  The tail kernel rebuilds the whole winning map for the peak statistics.
 #pragma once
 #include "sid_pm_tc_kernel.cuh"
 
@@ -46,7 +48,19 @@ constexpr int WS_NWIN = 2;                // window ring (each slot: the search 
 constexpr int WS_NENT = 8;                // point entries / template records
 constexpr int WS_MAX_SLOTS = 8;
 constexpr int WS_ACC_COLS = 256;          // tensor-memory columns per accumulator set (4 x blocks x 64)
-constexpr float WS_MARGIN = 4e-6f;
+// Screening estimate of a non-special position (window variance v = N wsq - wsum^2 > N, template variance
+// tv = N tsq - tsum^2 > 0, numerator n = N corr - wsum tsum; all exact in int64, N = s^2):
+//     e = f32(n) * rsqrt.approx(f32(v)) * f32(1 / sqrt(tv))          (the real value is r = n / sqrt(v tv), |r| <= 1)
+// Its relative error is at most 2^-24 (f32(n)) + 2^-25 (f32(v) under the root) + 2^-22 (rsqrt.approx, 2 ulp)
+// + 2^-24 (the per-angle factor) + 2 * 2^-24 (two products) < 5.3e-7.  OpenCV's FP64 value differs from r by < 2e-7: v > N
+// and tv >= N - 1 keep its denominator >= ~1 and window_den's argument >= 1, where the FP64 rounding of the numerator
+// (< 4e-8 absolute) and of the denominator (< 6e-8 relative) stay tiny, plus 2^-25 for its float rounding.  So
+// |e - exact| < ERR = 1e-6, and every position whose exact value can reach the peak has e >= (largest usable e) - 2 ERR.
+// Positions with v <= N (window_den's 10 FLT_EPSILON threshold can apply: the exact value may be 0) or |e| >= WS_NEAR1
+// (OpenCV's +-1 / 0 cases) are not estimated: they always go to the exact evaluation.
+constexpr float WS_MARGIN = 4e-6f;        // >= 2 ERR
+constexpr float WS_NEAR1 = 0.99f;
+constexpr int WS_LIST = 256;              // positions evaluated exactly per epilogue group and batch (more: full exact pass)
 
 // optional role profile (-DSID_WS_PROF): cycles per bucket, written to a.scratch as long long [cta][6 roles][8]
 #ifdef SID_WS_PROF
@@ -83,7 +97,7 @@ struct PmWsCfg {
     int pbw, pbh;     // template patch of image 1 (TMA box, bytes x rows): every sample of every angle lies inside
     int prad;         // its half size: ceil(0.7072 s + 3)
     int patch_bytes;
-    int off_a, off_tpl, tpl_buf_words, off_stat, stat_bytes, off_hs, off_c, smem_bytes;
+    int off_a, off_tpl, tpl_buf_words, off_stat, stat_bytes, off_hs, off_c, off_emax, off_list, smem_bytes;
 };
 
 inline bool pm_ws_geometry(int s, int Rmax, int Wmax, int n_angles, int max_rr, PmWsCfg &g, int Rtyp = 0, int nstat = WS_NSTAT) {
@@ -138,13 +152,15 @@ inline bool pm_ws_geometry(int s, int Rmax, int Wmax, int n_angles, int max_rr, 
     g.off_tpl = (int)off; off += (size_t)2 * g.tpl_buf_words * 4;
     off = (off + 127) & ~(size_t)127;
     g.off_stat = (int)off;
-    g.stat_bytes = (max_rr * 12 + 127) & ~127;           // wden f64 (its low words first hold the u32 sums of squares) | wsum u32
+    g.stat_bytes = (max_rr * 8 + 127) & ~127;            // wsq u32 | wsum u32
     g.nstat = nstat < 2 ? 2 : (nstat > WS_NSTAT ? WS_NSTAT : nstat);
     off += (size_t)g.nstat * g.stat_bytes;
     g.hs_words = Rmax * g.hp;
     g.off_hs = (int)off; off += (size_t)g.hs_words * 6;       // hq u32 | hs u16
     off = (off + 127) & ~(size_t)127;
     g.off_c = (int)off; off += (size_t)2 * g.nab * g.cpl * 4;
+    g.off_emax = (int)off; off += (size_t)2 * max_rr * 4;     // per epilogue group: largest estimate over the angles per position
+    g.off_list = (int)off; off += (size_t)2 * WS_LIST * 4;
     g.smem_bytes = (int)((off + 127) & ~(size_t)127);
     return true;
 }
@@ -158,7 +174,7 @@ struct WsBars {
     unsigned long long tpl_full[WS_NENT];
     unsigned long long stats_full[WS_NSTAT], stats_empty[WS_NSTAT];
 };
-struct WsEpi { TemplStats st[3]; float m[4][3]; unsigned long long key[4]; };
+struct WsEpi { TemplStats st[3]; float m[4]; unsigned long long key[4][3]; unsigned cnt; };
 
 // try_wait spin with a watchdog: a protocol error becomes a trap (launch failure), never a hung GPU
 #ifdef SID_WS_DEBUG
@@ -226,33 +242,58 @@ __device__ __forceinline__ void tc_ld16(uint32_t taddr, uint32_t (&v)[16]) {
                  : "r"(taddr));
 }
 
-// exact normalisation of one angle (OpenCV's formula, bit for bit the other kernels' epilogue); optional map store
+// exact normalisation of one angle with a non-flat template (OpenCV's formula, bit for bit the other kernels' epilogue):
+// this thread's part of the argmax key.  Only where the contender list overflows (flat or degenerate content).
 __device__ __forceinline__ unsigned long long ws_exact_pass(const int32_t *__restrict__ Ca, const uint32_t *__restrict__ wsum,
-                                                            const double *__restrict__ wden, const TemplStats st, int RR, int et,
-                                                            float *__restrict__ dst) {
+                                                            const uint32_t *__restrict__ wsq, const TemplStats st, double inv_area,
+                                                            int RR, int et) {
     float bv = -INFINITY;
     int bidx = -1;
     for (int base = 0; base < RR; base += 512) {
-        double num[4], tt[4];
+        int32_t cc[4];
+        uint32_t s4[4], q4[4];
         float v[4];
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
             const int idx = min(base + 128 * c + et, RR - 1);
-            num[c] = __dsub_rn((double)Ca[idx], __dmul_rn((double)wsum[idx], st.mean));
-            tt[c] = __dmul_rn(wden[idx], st.norm);
+            cc[c] = Ca[idx]; s4[c] = wsum[idx]; q4[c] = wsq[idx];
         }
-        ncc_finish4(num, tt, v);
+        ncc_ints4(cc, s4, q4, st, inv_area, v);
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
             const int idx = base + 128 * c + et;
-            if (idx < RR) {
-                const float vv = st.flat ? 1.0f : v[c];
-                if (dst) dst[idx] = vv;
-                if (vv > bv) { bv = vv; bidx = idx; }
-            }
+            if (idx < RR && v[c] > bv) { bv = v[c]; bidx = idx; }
         }
     }
     return bidx >= 0 ? peak_key(bv, (uint32_t)bidx) : 0ull;
+}
+
+// Screening sweep of one epilogue thread over the positions idx = et + 128 j of a batch of NB angles: stores per position the
+// largest estimate over the angles, +inf where one of them cannot be estimated (flat window, |e| >= WS_NEAR1), and returns
+// the largest estimate of the positions whose estimates are all usable (each is within ERR of an exact value).
+template <int NB>
+__device__ __forceinline__ float ws_screen(const int32_t *__restrict__ C, int cpl, const uint32_t *__restrict__ wsum,
+                                           const uint32_t *__restrict__ wsq, float *__restrict__ emax, int RR, int et, unsigned N,
+                                           const int (&tsm)[3], const float (&tinv)[3]) {
+    float mx = -INFINITY;
+#pragma unroll 2
+    for (int idx = et; idx < RR; idx += 128) {
+        const uint32_t ws = wsum[idx], wq = wsq[idx];
+        const unsigned long long v = (unsigned long long)N * wq - (unsigned long long)ws * ws;     // >= 0 (Cauchy-Schwarz)
+        float rv;
+        asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(rv) : "f"((float)v));
+        float hi = -INFINITY, lo = INFINITY;
+#pragma unroll
+        for (int k = 0; k < NB; ++k) {
+            const long long n = (long long)(int)N * (long long)C[k * cpl + idx] - (long long)(int)ws * (long long)tsm[k];
+            const float e = (float)n * rv * tinv[k];
+            hi = fmaxf(hi, e); lo = fminf(lo, e);
+        }
+        const bool judged = v > (unsigned long long)N && hi < WS_NEAR1 && lo > -WS_NEAR1;
+        emax[idx] = judged ? hi : INFINITY;
+        mx = fmaxf(mx, judged ? hi : -INFINITY);
+    }
+    return mx;
 }
 
 __global__ void __launch_bounds__(WS_THREADS, 1)
@@ -670,11 +711,14 @@ pm_ws_kernel(const PmArgs a, const PmWsCfg g, const __grid_constant__ CUtensorMa
             if (e.done) break;
             const int W = e.W, H = e.H, xoff = e.x0 & 15;
             const int RH = H - s + 1, RW = W - s + 1;
+            // the window sums also go to the work item's hand-off region, for pm_tail_kernel
+            uint32_t *gsum = reinterpret_cast<uint32_t *>(a.tail_maps) + (size_t)e.pi * tail_item_words(a.tail_stride, 1) + a.tail_stride;
+            uint32_t *gsq = gsum + a.tail_stride;
             const unsigned set = P % (unsigned)g.nstat;
             if (P >= (unsigned)g.nstat) ws_wait<200u>(BAR(&B.stats_empty[set]), ((P / (unsigned)g.nstat) - 1u) & 1u, __LINE__);
             WSP(2)
-            double *wden = reinterpret_cast<double *>(ws_smem + g.off_stat + (size_t)set * g.stat_bytes);
-            uint32_t *wsum = reinterpret_cast<uint32_t *>(wden + a.max_rr);
+            uint32_t *wsq = reinterpret_cast<uint32_t *>(ws_smem + g.off_stat + (size_t)set * g.stat_bytes);
+            uint32_t *wsum = wsq + a.max_rr;
             const uint8_t *win = sWin + (size_t)ws * g.win_bytes;
             // horizontal sliding sums: one (window row, x segment) per thread
             {
@@ -742,7 +786,6 @@ pm_ws_kernel(const PmArgs a, const PmWsCfg g, const __grid_constant__ CUtensorMa
             WSP(4)
             if (lane == 0) ws_arrive(BAR(&B.win_empty[ws]));        // this warp is done with the window
             // vertical sliding sums -> window sum / sum of squares per displacement
-            uint32_t *wsq2 = reinterpret_cast<uint32_t *>(wden);       // sums of squares in the low word of each wden slot (overwritten in place)
             {
                 int nseg = WS_NST / RW;
                 if (nseg < 1) nseg = 1;
@@ -756,39 +799,18 @@ pm_ws_kernel(const PmArgs a, const PmWsCfg g, const __grid_constant__ CUtensorMa
                     uint32_t sum = 0, sq = 0;
                     for (int i = 0; i < s; ++i) { sum += hs[ys + i]; sq += hq[ys + i]; }
                     for (int y = ys; y < ye; ++y) {
-                        wsum[y * RW + x] = sum;
-                        wsq2[2 * (y * RW + x)] = sq;
+                        const int idx = y * RW + x;
+                        wsum[idx] = sum; wsq[idx] = sq;
+                        gsum[idx] = sum; gsq[idx] = sq;
                         if (y + 1 < ye) { sum += (uint32_t)hs[y + s] - (uint32_t)hs[y]; sq += hq[y + s] - hq[y]; }
                     }
                 }
             }
             WSP(5)
-            ws_bar(2, WS_NST);                                          // hsT / hqT are free again; sums visible to the group
-            WSP(4)
-            // denominators: four independent FP64 chains per thread
-            {
-                const int RR = RH * RW;
-                for (int base = 0; base < RR; base += 4 * WS_NST) {
-                    double d[4];
-#pragma unroll
-                    for (int c = 0; c < 4; ++c) {
-                        // past the end: zeros, not a clamped index -- another thread may already have overwritten that slot's
-                        // sum of squares with its denominator (the value would be unused, but it is a read-write race)
-                        const int idx = base + WS_NST * c + st_;
-                        uint32_t vs = 0u, vq = 0u;
-                        if (idx < RR) { vs = wsum[idx]; vq = wsq2[2 * idx]; }
-                        d[c] = window_den(vs, vq, a.inv_area);
-                    }
-#pragma unroll
-                    for (int c = 0; c < 4; ++c) {
-                        const int idx = base + WS_NST * c + st_;
-                        if (idx < RR) wden[idx] = d[c];
-                    }
-                }
-            }
-            WSP(6)
             __syncwarp();
             if (lane == 0) ws_arrive(BAR(&B.stats_full[set]));
+            ws_bar(2, WS_NST);                                          // hsT / hqT are free again
+            WSP(4)
             ++P;
         }
         if (st_ == 0) WSP_OUT(3)
@@ -803,17 +825,21 @@ pm_ws_kernel(const PmArgs a, const PmWsCfg g, const __grid_constant__ CUtensorMa
         int32_t *C = reinterpret_cast<int32_t *>(ws_smem + g.off_c) + (size_t)eg * nab * g.cpl;
         const uint32_t lane_base = (uint32_t)(quarter * 32) << 16;
         const int dx = 4 * quarter + (lane >> 3), aa = (lane >> 1) & 3, ip = lane & 1;
-        const long long Nll = (long long)s * (long long)s;
+        const int Ni = s * s;
+        const long long Nll = (long long)Ni;
+        uint32_t *list = reinterpret_cast<uint32_t *>(ws_smem + g.off_list) + eg * WS_LIST;
+        float *emax = reinterpret_cast<float *>(ws_smem + g.off_emax) + (size_t)eg * a.max_rr;
         unsigned acc_use = 0;
         bool leave = false;
         WSP_DECL
         for (unsigned n = 0; !leave; ++n) {
             const unsigned P = (unsigned)eg + 2u * n;
             const unsigned sset = P % (unsigned)g.nstat;
-            const double *wden = reinterpret_cast<const double *>(ws_smem + g.off_stat + (size_t)sset * g.stat_bytes);
-            const uint32_t *wsum = reinterpret_cast<const uint32_t *>(wden + a.max_rr);
+            const uint32_t *wsq = reinterpret_cast<const uint32_t *>(ws_smem + g.off_stat + (size_t)sset * g.stat_bytes);
+            const uint32_t *wsum = wsq + a.max_rr;
             float best_r = -INFINITY;
             int best_a = -1, best_idx = 0;
+            uint32_t best_tsum = 0u, best_tsq = 0u;
             bool invalid = false;
             long long pt = 0, pi = 0;
             int W = 0, H = 0, xoff = 0, RH = 0, RW = 0, RR = 0;
@@ -872,96 +898,93 @@ pm_ws_kernel(const PmArgs a, const PmWsCfg g, const __grid_constant__ CUtensorMa
                 WSP(4)
                 if (invalid) continue;
 
-                // ---- float screening: an estimate (error < 5e-7) of every angle's maximum.  Per angle the loop keeps
-                //      max(n64 / wden) (n64 = N corr - wsum tsum, exact); the positive factor 1 / (N templNorm) comes after.
-                //      A value beyond ~0.99 in those units may be one of OpenCV's special cases (+-1 / 0): "can be 1".
-                float m[3] = {-INFINITY, -INFINITY, -INFINITY};
-                {
-                    double mean[3];
-                    float lim2[3];
-#pragma unroll
-                    for (int k = 0; k < 3; ++k) {
-                        const int kk = k < nb ? k : 0;
-                        mean[k] = (double)tr.tsum[kk] * a.inv_area;
-                        const double var = (double)tr.tsq[kk] * a.inv_area - mean[k] * mean[k];
-                        lim2[k] = (float)(0.98 * var * (double)Nll);
-                    }
-                    if (A_ == 1) m[0] = INFINITY;                                  // a single angle: nothing to screen
-                    else
-                    for (int base = 0; base < RR; base += 256) {
-#pragma unroll
-                        for (int c = 0; c < 2; ++c) {
-                            const int idx = min(base + 128 * c + et, RR - 1);      // the tail repeats the last element
-                            const double wsd = (double)wsum[idx];
-                            const float wd = (float)wden[idx];
-                            float iv;
-                            asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(iv) : "f"(wd));
-                            if (!(wd > 0.0f)) iv = 0.0f;                             // flat window: the exact value is 0
-#pragma unroll
-                            for (int k = 0; k < 3; ++k) {
-                                if (k < nb) {
-                                    const float qv = (float)fma(-wsd, mean[k], (double)C[k * g.cpl + idx]) * iv;
-                                    m[k] = fmaxf(m[k], qv * qv < lim2[k] ? qv : INFINITY);
-                                }
-                            }
-                        }
-                    }
-                }
+                // ---- screening from the exact integers (the estimate and its error bound: WS_MARGIN above)
+                float tinv[3];
+                int tsm[3];
+                unsigned flat = 0u;
 #pragma unroll
                 for (int k = 0; k < 3; ++k) {
-                    float v = m[k];
-#pragma unroll
-                    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-                    if (lane == 0) E.m[ew][k] = v;
+                    const int kk = k < nb ? k : 0;
+                    tsm[k] = (int)tr.tsum[kk];
+                    const long long tv = Nll * (long long)tr.tsq[kk] - (long long)tsm[k] * (long long)tsm[k];
+                    tinv[k] = tv > 0 ? (float)(1.0 / sqrt((double)tv)) : 0.0f;
+                    if (k < nb && E.st[k].flat) flat |= 1u << k;
                 }
+                float mx = nb == 3 ? ws_screen<3>(C, g.cpl, wsum, wsq, emax, RR, et, (unsigned)Ni, tsm, tinv)
+                         : nb == 2 ? ws_screen<2>(C, g.cpl, wsum, wsq, emax, RR, et, (unsigned)Ni, tsm, tinv)
+                                   : ws_screen<1>(C, g.cpl, wsum, wsq, emax, RR, et, (unsigned)Ni, tsm, tinv);
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+                if (lane == 0) E.m[ew] = mx;
+                if (et == 0) E.cnt = 0u;
                 WSP(5)
                 ws_bar(barid, 128);
                 WSP(4)
-                float M[3], Mx = -INFINITY;                               // ---- contenders (within the margin of the best estimate) -> exact normalisation, argmax, hand-off
+                // ---- contenders.  The peak of the batch is >= the best lower bound (largest usable estimate - ERR, or 1 for a
+                //      flat template, whose map is 1 everywhere); a position can hold it only if an estimate there is >= that
+                //      - ERR, or if one cannot be estimated.  Those positions are evaluated exactly, for every angle.
+                float Mx = fmaxf(fmaxf(E.m[0], E.m[1]), fmaxf(E.m[2], E.m[3]));
+                if (flat) Mx = fmaxf(Mx, 1.0f);
+                const float thr = fmaxf(Mx, best_r) - WS_MARGIN;
+                for (int idx = et; idx < RR; idx += 128) {
+                    if (emax[idx] >= thr) {
+                        const unsigned slot = atomicAdd(&E.cnt, 1u);
+                        if (slot < (unsigned)WS_LIST) list[slot] = (unsigned)idx;
+                    }
+                }
+                ws_bar(barid, 128);
+                unsigned long long key[3] = {0ull, 0ull, 0ull};
+                const unsigned cnt = E.cnt;
+                if (cnt <= (unsigned)WS_LIST) {
+                    for (unsigned t = (unsigned)et; t < cnt * (unsigned)nb; t += 128u) {
+                        const unsigned i = t / (unsigned)nb;
+                        const int k = (int)(t - i * (unsigned)nb), idx = (int)list[i];
+                        const TemplStats &sk = E.st[k];
+                        const uint32_t ws = wsum[idx];
+                        const double num = __dsub_rn((double)C[k * g.cpl + idx], __dmul_rn((double)ws, sk.mean));
+                        const double tt = __dmul_rn(window_den(ws, wsq[idx], a.inv_area), sk.norm);
+                        const unsigned long long kv = peak_key(__double2float_rn(ncc_finish(num, tt)), (uint32_t)idx);
+#pragma unroll
+                        for (int kk = 0; kk < 3; ++kk) if (kk == k && kv > key[kk]) key[kk] = kv;
+                    }
+                } else {
+                    // flat or degenerate content: too many positions the estimates cannot separate -- every angle in full
+                    for (int k = 0; k < nb; ++k)
+                        if (!((flat >> k) & 1u)) {
+                            const unsigned long long kv = ws_exact_pass(C + k * g.cpl, wsum, wsq, E.st[k], a.inv_area, RR, et);
+#pragma unroll
+                            for (int kk = 0; kk < 3; ++kk) if (kk == k) key[kk] = kv;
+                        }
+                }
 #pragma unroll
                 for (int k = 0; k < 3; ++k) {
-                    const float sc = (k < nb && !E.st[k].flat) ? (float)(1.0 / E.st[k].norm) : 0.0f;
-                    float v = fmaxf(fmaxf(E.m[0][k], E.m[1][k]), fmaxf(E.m[2][k], E.m[3][k])) * sc;
-                    if (!(v < 0.99999f)) v = 1.0f;
-                    if (k < nb && E.st[k].flat) v = 1.0f;
-                    M[k] = k < nb ? v : -INFINITY;
-                    Mx = fmaxf(Mx, M[k]);
+                    key[k] = warp_max_u64(key[k]);
+                    if (lane == 0) E.key[ew][k] = key[k];
                 }
-                const float thr = fmaxf(Mx, best_r) - WS_MARGIN;
-                int ncont = 0, first = -1;
+                ws_bar(barid, 128);
+                int pending = -1;
 #pragma unroll
-                for (int k = 0; k < 3; ++k) if (k < nb && M[k] >= thr) { ++ncont; if (first < 0) first = k; }
-                float *dst = a.tail_maps + (size_t)pi * a.tail_stride;
-                // group-wide maximum of a key (all threads return the same value)
-                auto group_max = [&](unsigned long long key) -> unsigned long long {
-                    key = warp_max_u64(key);
-                    ws_bar(barid, 128);                      // E.key free (previous readers done)
-                    if (lane == 0) E.key[ew] = key;
-                    ws_bar(barid, 128);
-                    unsigned long long k0 = E.key[0], k1 = E.key[1], k2 = E.key[2], k3 = E.key[3];
+                for (int k = 0; k < 3; ++k) {
+                    unsigned long long k0 = E.key[0][k], k1 = E.key[1][k], k2 = E.key[2][k], k3 = E.key[3][k];
                     k0 = k0 > k1 ? k0 : k1; k2 = k2 > k3 ? k2 : k3;
-                    return k0 > k2 ? k0 : k2;
-                };
-                if (ncont == 1 && M[first] > best_r + WS_MARGIN) {
-                    const unsigned long long key = group_max(ws_exact_pass(C + first * g.cpl, wsum, wden, E.st[first], RR, et, dst));
-                    best_r = key_f32((uint32_t)(key >> 32));
-                    best_idx = (int)(0xffffffffu - (uint32_t)(key & 0xffffffffull));
-                    best_a = a0 + first;
-                } else {
-                    int pending = -1;
-                    for (int k = 0; k < nb; ++k) {
-                        if (!(M[k] >= thr)) continue;
-                        const unsigned long long key = group_max(ws_exact_pass(C + k * g.cpl, wsum, wden, E.st[k], RR, et, nullptr));
-                        const float v = key_f32((uint32_t)(key >> 32));
-                        if (v > best_r) {
-                            best_r = v; best_idx = (int)(0xffffffffu - (uint32_t)(key & 0xffffffffull));
-                            best_a = a0 + k; pending = k;
-                        }
+                    unsigned long long kv = k0 > k2 ? k0 : k2;
+                    if ((flat >> k) & 1u) kv = peak_key(1.0f, 0u);
+                    if (kv == 0ull) continue;                   // no position of this angle listed
+                    const float v = key_f32((uint32_t)(kv >> 32));
+                    if (v > best_r) {
+                        best_r = v; best_idx = (int)(0xffffffffu - (uint32_t)(kv & 0xffffffffull));
+                        best_a = a0 + k; pending = k;
                     }
-                    if (pending >= 0) (void)ws_exact_pass(C + pending * g.cpl, wsum, wden, E.st[pending], RR, et, dst);
+                }
+                if (pending >= 0) {
+                    // hand-off: the winning angle's numerators (pm_tail_kernel rebuilds its float map)
+                    int32_t *gc = reinterpret_cast<int32_t *>(a.tail_maps) + (size_t)pi * tail_item_words(a.tail_stride, 1);
+                    const int32_t *cs = C + pending * g.cpl;
+                    for (int idx = et; idx < RR; idx += 128) gc[idx] = cs[idx];
+                    best_tsum = tr.tsum[pending]; best_tsq = tr.tsq[pending];
                 }
                 WSP(6)
-                ws_bar(barid, 128);          // C and E.st are free for the next batch
+                ws_bar(barid, 128);          // C, E.st, E.key, the estimates and the list are free for the next batch
                 WSP(4)
             }
             if (leave) {
@@ -980,6 +1003,7 @@ pm_ws_kernel(const PmArgs a, const PmWsCfg g, const __grid_constant__ CUtensorMa
                     PmTailRec rec;
                     rec.pt = (int)pt; rec.RH = RH; rec.RW = RW; rec.H = H; rec.W = W;
                     rec.best_idx = best_idx; rec.best_a = best_a; rec.best_r = best_r;
+                    rec.mode = 1; rec.tsum = best_tsum; rec.tsq = best_tsq;
                     a.tail_recs[pi] = rec;
                 }
             }
