@@ -9,6 +9,8 @@
  *                              pmlib.py:430-448 (_init_pool + Pool.map(use_mcc_mp)),
  *                              i.e. use_mcc (pmlib.py:176-212) for every grid point.
  *                              Argument order mirrors _init_pool's tuple (pmlib.py:438).
+ *   sid_run_maps               sid_run that also returns every point's winning NCC map and
+ *                              template (rotate_and_match's best_result / best_template).
  *   sid_rotate_and_match       replaces rotate_and_match, pmlib.py:117-174.
  *   sid_get_template           replaces get_template, pmlib.py:89-115.
  *   sid_match_template         replaces the template_matcher plug-in call
@@ -165,6 +167,34 @@ int sid_run_device(sid_ctx *ctx, int64_t n,
                    int img_size, int n_angles, const double *angles, const double *angle_tab,
                    int rot_order, unsigned flags, int mtype,
                    double *d_out, int *d_status);
+
+/* Shapes of the correlation maps sid_run_maps returns for these points on the RESIDENT pair: map i is
+ * map_shape[2i] x map_shape[2i+1] = (H - img_size + 1) x (W - img_size + 1), where H x W is the point's search
+ * window as use_mcc slices it (pmlib.py:200-208: truncation of r2fg +- hws +- border, NumPy's clipping of the far
+ * edge), so fractional first guesses or borders and windows at the far edge give non-square maps.  Points the
+ * window rule rejects (their status is SID_PT_REJECTED) get 0 x 0; NaN rows (SID_PT_NAN) keep their shape.
+ * *total = sum of the map sizes (floats).  map_shape may be NULL. */
+int sid_map_layout(sid_ctx *ctx, int64_t n,
+                   const double *c1, const double *r1,
+                   const double *c2fg, const double *r2fg, const double *border,
+                   int img_size, int32_t *map_shape, int64_t *total);
+
+/* sid_run plus, for every point, what rotate_and_match returns as best_result and best_template
+ * (pmlib.py:117-174, [5] and [6]); host pointers, resident pair, synchronous.  out / status are those of sid_run,
+ * bit for bit.
+ *   maps        maps_capacity floats: the maps of sid_map_layout packed in point order.  For a valid row, the raw
+ *               float32 NCC map of the winning angle (the first of equal peaks; hes_smth and mcc_norm do not touch
+ *               it; a flat template gives all 1.0).  Segments of rows that are not valid are NaN.
+ *   templates   optional (may be NULL), n x img_size x img_size bytes: the winning angle's template; 0 for rows
+ *               that are not valid.
+ * maps_capacity below sid_map_layout's total -> SID_EINVAL before anything is launched. */
+int sid_run_maps(sid_ctx *ctx, int64_t n,
+                 const double *c1, const double *r1,
+                 const double *c2fg, const double *r2fg, const double *border,
+                 int img_size, int n_angles, const double *angles, const double *angle_tab,
+                 int rot_order, unsigned flags, int mtype,
+                 double *out, int *status,
+                 int64_t maps_capacity, float *maps, uint8_t *templates);
 
 /* Number of kernel launches issued by this context so far (bench accounting). */
 int64_t sid_launch_count(const sid_ctx *ctx);

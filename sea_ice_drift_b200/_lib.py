@@ -22,7 +22,7 @@ SID_HES_NORM, SID_HES_SMTH, SID_MCC_NORM = 1, 2, 4
 
 EXPORTS = [
     "sid_version", "sid_create", "sid_destroy", "sid_last_error", "sid_set_stream", "sid_synchronize",
-    "sid_set_pair", "sid_set_pair_device", "sid_pair_layout", "sid_adopt_pair_device", "sid_upload_rows", "sid_pm_epilogue_affine", "sid_first_guess", "sid_run", "sid_run_pair", "sid_run_device", "sid_launch_count", "sid_last_kernel_ms", "sid_last_kernel_name",
+    "sid_set_pair", "sid_set_pair_device", "sid_pair_layout", "sid_adopt_pair_device", "sid_upload_rows", "sid_pm_epilogue_affine", "sid_first_guess", "sid_run", "sid_run_pair", "sid_run_device", "sid_map_layout", "sid_run_maps", "sid_launch_count", "sid_last_kernel_ms", "sid_last_kernel_name",
     "sid_rotate_and_match", "sid_get_template", "sid_match_template", "sid_get_hessian", "sid_knn_hamming2",
     "sid_deformation",
 ]
@@ -77,6 +77,8 @@ def load_library():
             [C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_uint, C.c_int, C.c_void_p, C.c_void_p]
         lib.sid_run_device.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 5 + \
             [C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_uint, C.c_int, C.c_void_p, C.c_void_p]
+        lib.sid_map_layout.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 5 + [C.c_int, C.c_void_p, C.POINTER(C.c_int64)]
+        lib.sid_run_maps.argtypes = lib.sid_run.argtypes + [C.c_int64, C.c_void_p, C.c_void_p]
         lib.sid_rotate_and_match.argtypes = [
             C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_double, C.c_double, C.c_int,
             C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_void_p, C.c_int, C.c_uint, C.c_int,
@@ -271,6 +273,35 @@ class Context(object):
         if keep_on_device:
             return status if want_status else None
         return (out, status) if want_status else out
+
+    def run_maps(self, c1, r1, c2fg, r2fg, border, img_size, angles, alpha0, rot_order=0, flags=SID_HES_NORM,
+                 mtype=SID_TM_CCOEFF_NORMED, want_status=False):
+        """:meth:`run` on the resident pair that also returns every valid row's winning NCC map and template
+        (``rotate_and_match(...)[5]`` / ``[6]``, sid_run_maps): ``(table, maps, templates[, status])``.  ``maps`` is a
+        list of N float32 2-D views into one contiguous buffer (point order), None where the row is not valid;
+        ``templates`` an (N, img_size, img_size) uint8 array, 0 where the row is not valid."""
+        arrs = [np.ascontiguousarray(np.atleast_1d(x), dtype=np.float64) for x in (c1, r1, c2fg, r2fg, border)]
+        n = arrs[0].size
+        if any(a.size != n for a in arrs):
+            raise ValueError("point arrays must have equal length")
+        ang = np.ascontiguousarray(np.asarray(angles, dtype=np.float64))
+        tab = angle_table(angles, alpha0, img_size)
+        shape = np.zeros((n, 2), dtype=np.int32)
+        total = C.c_int64(0)
+        self._check(self._lib.sid_map_layout(self._h, n, *[a.ctypes.data for a in arrs], int(img_size),
+                                             shape.ctypes.data, C.byref(total)))
+        buf = np.empty(total.value, dtype=np.float32)
+        templates = np.zeros((n, int(img_size), int(img_size)), dtype=np.uint8)
+        out = np.full((n, 5), np.nan, dtype=np.float64)
+        status = np.zeros(n, dtype=np.int32)
+        self._check(self._lib.sid_run_maps(
+            self._h, n, *[a.ctypes.data for a in arrs], int(img_size), len(ang), ang.ctypes.data,
+            tab.ctypes.data, int(rot_order), int(flags), int(mtype), out.ctypes.data, status.ctypes.data,
+            buf.size, buf.ctypes.data, templates.ctypes.data))
+        ends = np.cumsum(shape[:, 0].astype(np.int64) * shape[:, 1])
+        maps = [buf[e - h * w:e].reshape(h, w) if st == 1 else None
+                for (h, w), e, st in zip(shape.tolist(), ends.tolist(), status.tolist())]
+        return (out, maps, templates, status) if want_status else (out, maps, templates)
 
     def run_pair(self, img1, img2, c1, r1, c2fg, r2fg, border, img_size, angles, alpha0, rot_order=0,
                  flags=SID_HES_NORM, mtype=SID_TM_CCOEFF_NORMED, want_status=False, keep_on_device=False):

@@ -110,6 +110,10 @@ struct sid_ctx {
     bool have_pair = false;
     // per-call buffers
     DevBuf pts, order, out, status, angles, scratch, counter, misc, tail_maps, tail_recs, epi, fg;
+    DevBuf maps, map_off, tpl;               // sid_run_maps: packed maps, their offsets, the templates
+    float *maps_out = nullptr;               // set for the duration of a sid_run_maps call (PmArgs::maps_out etc.)
+    const long long *map_off_dev = nullptr;
+    uint8_t *tpl_out = nullptr;
     void *pin = nullptr;
     size_t pin_cap = 0;
     cudaEvent_t k_ev[2] = {};                // bracket the last fused-kernel launch (sid_last_kernel_ms)
@@ -276,6 +280,7 @@ int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1,
     a.sqrt_inv_area = std::sqrt(a.inv_area);
     gaussian_weights(a.gw);
     a.out = d_out; a.status = d_status;
+    a.maps_out = ctx->maps_out; a.map_off = ctx->map_off_dev; a.tpl_out = ctx->tpl_out;
     a.max_rr = Rmax * Rmax;
     a.max_hrw = Wmax * Rmax;
     // correlation path: tcgen05 tensor cores (default), legacy mma.sync (SID_PM_PATH=imma) or the integer pipe
@@ -594,7 +599,8 @@ void sid_destroy(sid_ctx *ctx) {
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
     DevBuf *bufs[] = {&ctx->img1, &ctx->img2, &ctx->pts, &ctx->order, &ctx->out, &ctx->status,
-                      &ctx->angles, &ctx->scratch, &ctx->counter, &ctx->misc, &ctx->tail_maps, &ctx->tail_recs, &ctx->epi, &ctx->fg};
+                      &ctx->angles, &ctx->scratch, &ctx->counter, &ctx->misc, &ctx->tail_maps, &ctx->tail_recs, &ctx->epi, &ctx->fg,
+                      &ctx->maps, &ctx->map_off, &ctx->tpl};
     for (DevBuf *b : bufs) if (b->p && b->owned) cudaFree(b->p);
     if (ctx->pin) cudaFreeHost(ctx->pin);
     if (ctx->stage) cudaFreeHost(ctx->stage);
@@ -1193,6 +1199,73 @@ int sid_run_device(sid_ctx *ctx, int64_t n, const double *d_c1, const double *d_
     }
     return launch_pm(ctx, n, d_c1, d_r1, d_c2fg, d_r2fg, d_border, nullptr, max_border, max_border, img_size,
                      n_angles, d_angles, d_tab, rot_order, flags, d_out, d_status);
+}
+
+// ------------------------------------------------------------------ winning maps and templates (sid_run_maps)
+namespace {
+// Map shapes by the kernels' window rule (window_rect) on the resident pair; `off` (optional) gets the packed offsets
+int map_layout(sid_ctx *ctx, int64_t n, const double *c1, const double *r1, const double *c2fg, const double *r2fg,
+               const double *border, int img_size, int32_t *shape, std::vector<long long> *off, int64_t *total) {
+    if (!ctx) return SID_EINVAL;
+    if (!ctx->have_pair) return fail(ctx, SID_ENOPAIR, "sid_set_pair has not been called");
+    if (img_size < 2 || img_size > 128) return fail(ctx, SID_EUNSUPPORTED, "img_size must be in [2, 128]");
+    if (n < 0 || (n > 0 && (!c1 || !r1 || !c2fg || !r2fg || !border)) || !total) return fail(ctx, SID_EINVAL, "null point array");
+    if (off) off->resize((size_t)n);
+    const WindowGeom g{img_size, ctx->rows2, ctx->cols2};
+    long long acc = 0;
+    for (int64_t i = 0; i < n; ++i) {
+        long long x0, y0;
+        int W, H, RH = 0, RW = 0;
+        if (window_rect(g, c1[i], r1[i], c2fg[i], r2fg[i], border[i], x0, y0, W, H)) {
+            RH = H - img_size + 1; RW = W - img_size + 1;
+        }
+        if (shape) { shape[2 * i] = RH; shape[2 * i + 1] = RW; }
+        if (off) (*off)[(size_t)i] = acc;
+        acc += (long long)RH * RW;
+    }
+    *total = acc;
+    return SID_OK;
+}
+}  // namespace
+
+int sid_map_layout(sid_ctx *ctx, int64_t n, const double *c1, const double *r1, const double *c2fg, const double *r2fg,
+                   const double *border, int img_size, int32_t *map_shape, int64_t *total) {
+    return map_layout(ctx, n, c1, r1, c2fg, r2fg, border, img_size, map_shape, nullptr, total);
+}
+
+int sid_run_maps(sid_ctx *ctx, int64_t n, const double *c1, const double *r1, const double *c2fg,
+                 const double *r2fg, const double *border, int img_size, int n_angles, const double *angles,
+                 const double *angle_tab, int rot_order, unsigned flags, int mtype, double *out, int *status,
+                 int64_t maps_capacity, float *maps, uint8_t *templates) {
+    int rc = check_common(ctx, img_size, n_angles, angle_tab, rot_order, mtype);
+    if (rc) return rc;
+    if (!angles) return fail(ctx, SID_EINVAL, "null point array");
+    if (n > 0x7fffffffLL) return fail(ctx, SID_EINVAL, "too many points");
+    std::vector<long long> off;
+    int64_t total = 0;
+    if ((rc = map_layout(ctx, n, c1, r1, c2fg, r2fg, border, img_size, nullptr, &off, &total))) return rc;
+    if (maps_capacity < total) return fail(ctx, SID_EINVAL, "maps_capacity below the total of sid_map_layout");
+    if (total > 0 && !maps) return fail(ctx, SID_EINVAL, "null maps buffer");
+    if (n == 0) return SID_OK;
+    CU(cudaSetDevice(ctx->device));
+    const size_t tpl_bytes = (size_t)n * img_size * img_size;
+    if ((rc = reserve(ctx, ctx->maps, (size_t)std::max<int64_t>(total, 1) * sizeof(float)))) return rc;
+    if ((rc = reserve(ctx, ctx->map_off, (size_t)n * sizeof(long long)))) return rc;
+    if (templates && (rc = reserve(ctx, ctx->tpl, tpl_bytes))) return rc;
+    // segments of rows that end up not valid keep these: NaN (all bits set) maps, zero templates
+    CU(cudaMemsetAsync(ctx->maps.p, 0xff, (size_t)total * sizeof(float), ctx->stream));
+    if (templates) CU(cudaMemsetAsync(ctx->tpl.p, 0, tpl_bytes, ctx->stream));
+    CU(cudaMemcpyAsync(ctx->map_off.p, off.data(), (size_t)n * sizeof(long long), cudaMemcpyHostToDevice, ctx->stream));
+    ctx->maps_out = (float *)ctx->maps.p;
+    ctx->map_off_dev = (const long long *)ctx->map_off.p;
+    ctx->tpl_out = templates ? (uint8_t *)ctx->tpl.p : nullptr;
+    rc = run_host(ctx, nullptr, n, c1, r1, c2fg, r2fg, border, img_size, n_angles, angles, angle_tab, rot_order,
+                  flags, mtype, out, status);
+    ctx->maps_out = nullptr; ctx->map_off_dev = nullptr; ctx->tpl_out = nullptr;
+    if (rc) return rc;
+    if (total > 0) CU(cudaMemcpy(maps, ctx->maps.p, (size_t)total * sizeof(float), cudaMemcpyDeviceToHost));
+    if (templates) CU(cudaMemcpy(templates, ctx->tpl.p, tpl_bytes, cudaMemcpyDeviceToHost));
+    return SID_OK;
 }
 
 // ------------------------------------------------------------------ post-processing epilogue (SURVEY 8f rank 2)

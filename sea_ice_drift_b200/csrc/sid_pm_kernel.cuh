@@ -85,6 +85,11 @@ struct PmArgs {
     float *tail_maps;             // n x tail_stride
     int tail_stride;              // floats per handed-over map: max_rr rounded up to 4 (16-byte rows for the tail's vector loads)
     PmTailRec *tail_recs;         // n
+    // sid_run_maps only (null otherwise): the winning angle's raw NCC map of point pt goes to maps_out + map_off[pt],
+    // its template (s x s) to tpl_out + pt * s * s when tpl_out is set
+    float *maps_out;
+    const long long *map_off;
+    uint8_t *tpl_out;
 };
 
 __host__ __device__ inline int pm_window_pitch_words(int W, bool imma = false) {
@@ -385,8 +390,11 @@ __host__ __device__ inline int pm_pick_tx(int RW) {
 
 // Search window of one point: img2[int(r2-hws-b):int(r2+hws+b+1), int(c2-hws-b):int(c2+hws+b+1)] with NumPy's
 // clipping of the far end (reference pmlib.py:200-202).  Returns false for windows the reference cannot process.
-__device__ __forceinline__ bool pm_window_rect(const PmArgs &a, double c1, double r1, double c2, double r2, double brd,
-                                               long long &x0, long long &y0, int &W, int &H) {
+// The one definition of the rule, for the kernels (G = PmArgs) and for sid_map_layout on the host (G = WindowGeom).
+struct WindowGeom { int s, rows2, cols2; };
+template <class G>
+__host__ __device__ __forceinline__ bool window_rect(const G &a, double c1, double r1, double c2, double r2, double brd,
+                                                     long long &x0, long long &y0, int &W, int &H) {
     const int s = a.s, hws = s / 2;
     bool ok = isfinite(c1) && isfinite(r1) && isfinite(c2) && isfinite(r2) && isfinite(brd) &&
               fabs(c2) < 1e9 && fabs(r2) < 1e9 && fabs(brd) < 1e9;
@@ -402,6 +410,32 @@ __device__ __forceinline__ bool pm_window_rect(const PmArgs &a, double c1, doubl
     ok = y0 >= 0 && x0 >= 0 && (y1 - y0) >= s + 1 && (x1 - x0) >= s + 1;
     H = (int)(y1 - y0); W = (int)(x1 - x0);
     return ok;
+}
+__device__ __forceinline__ bool pm_window_rect(const PmArgs &a, double c1, double r1, double c2, double r2, double brd,
+                                               long long &x0, long long &y0, int &W, int &H) {
+    return window_rect(a, c1, r1, c2, r2, brd, x0, y0, W, H);
+}
+
+// sid_run_maps: store the winning angle's raw NCC map (RR floats at `map`), read before peak_statistics may smooth or
+// reuse it.  Called by every thread of the CTA; ends with a barrier, so the caller may overwrite `map` afterwards.
+__device__ __forceinline__ void pm_store_map(const PmArgs &a, long long pt, const float *map, int RR) {
+    float *dst = a.maps_out + a.map_off[pt];
+    for (int k = threadIdx.x; k < RR; k += blockDim.x) dst[k] = map[k];
+    __syncthreads();
+}
+// sid_run_maps: the winning angle's template, regathered with template_pixel so that it is bit-identical to
+// templates_kernel.  The fused kernels call it at the very end of a point, where little else is live (inside their
+// tail it would raise the register pressure of the whole loop).
+__device__ __forceinline__ void pm_store_template(const PmArgs &a, long long pt, int best_a) {
+    const int s = a.s;
+    const double *tab = a.tab + 4 * best_a;
+    const double cs = tab[0], sn = tab[1];
+    const double off0 = __dsub_rn(a.r1[pt], tab[2]), off1 = __dsub_rn(a.c1[pt], tab[3]);
+    uint8_t *dst = a.tpl_out + (size_t)pt * s * s;
+    for (int k = threadIdx.x; k < s * s; k += blockDim.x) {
+        const int i = k / s, j = k - i * s;
+        dst[k] = template_pixel(a.img1, a.rows1, a.cols1, a.pitch1, off0, off1, cs, sn, i, j, a.rot_order);
+    }
 }
 
 // Scratch footprint of one CTA (bytes): wden f64[rr] | wsum u32[rr] | region, where the region
@@ -715,6 +749,7 @@ pm_points_kernel(const PmArgs a, const __grid_constant__ CUtensorMap tmap2) {
             }
             continue;
         }
+        if (a.maps_out) pm_store_map(a, pt, best, RR);
         float *tmp_a = maps + (size_t)(best_slot == 0 ? 1 : 0) * a.max_rr;
         float *hes = maps + (size_t)(ab + 1) * a.max_rr;
         float *tmp_b = maps + (size_t)(ab + 2) * a.max_rr;      // only allocated (and touched) with hes_smth
@@ -732,6 +767,7 @@ pm_points_kernel(const PmArgs a, const __grid_constant__ CUtensorMap tmap2) {
             o[4] = (double)ps.h;
             if (a.status) a.status[pt] = 1;
         }
+        if (a.tpl_out) pm_store_template(a, pt, S.best_a);
     }
 }
 
@@ -773,6 +809,10 @@ __global__ void __launch_bounds__(PM_TAIL_MAX_THREADS) pm_tail_kernel(const PmAr
         }
     }
     __syncthreads();
+    if (a.maps_out) {
+        pm_store_map(a, rec.pt, map, RR);
+        if (a.tpl_out) pm_store_template(a, rec.pt, rec.best_a);
+    }
     // hes_norm-only maps take peak_statistics' three-sweep fast path (sid_common.cuh) on the 2048-word histogram
     const PeakStats ps = peak_statistics(map, rec.RH, rec.RW, rec.best_idx, rec.best_r, a.flags, a.gw, tmp_a, tmp_b, hes, bs, wide_hist);
     if (tid == 0) {

@@ -793,6 +793,7 @@ pm_tc_kernel(const PmArgs a, const PmTcCfg g, const __grid_constant__ CUtensorMa
             }
             continue;
         }
+        if (a.maps_out) pm_store_map(a, pt, best, RR);
         float *tmp_a = maps + (size_t)(best_slot == 0 ? 1 : 0) * a.max_rr;
         float *hes = maps + (size_t)(nab + 1) * a.max_rr;
         float *tmp_b = maps + (size_t)(nab + 2) * a.max_rr;
@@ -813,6 +814,7 @@ pm_tc_kernel(const PmArgs a, const PmTcCfg g, const __grid_constant__ CUtensorMa
             o[4] = (double)ps.h;
             if (a.status) a.status[pt] = 1;
         }
+        if (a.tpl_out) pm_store_template(a, pt, S.best_a);
     }
     // a window requested for a work item that never ran (the list ended) must land before the CTA exits
     if (S.tma_for != 0xffffffffu && (long long)S.tma_for >= a.n) { /* never requested past the end: nok == 0 there */ }

@@ -112,8 +112,17 @@ def use_mcc_batch(c1, r1, c2fg, r2fg, border, img1, img2, img_size, alpha0, **kw
 
     ``resident=True`` (extension): reuse the image pair uploaded by this context's previous call instead of
     uploading ``img1`` / ``img2`` again -- an explicit contract, for callers that run several grids or kwargs
-    sets over one pair; raises nothing and uploads anyway when no pair is resident."""
+    sets over one pair; raises nothing and uploads anyway when no pair is resident.
+
+    ``return_maps=True`` (extension): return ``(table, maps, templates)`` where ``maps[i]`` is what
+    ``rotate_and_match(...)[5]`` gives for point i's window -- the float32 NCC map of the winning angle -- or None
+    where the row is NaN, and ``templates[i]`` (an (N, img_size, img_size) uint8 array) is ``[6]``, the winning
+    angle's template (zeros where the row is NaN)."""
     matcher = kwargs.get('template_matcher')
+    return_maps = kwargs.get('return_maps', False)
+    if return_maps and not _is_builtin_matcher(matcher):
+        raise ValueError("return_maps=True needs the built-in matcher (template_matcher None, match_template or "
+                         "cv2.matchTemplate)")
     if not _is_builtin_matcher(matcher):
         rows = [use_mcc(a, b, c, d, e, img1, img2, img_size, alpha0, **kwargs)
                 for a, b, c, d, e in zip(c1, r1, c2fg, r2fg, border)]
@@ -127,6 +136,11 @@ def use_mcc_batch(c1, r1, c2fg, r2fg, border, img1, img2, img_size, alpha0, **kw
     # the caller states explicitly that the pair of its previous call is still the one to match: the library
     # never infers identity from pointers or sampled checksums (an in-place edit such as masking land, or a new
     # array at a recycled address, would silently match against the old pair).
+    if return_maps:
+        if not (kwargs.get('resident') and ctx._pair_key is not None):
+            ctx.set_pair(img1, img2)
+            ctx._pair_key = (np.shape(img1), np.shape(img2))
+        return ctx.run_maps(*args)
     if kwargs.get('resident') and ctx._pair_key is not None:
         return ctx.run(*args)
     out = ctx.run_pair(img1, img2, *args)
