@@ -1389,7 +1389,16 @@ int sid_first_guess(sid_ctx *ctx, int n_src, const double *sx, const double *sy,
     if (n_src >= 3) convex_hull(sx, sy, n_src, hull);
     const int nh = (int)hull.size();
     std::vector<double> hx((size_t)nh), hy((size_t)nh);
-    for (int i = 0; i < nh; ++i) { hx[(size_t)i] = sx[hull[(size_t)i]]; hy[(size_t)i] = sy[hull[(size_t)i]]; }
+    double bx0 = 1e300, bx1 = -1e300, by0 = 1e300, by1 = -1e300;      // the hull's bounding box is the sources'
+    for (int i = 0; i < nh; ++i) {
+        hx[(size_t)i] = sx[hull[(size_t)i]]; hy[(size_t)i] = sy[hull[(size_t)i]];
+        bx0 = std::min(bx0, hx[(size_t)i]); bx1 = std::max(bx1, hx[(size_t)i]); by0 = std::min(by0, hy[(size_t)i]); by1 = std::max(by1, hy[(size_t)i]);
+    }
+    std::vector<double> hband((size_t)nh);                             // SciPy's band around every hull edge (sid_fg_kernel.cuh)
+    for (int i = 0; i < nh; ++i) {
+        const int j = i + 1 == nh ? 0 : i + 1;
+        hband[(size_t)i] = FG_HULL_BAND_EPS * std::hypot(bx1 - bx0, by1 - by0) * std::hypot(hx[(size_t)j] - hx[(size_t)i], hy[(size_t)j] - hy[(size_t)i]);
+    }
     // one staging block: everything the kernel reads, 256-byte aligned pieces
     struct Piece { const void *src; size_t bytes; size_t off; };
     std::vector<Piece> pieces;
@@ -1399,6 +1408,7 @@ int sid_first_guess(sid_ctx *ctx, int n_src, const double *sx, const double *sy,
     const size_t i_ss = add(gs.start.data(), gs.start.size() * 4), i_si = add(gs.index.data(), (size_t)n_src * 4);
     const size_t i_vx = add(vx, (size_t)n_src * 8), i_vy = add(vy, (size_t)n_src * 8);
     const size_t i_hx = add(hx.data(), (size_t)nh * 8), i_hy = add(hy.data(), (size_t)nh * 8), i_hi = add(hull.data(), (size_t)nh * 4);
+    const size_t i_hb = add(hband.data(), (size_t)nh * 8);
     const size_t i_kx = add(gk.x.data(), (size_t)n_seed * 8), i_ky = add(gk.y.data(), (size_t)n_seed * 8);
     const size_t i_ks = add(gk.start.data(), gk.start.size() * 4), i_ki = add(gk.index.data(), (size_t)n_seed * 4);
     const size_t i_qx = add(qx, (size_t)n_q * 8), i_qy = add(qy, (size_t)n_q * 8);
@@ -1418,6 +1428,7 @@ int sid_first_guess(sid_ctx *ctx, int n_src, const double *sx, const double *sy,
     a.src.x0 = gs.x0; a.src.y0 = gs.y0; a.src.cell = gs.cell; a.src.inv_cell = 1.0 / gs.cell; a.src.nx = gs.nx; a.src.ny = gs.ny; a.src.n = n_src;
     a.vx = (const double *)at(i_vx); a.vy = (const double *)at(i_vy);
     a.hx = (const double *)at(i_hx); a.hy = (const double *)at(i_hy); a.hidx = (const int *)at(i_hi); a.nh = nh;
+    a.hband = (const double *)at(i_hb);
     a.seed.x = (const double *)at(i_kx); a.seed.y = (const double *)at(i_ky); a.seed.start = (const int *)at(i_ks); a.seed.index = (const int *)at(i_ki);
     a.seed.x0 = gk.x0; a.seed.y0 = gk.y0; a.seed.cell = gk.cell; a.seed.inv_cell = 1.0 / gk.cell; a.seed.nx = gk.nx; a.seed.ny = gk.ny; a.seed.n = n_seed;
     a.nq = n_q; a.qx = (const double *)at(i_qx); a.qy = (const double *)at(i_qy);

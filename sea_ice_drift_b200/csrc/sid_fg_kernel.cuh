@@ -31,12 +31,14 @@ struct FgArgs {
     const double *vx, *vy; // values at the sources (matched positions on image 2), original order
     const double *hx, *hy; // convex hull of the sources, counter-clockwise, nh vertices
     const int *hidx;       // source index of every hull vertex
+    const double *hband;   // per hull edge k -> k + 1: FG_HULL_BAND_EPS * |edge| * diagonal of the sources' bounding box
     int nh;
     FgGrid seed;           // integer keypoint positions on image 2 (nearest-keypoint distance)
     long long nq;
     const double *qx, *qy; // query points
     double *out_vx, *out_vy, *out_dist;
-    int *out_flag;         // 0 ok, 1 outside the hull (NaN), 2 not resolved numerically, 3 ok but a further keypoint lies ON the
+    int *out_flag;         // 0 ok, 1 outside the hull (NaN), 2 not resolved numerically or within SciPy's band around the hull
+                           // boundary (NaN there), 3 ok but a further keypoint lies ON the
                            // circumcircle: the Delaunay triangulation is not unique there (Qhull's choice may differ)
 };
 
@@ -49,12 +51,30 @@ __device__ __forceinline__ double fg_incircle(double ax, double ay, double bx, d
     const double ad = adx * adx + ady * ady, bd = bdx * bdx + bdy * bdy, cd = cdx * cdx + cdy * cdy;
     return adx * (bdy * cd - bd * cdy) - ady * (bdx * cd - bd * cdx) + ad * (bdx * cdy - bdy * cdx);
 }
+// Closed triangle test by orientation signs.  The hull test in first_guess_kernel is the same test against the hull edges, but
+// SciPy decides "inside" differently: _find_simplex_directed (scipy/spatial/_qhull.pyx) accepts q in a simplex when
+// every barycentric coordinate is >= -eps, eps = 100 * DBL_EPSILON, so LinearNDInterpolator / griddata return a value
+// slightly OUTSIDE the hull.  Bound on that band: if SciPy accepts q in the triangle v0 v1 v2, q = sum c_i v_i with
+// sum c_i = 1 and c_i >= -eps; orient(a, b, .) against a hull edge a b is affine and lies in [0, |ab| * D] on every source
+// (D the diagonal of the sources' bounding box), and at most two c_i are negative, so
+// orient(a, b, q) >= -2 * eps * |ab| * D.  The kernel widens that by ~10x (FG_HULL_BAND_EPS) to cover the rounding of
+// fg_orient and of SciPy's barycentric transform.  That rounding also makes SciPy's answer for a query ON the hull
+// boundary arbitrary: on the thin hull triangles of a ring of integer points it returns NaN for integer queries exactly
+// on a hull edge.  So the band is two-sided: a query whose orientation against some hull edge lies within
+// +-FG_HULL_BAND_EPS * D * |ab| (and below none) is undecided, flag 2, and the host decides.
+constexpr double FG_HULL_BAND_EPS = 2048.0 * 2.220446049250313e-16;
+// fg_orient without fused multiply-adds: with the two products rounded alike, fg_orient_rn(a, b, b) is exactly 0 (with an
+// FMA it is the rounding error of one product, of either sign), so a query ON a keypoint lies on the closed triangles
+// that have the keypoint as a vertex; otherwise a pivot onto a keypoint equal to q could find no triangle holding q.
+__device__ __forceinline__ double fg_orient_rn(double ax, double ay, double bx, double by, double cx, double cy) {
+    return __dsub_rn(__dmul_rn(bx - ax, cy - ay), __dmul_rn(by - ay, cx - ax));
+}
 __device__ __forceinline__ bool fg_contains(double ax, double ay, double bx, double by, double cx, double cy, double qx, double qy) {
-    const double o = fg_orient(ax, ay, bx, by, cx, cy);
+    const double o = fg_orient_rn(ax, ay, bx, by, cx, cy);
     if (o == 0.0) return false;
     const double s = o > 0.0 ? 1.0 : -1.0;
-    return s * fg_orient(ax, ay, bx, by, qx, qy) >= 0.0 && s * fg_orient(bx, by, cx, cy, qx, qy) >= 0.0 &&
-           s * fg_orient(cx, cy, ax, ay, qx, qy) >= 0.0;
+    return s * fg_orient_rn(ax, ay, bx, by, qx, qy) >= 0.0 && s * fg_orient_rn(bx, by, cx, cy, qx, qy) >= 0.0 &&
+           s * fg_orient_rn(cx, cy, ax, ay, qx, qy) >= 0.0;
 }
 __device__ __forceinline__ int fg_cell(double v, double v0, double inv, int n) {
     int c = (int)floor((v - v0) * inv);
@@ -101,10 +121,17 @@ __global__ void __launch_bounds__(128) first_guess_kernel(const FgArgs a) {
     const FgGrid &g = a.src;
     int fan = -1;
     if (a.nh >= 3) {
-        bool inside = true;
+        bool inside = true, band = false;
         for (int k = 0; k < a.nh && inside; ++k) {
             const int k2 = k + 1 == a.nh ? 0 : k + 1;
-            inside = fg_orient(a.hx[k], a.hy[k], a.hx[k2], a.hy[k2], qx, qy) >= 0.0;
+            const double o = fg_orient(a.hx[k], a.hy[k], a.hx[k2], a.hy[k2], qx, qy);
+            if (o < -a.hband[k]) inside = false;
+            else if (o <= a.hband[k]) band = true;               // on the hull boundary up to SciPy's band (see fg_contains)
+        }
+        if (inside && band) {
+            a.out_vx[t] = a.out_vy[t] = nan("");
+            a.out_flag[t] = 2;
+            return;
         }
         if (inside)
             for (int k = 1; k + 1 < a.nh; ++k)

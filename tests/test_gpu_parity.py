@@ -624,7 +624,9 @@ def test_first_guess_on_device_ew_size_and_interpolant_values():
 def test_first_guess_integer_keypoints_cocircular_degeneracies():
     """ORB keypoints of pyramid level 0 sit on integer pixels, so four of them can be cocircular and the Delaunay
     triangulation is then not unique (Qhull's choice is arbitrary too): the device result must still be a valid
-    Delaunay interpolant -- equal to the SciPy path except at grid points inside such degenerate cells."""
+    Delaunay interpolant -- the lifted-paraboloid check of tests/test_first_guess_geometry.py, whose expected value is
+    the same over every valid triangulation of a cocircular cell."""
+    from tests import test_first_guess_geometry as fgg
     n1, n2, kx, ky, k2x, k2y, gx, gy = _fg_case(1200, 3000, 60, 4, integer_keypoints=True)
     dev = sid.prepare_first_guess(gx, gy, n1, kx, ky, n2, k2x, k2y, 35, first_guess='device')
     host = sid.prepare_first_guess(gx, gy, n1, kx, ky, n2, k2x, k2y, 35, first_guess='host')
@@ -634,6 +636,6 @@ def test_first_guess_integer_keypoints_cocircular_degeneracies():
     flag = _lib.default_context().first_guess(kx, ky, k2x, k2y, kx, ky, gx, gy)[3]
     assert (flag == 3).any() and not (flag == 2).any()
     assert np.array_equal(dev[2], host[2])                                   # distances are exact either way
-    differ = (dev[0] != host[0]) | (dev[1] != host[1])
-    assert differ.mean() < 0.02, differ.mean()
-    assert np.abs(dev[0] - host[0]).max() <= 3 and np.abs(dev[1] - host[1]).max() <= 3
+    fgg.add_layout("integer_keypoints", kx, ky, k2x, k2y, gx, gy)
+    census = fgg.check_device(_lib.default_context(), "integer_keypoints", generic=False)
+    assert census[3] > 0 and census[2] == 0
