@@ -57,6 +57,13 @@ typedef struct sid_ctx sid_ctx;
 #define SID_HES_NORM 1u      /* get_hessian(hes_norm=True)  -- reference default */
 #define SID_HES_SMTH 2u      /* get_hessian(hes_smth=True)                       */
 #define SID_MCC_NORM 4u      /* rotate_and_match(mcc_norm=True)                  */
+/* SID_SUBPIXEL (extension, not in the reference): refine c2 / r2 (dc / dr) to sub-pixel precision by the vertex of the
+ * parabola through the peak of the winning angle's RAW float32 NCC map and its two neighbours, per axis:
+ *   a, b, c = m[bi][bj-1], m[bi][bj], m[bi][bj+1] widened to double;  p = b - a, q = b - c;
+ *   dx = (p - q) / (2 (p + q));  c2 = (c2fg + dc) + dx     (IEEE double, round to nearest, no fused operations)
+ * and the same down the column for dy and r2.  |dx|, |dy| <= 0.5; a peak on the first or last column (row) leaves c2
+ * (r2) exactly as without the flag.  Angle, r, h, the NaN rows and status are bit-identical to the call without it. */
+#define SID_SUBPIXEL 8u
 
 /* point status written by sid_run* (optional output) */
 #define SID_PT_VALID 1
@@ -130,7 +137,8 @@ int sid_upload_rows(sid_ctx *ctx, uint8_t *d_dst, int64_t dst_pitch, const uint8
  *   c1, r1        float pixel coordinates on image 1
  *   c2fg, r2fg    integer-valued first guess on image 2
  *   border        integer-valued search radius per point
- *   out           n x 5 row-major doubles: c2, r2, angle, r, h  (NaN rows = invalid)
+ *   out           n x 5 row-major doubles: c2, r2, angle, r, h  (NaN rows = invalid); with SID_SUBPIXEL in `flags`
+ *                 c2 / r2 are refined to sub-pixel precision, the other columns do not change
  *   status        optional (may be NULL), n ints, SID_PT_*                          */
 int sid_run(sid_ctx *ctx, int64_t n,
             const double *c1, const double *r1,
@@ -145,7 +153,8 @@ int sid_run(sid_ctx *ctx, int64_t n,
  * identical to sid_set_pair followed by sid_run; the pair stays resident afterwards.  Page-locked host
  * images are copied by DMA directly; pageable ones (plain malloc / NumPy memory) go band by band through
  * a pinned double buffer that a few host threads fill while the previous band is in flight (EW-sized
- * pair, B200: 6.1 ms per call pinned, 9.7 ms pageable, against 26 ms for a plain pageable cudaMemcpy). */
+ * pair, B200: 6.1 ms per call pinned, 9.7 ms pageable, against 26 ms for a plain pageable cudaMemcpy).
+ * SID_SUBPIXEL refines c2 / r2 as in sid_run. */
 int sid_run_pair(sid_ctx *ctx,
                  const uint8_t *img1, int rows1, int cols1, int64_t pitch1,
                  const uint8_t *img2, int rows2, int cols2, int64_t pitch2,
@@ -159,7 +168,7 @@ int sid_run_pair(sid_ctx *ctx,
 /* Same with DEVICE pointers for the point arrays and outputs; asynchronous on
  * the context's stream (no host synchronisation).  `max_border` must bound
  * border[] (it sizes shared memory / scratch); pass <= 0 to have the library
- * read the borders back (synchronises). */
+ * read the borders back (synchronises).  SID_SUBPIXEL refines c2 / r2 as in sid_run. */
 int sid_run_device(sid_ctx *ctx, int64_t n,
                    const double *d_c1, const double *d_r1,
                    const double *d_c2fg, const double *d_r2fg, const double *d_border,
@@ -181,7 +190,8 @@ int sid_map_layout(sid_ctx *ctx, int64_t n,
 
 /* sid_run plus, for every point, what rotate_and_match returns as best_result and best_template
  * (pmlib.py:117-174, [5] and [6]); host pointers, resident pair, synchronous.  out / status are those of sid_run,
- * bit for bit.
+ * bit for bit.  With SID_SUBPIXEL the table is refined as in sid_run and the maps are unchanged (the offsets are
+ * computed from them).
  *   maps        maps_capacity floats: the maps of sid_map_layout packed in point order.  For a valid row, the raw
  *               float32 NCC map of the winning angle (the first of equal peaks; hes_smth and mcc_norm do not touch
  *               it; a flat template gives all 1.0).  Segments of rows that are not valid are NaN.
@@ -209,7 +219,8 @@ const char *sid_last_kernel_name(const sid_ctx *ctx);
 /* rotate_and_match for one point against an explicit search window `image2`
  * (host pointers).  Outputs: *valid (0 -> the reference returns 7 x NaN),
  * dc, dr, best_angle_idx (index into the angle list), best_r, best_h, and
- * optionally the best NCC map ((H-s+1) x (W-s+1) floats) and template (s x s). */
+ * optionally the best NCC map ((H-s+1) x (W-s+1) floats) and template (s x s).
+ * SID_SUBPIXEL adds the sub-pixel offsets of sid_run to *dc / *dr; best_result is the unrefined map. */
 int sid_rotate_and_match(sid_ctx *ctx,
                          const uint8_t *img1, int rows1, int cols1, int64_t pitch1,
                          double c1, double r1, int img_size,

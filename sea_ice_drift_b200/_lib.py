@@ -19,6 +19,7 @@ _i32p = C.POINTER(C.c_int)
 
 SID_TM_CCOEFF_NORMED = 5
 SID_HES_NORM, SID_HES_SMTH, SID_MCC_NORM = 1, 2, 4
+SID_SUBPIXEL = 8                # extension: sub-pixel c2 / r2 (include/sid_b200.h)
 
 EXPORTS = [
     "sid_version", "sid_create", "sid_destroy", "sid_last_error", "sid_set_stream", "sid_synchronize",
@@ -128,8 +129,16 @@ def pair_layout(rows, cols):
     return int(pitch.value), int(nbytes.value)
 
 
-def flags_from_kwargs(hes_norm=True, hes_smth=False, mcc_norm=False):
-    return (SID_HES_NORM if hes_norm else 0) | (SID_HES_SMTH if hes_smth else 0) | (SID_MCC_NORM if mcc_norm else 0)
+def flags_from_kwargs(hes_norm=True, hes_smth=False, mcc_norm=False, subpixel=False):
+    return (SID_HES_NORM if hes_norm else 0) | (SID_HES_SMTH if hes_smth else 0) | (SID_MCC_NORM if mcc_norm else 0) | \
+        (SID_SUBPIXEL if subpixel else 0)
+
+
+def flags_from_options(kwargs):
+    """The sid_run* flags of a kwargs dict of the drop-in API: ``hes_norm`` (default True), ``hes_smth``, ``mcc_norm``
+    and the extension ``subpixel`` (default False), so every entry point maps its keyword arguments the same way."""
+    return flags_from_kwargs(kwargs.get('hes_norm', True), kwargs.get('hes_smth', False), kwargs.get('mcc_norm', False),
+                             kwargs.get('subpixel', False))
 
 
 class Context(object):

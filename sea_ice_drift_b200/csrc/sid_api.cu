@@ -1668,6 +1668,7 @@ int sid_rotate_and_match(sid_ctx *ctx, const uint8_t *img1, int rows1, int cols1
     uint32_t *d_ts = d_stats + (size_t)n_angles * 3 + 4;              // 2
     unsigned long long *d_key = (unsigned long long *)(((uintptr_t)(d_ts + 4) + 15) & ~(uintptr_t)15);   // one per angle
     float *d_peak = (float *)(d_key + n_angles + 1);
+    double *d_offsets = (double *)(d_peak + 2);                       // 2, with SID_SUBPIXEL
     const size_t mstride = map_bytes / 4;
 
     CU(cudaMemcpyAsync(d_tab, angle_tab, (size_t)n_angles * 32, cudaMemcpyHostToDevice, ctx->stream));
@@ -1715,10 +1716,13 @@ int sid_rotate_and_match(sid_ctx *ctx, const uint8_t *img1, int rows1, int cols1
     pa.best = d_maps + (size_t)ba * mstride; pa.rows = RH; pa.cols = RW; pa.idx = (int)bidx; pa.r = br; pa.flags = flags;
     gaussian_weights(pa.gw);
     pa.tmp_a = d_maps + (size_t)n_angles * mstride; pa.tmp_b = pa.tmp_a + mstride; pa.hes = pa.tmp_b + mstride; pa.out = d_peak;
+    pa.offsets = d_offsets;
     peak_stats_kernel<<<1, 1024, 0, ctx->stream>>>(pa);
     ctx->launches += 1;
     float hp[2];
+    double offsets[2] = {0.0, 0.0};
     CU(cudaMemcpyAsync(hp, d_peak, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    if (flags & SID_SUBPIXEL) CU(cudaMemcpyAsync(offsets, d_offsets, 16, cudaMemcpyDeviceToHost, ctx->stream));
     if (best_result) CU(cudaMemcpyAsync(best_result, pa.best, rr * 4, cudaMemcpyDeviceToHost, ctx->stream));
     if (best_template) CU(cudaMemcpyAsync(best_template, d_tpl + (size_t)ba * s * s, (size_t)s * s, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
@@ -1726,6 +1730,10 @@ int sid_rotate_and_match(sid_ctx *ctx, const uint8_t *img1, int rows1, int cols1
     const int bi = (int)(bidx / (uint32_t)RW), bj = (int)(bidx % (uint32_t)RW);
     *dr = (double)bi - (double)(H - s) / 2.0;
     *dc = (double)bj - (double)(W - s) / 2.0;
+    if (flags & SID_SUBPIXEL) {         // the batched kernels' order: (unrefined) + offset
+        *dr = *dr + offsets[1];
+        *dc = *dc + offsets[0];
+    }
     *best_angle_idx = ba;
     *best_r = hp[0];
     *best_h = hp[1];

@@ -617,7 +617,7 @@ __device__ PeakStats peak_statistics(const float *__restrict__ best, int rows, i
                                      float *__restrict__ tmp_a, float *__restrict__ tmp_b, float *__restrict__ hes,
                                      BlockScratch &bs, uint32_t *wide_hist = nullptr) {
     const int tid = threadIdx.x, nt = blockDim.x, n = rows * cols;
-    if (flags == 1u && wide_hist != nullptr && rows >= 5 && cols >= 5 && (n & 1) && (nt == 128 || nt == 256 || nt == 512)) {
+    if ((flags & 7u) == 1u && wide_hist != nullptr && rows >= 5 && cols >= 5 && (n & 1) && (nt == 128 || nt == 256 || nt == 512)) {
         PeakStats fast;
         fast.r = peak_r;
         fast.h = hes_norm_fast(best, rows, cols, peak_idx, hes, wide_hist, bs);
@@ -682,6 +682,27 @@ __device__ PeakStats peak_statistics(const float *__restrict__ best, int rows, i
         ps.r = __fdiv_rn(__fsub_rn(peak_r, med), sd);
     }
     return ps;
+}
+
+// Sub-pixel offsets of the peak (SID_SUBPIXEL): the vertex of the parabola through the peak b and its neighbours a (lower
+// index) and c (higher index), one axis at a time, on the RAW float32 map of the winning angle (the map peak_statistics
+// reads, never the smoothed one).  p = b - a, q = b - c, d = (p - q) / (2 (p + q)) in FP64 intrinsics without
+// contraction, so a NumPy float64 restatement is bit-identical.  A peak on the first or last column (row)
+// gives +0.0 on that axis.  No guard is needed: the map is finite (flat template -> 1, tiny variance -> 0) and (bi, bj) is
+// np.argmax's FIRST maximum, so the lower-index neighbour is strictly smaller and the other one no larger: p > 0,
+// q >= 0, p + q > 0.  |p - q| <= p + q survives monotone rounding, so |d| <= 0.5 exactly, and d = +0.5 exactly when the
+// higher-index neighbour ties the peak.  Called by the one thread that writes the row.
+struct PeakOffsets { double dx, dy; };
+__device__ __forceinline__ double parabola_vertex(float a, float b, float c) {
+    const double p = __dsub_rn((double)b, (double)a), q = __dsub_rn((double)b, (double)c);
+    return __ddiv_rn(__dsub_rn(p, q), __dmul_rn(2.0, __dadd_rn(p, q)));
+}
+__device__ __forceinline__ PeakOffsets peak_offsets(const float *map, int rows, int cols, int bi, int bj) {
+    const float *pk = map + (size_t)bi * cols + bj;
+    PeakOffsets d;
+    d.dx = (bj > 0 && bj < cols - 1) ? parabola_vertex(pk[-1], pk[0], pk[1]) : 0.0;
+    d.dy = (bi > 0 && bi < rows - 1) ? parabola_vertex(pk[-cols], pk[0], pk[cols]) : 0.0;
+    return d;
 }
 
 // ---------------------------------------------------------------- TMA (cp.async.bulk.tensor) + mbarrier

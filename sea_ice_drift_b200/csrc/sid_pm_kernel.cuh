@@ -762,6 +762,11 @@ pm_points_kernel(const PmArgs a, const __grid_constant__ CUtensorMap tmap2) {
             const double dc = (double)bj - (double)(W - s) / 2.0;
             o[0] = c2 + dc;
             o[1] = r2 + dr;
+            if (a.flags & 8u) {         // SID_SUBPIXEL: peak_statistics leaves `best` intact
+                const PeakOffsets d = peak_offsets(best, RH, RW, bi, bj);
+                o[0] = __dadd_rn(o[0], d.dx);
+                o[1] = __dadd_rn(o[1], d.dy);
+            }
             o[2] = a.angles[S.best_a];
             o[3] = (double)ps.r;
             o[4] = (double)ps.h;
@@ -820,8 +825,14 @@ __global__ void __launch_bounds__(PM_TAIL_MAX_THREADS) pm_tail_kernel(const PmAr
         const double dr = (double)bi - (double)(rec.H - a.s) / 2.0;
         const double dc = (double)bj - (double)(rec.W - a.s) / 2.0;
         double *o = a.out + 5 * (long long)rec.pt;
-        o[0] = a.c2fg[rec.pt] + dc;
-        o[1] = a.r2fg[rec.pt] + dr;
+        double c2o = a.c2fg[rec.pt] + dc, r2o = a.r2fg[rec.pt] + dr;
+        if (a.flags & 8u) {             // SID_SUBPIXEL: peak_statistics leaves `map` intact
+            const PeakOffsets d = peak_offsets(map, rec.RH, rec.RW, bi, bj);
+            c2o = __dadd_rn(c2o, d.dx);
+            r2o = __dadd_rn(r2o, d.dy);
+        }
+        o[0] = c2o;
+        o[1] = r2o;
         o[2] = a.angles[rec.best_a];
         o[3] = (double)ps.r;
         o[4] = (double)ps.h;

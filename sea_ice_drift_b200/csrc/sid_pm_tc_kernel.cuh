@@ -809,6 +809,11 @@ pm_tc_kernel(const PmArgs a, const PmTcCfg g, const __grid_constant__ CUtensorMa
             const double dc = (double)bj - (double)(W - s) / 2.0;
             o[0] = c2 + dc;
             o[1] = r2 + dr;
+            if (a.flags & 8u) {         // SID_SUBPIXEL: peak_statistics leaves `best` intact
+                const PeakOffsets d = peak_offsets(best, RH, RW, bi, bj);
+                o[0] = __dadd_rn(o[0], d.dx);
+                o[1] = __dadd_rn(o[1], d.dy);
+            }
             o[2] = a.angles[S.best_a];
             o[3] = (double)ps.r;
             o[4] = (double)ps.h;

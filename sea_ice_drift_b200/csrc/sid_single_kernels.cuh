@@ -154,10 +154,16 @@ __global__ void __launch_bounds__(1024) argmax_kernel(const float *__restrict__ 
     }
 }
 
-// ---- tail of rotate_and_match on a map in global memory: out[0] = r, out[1] = h
-struct PeakArgs { const float *best; int rows, cols, idx; float r; unsigned flags; double gw[5]; float *tmp_a, *tmp_b, *hes; float *out; };
+// ---- tail of rotate_and_match on a map in global memory: out[0] = r, out[1] = h; with SID_SUBPIXEL also
+// offsets[0] = dx, offsets[1] = dy (peak_offsets)
+struct PeakArgs { const float *best; int rows, cols, idx; float r; unsigned flags; double gw[5]; float *tmp_a, *tmp_b, *hes; float *out; double *offsets; };
 __global__ void __launch_bounds__(1024) peak_stats_kernel(const PeakArgs a) {
     __shared__ BlockScratch bs;
+    if (threadIdx.x == 0 && (a.flags & 8u)) {
+        const int bi = a.idx / a.cols;
+        const PeakOffsets d = peak_offsets(a.best, a.rows, a.cols, bi, a.idx - bi * a.cols);
+        a.offsets[0] = d.dx; a.offsets[1] = d.dy;
+    }
     const PeakStats ps = peak_statistics(a.best, a.rows, a.cols, a.idx, a.r, a.flags, a.gw, a.tmp_a, a.tmp_b, a.hes, bs);
     if (threadIdx.x == 0) { a.out[0] = ps.r; a.out[1] = ps.h; }
 }

@@ -19,7 +19,7 @@ from scipy import ndimage
 from scipy.spatial import cKDTree
 
 from . import _lib
-from ._lib import SID_TM_CCOEFF_NORMED, flags_from_kwargs
+from ._lib import SID_TM_CCOEFF_NORMED, flags_from_kwargs, flags_from_options
 from .lib import interpolation_poly, interpolation_near, _fill_gpi
 
 TM_CCOEFF_NORMED = SID_TM_CCOEFF_NORMED          # == cv2.TM_CCOEFF_NORMED
@@ -77,9 +77,16 @@ def rotate_and_match(img1, c1, r1, img_size, image2, alpha0,
 
     ``template_matcher`` left at None, set to :func:`match_template` or to
     ``cv2.matchTemplate`` selects the GPU matcher; any other callable is honoured
-    as the reference's plug-in and called once per angle."""
+    as the reference's plug-in and called once per angle.
+
+    ``subpixel=True`` (extension): ``dc`` / ``dr`` refined to sub-pixel precision by a parabola through the peak of
+    ``best_result`` and its two neighbours per axis (``SID_SUBPIXEL``, include/sid_b200.h); needs the built-in
+    matcher."""
     rot_order = kwargs.get('rot_order', 0)
-    flags = flags_from_kwargs(kwargs.get('hes_norm', True), kwargs.get('hes_smth', False), mcc_norm)
+    if kwargs.get('subpixel') and not _is_builtin_matcher(template_matcher):
+        raise ValueError("subpixel=True needs the built-in matcher (template_matcher None, match_template or "
+                         "cv2.matchTemplate)")
+    flags = flags_from_options(dict(kwargs, mcc_norm=mcc_norm))
     ctx = _ctx(kwargs)
     if _is_builtin_matcher(template_matcher):
         res = ctx.rotate_and_match(img1, c1, r1, img_size, image2, list(angles), alpha0, rot_order, flags, mtype)
@@ -117,19 +124,23 @@ def use_mcc_batch(c1, r1, c2fg, r2fg, border, img1, img2, img_size, alpha0, **kw
     ``return_maps=True`` (extension): return ``(table, maps, templates)`` where ``maps[i]`` is what
     ``rotate_and_match(...)[5]`` gives for point i's window -- the float32 NCC map of the winning angle -- or None
     where the row is NaN, and ``templates[i]`` (an (N, img_size, img_size) uint8 array) is ``[6]``, the winning
-    angle's template (zeros where the row is NaN)."""
+    angle's template (zeros where the row is NaN).
+
+    ``subpixel=True`` (extension): ``c2`` / ``r2`` refined to sub-pixel precision on the device by a parabola through
+    the peak of the winning map and its two neighbours per axis (``SID_SUBPIXEL``, include/sid_b200.h); the other
+    columns, the NaN rows and the maps of ``return_maps`` are unchanged.  Needs the built-in matcher."""
     matcher = kwargs.get('template_matcher')
     return_maps = kwargs.get('return_maps', False)
-    if return_maps and not _is_builtin_matcher(matcher):
-        raise ValueError("return_maps=True needs the built-in matcher (template_matcher None, match_template or "
-                         "cv2.matchTemplate)")
+    for option in ('return_maps', 'subpixel'):
+        if kwargs.get(option) and not _is_builtin_matcher(matcher):
+            raise ValueError("%s=True needs the built-in matcher (template_matcher None, match_template or "
+                             "cv2.matchTemplate)" % option)
     if not _is_builtin_matcher(matcher):
         rows = [use_mcc(a, b, c, d, e, img1, img2, img_size, alpha0, **kwargs)
                 for a, b, c, d, e in zip(c1, r1, c2fg, r2fg, border)]
         return np.array(rows, dtype=np.float64).reshape(-1, 5)
     ctx = _ctx(kwargs)
-    flags = flags_from_kwargs(kwargs.get('hes_norm', True), kwargs.get('hes_smth', False),
-                              kwargs.get('mcc_norm', False))
+    flags = flags_from_options(kwargs)
     args = (c1, r1, c2fg, r2fg, border, img_size, list(kwargs.get('angles', [-3, 0, 3])), alpha0,
             kwargs.get('rot_order', 0), flags, kwargs.get('mtype', TM_CCOEFF_NORMED))
     # The pair is uploaded on EVERY call (overlapped with the matching, so it costs ~1.5 ms per EW pair) unless
@@ -303,7 +314,9 @@ def pattern_matching(lon_pm1, lat_pm1, n1, c1, r1, n2, c2, r2,
     Returns ``(u, v, a, r, h, lon2_dst, lat2_dst)``, each shaped like ``lon_pm1``
     with NaN where no vector could be found.  ``threads`` is accepted for
     compatibility and ignored: all grid points go through one GPU launch (or one
-    launch per rank when ``torch.distributed`` is initialised, see sharding.py)."""
+    launch per rank when ``torch.distributed`` is initialised, see sharding.py).
+
+    ``subpixel=True`` (extension): sub-pixel drift vectors (see :func:`use_mcc_batch`)."""
     t0 = time.time()
     img1, img2 = n1[1], n2[1]
     dst_shape = lon_pm1.shape
@@ -338,7 +351,7 @@ def pattern_matching(lon_pm1, lat_pm1, n1, c1, r1, n2, c2, r2,
             and _is_builtin_matcher(kwargs.get('template_matcher'))):
         xy, ll = affine(srs)
         ctx = _ctx(kwargs)
-        flags = flags_from_kwargs(kwargs.get('hes_norm', True), kwargs.get('hes_smth', False), kwargs.get('mcc_norm', False))
+        flags = flags_from_options(kwargs)
         ctx.run_pair(img1, img2, c1pm1i[gpi], r1pm1i[gpi], c2fg[gpi], r2fg[gpi], brd2[gpi], img_size,
                      list(kwargs.get('angles', [-3, 0, 3])), alpha0, kwargs.get('rot_order', 0), flags,
                      kwargs.get('mtype', TM_CCOEFF_NORMED), keep_on_device=True)

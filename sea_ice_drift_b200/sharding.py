@@ -187,7 +187,7 @@ def use_mcc_batch_split(c1, r1, c2fg, r2fg, border, img1, img2, img_size, alpha0
             pts[k, :len(idx)] = np.asarray(arr, dtype=np.float64)[idx]
         d_pts = torch.from_numpy(pts).to(dev, non_blocking=True)
         table = torch.empty((world, n_max, 5), dtype=torch.float64, device=dev)
-        flags = _lib.flags_from_kwargs(kwargs.get('hes_norm', True), kwargs.get('hes_smth', False), kwargs.get('mcc_norm', False))
+        flags = _lib.flags_from_options(kwargs)
         ctx.run_device(n_max, *[d_pts[k].data_ptr() for k in range(5)], int(np.nanmax(border)), img_size,
                        list(kwargs.get('angles', [-3, 0, 3])), alpha0, table[rank].data_ptr(),
                        rot_order=kwargs.get('rot_order', 0), flags=flags, mtype=kwargs.get('mtype', _lib.SID_TM_CCOEFF_NORMED))
@@ -241,8 +241,7 @@ def use_mcc_series(pairs, img_size, alpha0=0.0, n_contexts=1, compute=None, gath
     if compute is None:
         from . import _lib
         # the reference's own defaults (pmlib.py:36, 118-121): hes_norm=True, hes_smth=False, mcc_norm=False
-        flags = _lib.flags_from_kwargs(kwargs.get('hes_norm', True), kwargs.get('hes_smth', False),
-                                       kwargs.get('mcc_norm', False))
+        flags = _lib.flags_from_options(kwargs)
         angles = kwargs.get('angles', [-3, 0, 3])
         rot_order = kwargs.get('rot_order', 0)
         mtype = kwargs.get('mtype', _lib.SID_TM_CCOEFF_NORMED)
