@@ -63,7 +63,7 @@ int sido_get_template(const uint8_t *img, int rows, int cols, int64_t pitch,
             double row = off0 + t0; row = row + t1;
             double col = off1 + t2; col = col + t3;
             uint8_t v = 0;
-            if (!(row < 0.0 || row > (double)(rows - 1) || col < 0.0 || col > (double)(cols - 1))) {
+            if (row >= 0.0 && row <= (double)(rows - 1) && col >= 0.0 && col <= (double)(cols - 1)) {   /* NaN: outside */
                 if (order == 0) {
                     int64_t ri = (int64_t)floor(row + 0.5), ci = (int64_t)floor(col + 0.5);
                     if (ri > rows - 1) ri = rows - 1;
@@ -381,6 +381,13 @@ int sido_use_mcc_batch(int64_t n, const double *c1, const double *r1,
     for (int64_t i = 0; i < n; ++i) {
         double *o = out + 5 * i;
         o[0] = o[1] = o[2] = o[3] = o[4] = NAN;
+        /* a non-finite input has no window and no template (the reference fails on it; the kernels reject it, as
+         * here): never sample image 1 at a NaN coordinate */
+        if (!isfinite(c1[i]) || !isfinite(r1[i]) || !isfinite(c2fg[i]) || !isfinite(r2fg[i]) || !isfinite(border[i]) ||
+            fabs(c2fg[i]) >= 1e9 || fabs(r2fg[i]) >= 1e9 || fabs(border[i]) >= 1e9) {
+            if (status) status[i] = -1;
+            continue;
+        }
         /* python int() truncates toward zero */
         int64_t y0 = (int64_t)(r2fg[i] - hws - border[i]);
         int64_t y1 = (int64_t)(r2fg[i] + hws + border[i] + 1);

@@ -372,6 +372,7 @@ int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1,
 #endif
         const size_t tsm = pm_tail_smem_bytes(a.max_rr, smth);
         if (int arc = allow_max_smem(ctx, (const void *)pm_tail_kernel)) return arc;
+        if (getenv("SID_DEBUG")) fprintf(stderr, "[sid] launch: tail threads=%d smem=%zu\n", pm_tail_threads(a.max_rr), tsm);
         pm_tail_kernel<<<(unsigned)n, pm_tail_threads(a.max_rr), tsm, st>>>(a);
         ctx->launches += 1;
         CU(cudaGetLastError());
@@ -412,6 +413,12 @@ int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1,
         if (smem > (size_t)ctx->max_smem_optin - 4096 - (smem_scratch ? 0 : 8192)) use_tc = false;      // window too large: legacy kernels
                                                                           // (the global-scratch variant has 8 KB more static shared memory)
     }
+    const void *ktab[8] = {(const void *)pm_points_kernel<9, false, false>, (const void *)pm_points_kernel<13, false, false>,
+                           (const void *)pm_points_kernel<0, false, false>, (const void *)pm_points_kernel<9, true, false>,
+                           (const void *)pm_points_kernel<13, true, false>, (const void *)pm_points_kernel<0, true, false>,
+                           (const void *)pm_points_kernel<0, false, true>, (const void *)pm_points_kernel<0, true, true>};
+    // the legacy kernel of this launch in ktab: mma.sync (imma) or a dp4a specialisation, per-point scratch in shared or global memory
+    auto legacy_kidx = [&](bool smem_scr) { return imma ? (smem_scr ? 7 : 6) : variant + (smem_scr ? 3 : 0); };
     if (!use_tc) {
     // window staging by TMA when the padded window (+15 bytes: the box must start 16-byte aligned) fits one
     // box of <= 256 x 256 bytes
@@ -452,10 +459,21 @@ int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1,
     }
     if (getenv("SID_PM_GLOBAL_SCRATCH")) smem_scratch = false;
     if (!smem_scratch) {
+        // the kernel's static shared memory (PmShared, the window barrier: 1920 B as cudaFuncGetAttributes reports it) comes
+        // out of the same per-block budget.  Without it a window that left less than that free was neither given fewer
+        // angles per batch nor refused here, and failed the occupancy check below with SID_ECUDA instead (measured on a
+        // B200: img_size 35, 3 angles, borders 206, 207, 209 and 210; img_size 128, 3 angles, borders 124 and 125)
+        cudaFuncAttributes fa;
+        CU(cudaFuncGetAttributes(&fa, ktab[legacy_kidx(false)]));
+        const size_t smem_max = (size_t)ctx->max_smem_optin - fa.sharedSizeBytes;
         smem = base_smem(a.ab);
-        while (smem > (size_t)ctx->max_smem_optin && a.ab > 1) { --a.ab; smem = base_smem(a.ab); }
-        if (smem > (size_t)ctx->max_smem_optin)
+        while (smem > smem_max && a.ab > 1) { --a.ab; smem = base_smem(a.ab); }
+        if (smem > smem_max) {
+            if (getenv("SID_DEBUG"))
+                fprintf(stderr, "[sid] refuse: legacy smem=%zu limit=%zu static=%zu optin=%d\n", smem, smem_max,
+                        (size_t)fa.sharedSizeBytes, ctx->max_smem_optin);
             return fail(ctx, SID_EUNSUPPORTED, "search window too large for the fused kernel (border too big)");
+        }
     }
     }
 
@@ -488,11 +506,7 @@ int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1,
         if (v >= 32 && v <= (imma ? PM_IMMA_THREADS : PM_THREADS) && v % 32 == 0) threads = v;
     }
 
-    const void *ktab[8] = {(const void *)pm_points_kernel<9, false, false>, (const void *)pm_points_kernel<13, false, false>,
-                           (const void *)pm_points_kernel<0, false, false>, (const void *)pm_points_kernel<9, true, false>,
-                           (const void *)pm_points_kernel<13, true, false>, (const void *)pm_points_kernel<0, true, false>,
-                           (const void *)pm_points_kernel<0, false, true>, (const void *)pm_points_kernel<0, true, true>};
-    const int kidx = use_tc ? (smem_scratch ? 9 : 8) : imma ? (smem_scratch ? 7 : 6) : variant + (smem_scratch ? 3 : 0);
+    const int kidx = use_tc ? (smem_scratch ? 9 : 8) : legacy_kidx(smem_scratch);
     const void *kfn = use_tc ? (smem_scratch ? (const void *)pm_tc_kernel<true> : (const void *)pm_tc_kernel<false>) : ktab[kidx];
     if (int arc = allow_max_smem(ctx, kfn)) return arc;
     int occ = 0;
@@ -504,8 +518,8 @@ int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1,
         return fail(ctx, SID_ECUDA, msg);
     }
     if (getenv("SID_DEBUG"))
-        fprintf(stderr, "[sid] launch: tc=%d kidx=%d threads=%d smem=%zu occ(api)=%d tmem_cols=%d nab=%d ks=%d nacc=%d nb8=%d slotc=%d nslot=%d n16max=%d wrows=%d npanels=%d mma_sums=%d\n",
-                (int)use_tc, kidx, threads, smem, occ, tg.tmem_cols, tg.nab, tg.ks, tg.nacc, tg.nb8, tg.slotc, tg.nslot, tg.n16max, tg.wrows, tg.npanels, tg.mma_sums);
+        fprintf(stderr, "[sid] launch: tc=%d kidx=%d threads=%d smem=%zu occ(api)=%d tmem_cols=%d nab=%d ks=%d nacc=%d nb8=%d slotc=%d nslot=%d n16max=%d wrows=%d npanels=%d mma_sums=%d tma=%d nc=%d\n",
+                (int)use_tc, kidx, threads, smem, occ, tg.tmem_cols, tg.nab, tg.ks, tg.nacc, tg.nb8, tg.slotc, tg.nslot, tg.n16max, tg.wrows, tg.npanels, tg.mma_sums, a.tma, a.nc);
     if (use_tc) {
         // The occupancy API answers 1 for a kernel that executes tcgen05.alloc with a run-time column count (it has to
         // assume all 512 columns); residency is really bounded by registers, shared memory and the columns we ask for.
@@ -559,6 +573,7 @@ int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1,
     if (split_tail) {
         const size_t tsm = pm_tail_smem_bytes(a.max_rr, smth);
         if (int arc = allow_max_smem(ctx, (const void *)pm_tail_kernel)) return arc;
+        if (getenv("SID_DEBUG")) fprintf(stderr, "[sid] launch: tail threads=%d smem=%zu\n", pm_tail_threads(a.max_rr), tsm);
         pm_tail_kernel<<<(unsigned)n, pm_tail_threads(a.max_rr), tsm, st>>>(a);
         ctx->launches += 1;
         CU(cudaGetLastError());
