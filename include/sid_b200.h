@@ -133,6 +133,19 @@ int sid_pm_epilogue_affine(sid_ctx *ctx, int64_t n_valid, const int32_t *grid_in
  * pair, before the all-gather that completes the adopted buffers). */
 int sid_upload_rows(sid_ctx *ctx, uint8_t *d_dst, int64_t dst_pitch, const uint8_t *src, int64_t src_pitch, int cols, int rows);
 
+/* k x k box downsampling of the RESIDENT pair (k = factor in [2, 16]) into caller-owned device buffers laid out by
+ * sid_pair_layout(rows / k, cols / k) of each image (floor: trailing rows and columns are dropped).  Output pixel
+ * (i, j) is 0 if any of the k * k source pixels (rows k*i ... k*i+k-1, columns k*j ... k*j+k-1) is 0 (invalid, as
+ * everywhere in this library), else floor(mean + 0.5) computed exactly in integers, (2 * sum + k*k) / (2 * k*k).  Only
+ * the rows * cols bytes of each image are written, never the pitch padding.  The buffers can then be adopted as the
+ * pair of another context (sid_adopt_pair_device) to match on the coarse pair (pmlib.coarse_tracking).  Checked on the
+ * host before any launch: SID_ENOPAIR without a resident pair; SID_EINVAL for a factor outside [2, 16], a downsampled
+ * image smaller than 1 x 1, or a buffer whose pitch or size is below sid_pair_layout's (or a pitch not a multiple of
+ * 16); the context stays usable.  One launch (sid::downsample_kernel), asynchronous on the context's stream. */
+int sid_downsample_pair(sid_ctx *ctx, int factor,
+                        uint8_t *d_img1, int64_t pitch1, int64_t bytes1,
+                        uint8_t *d_img2, int64_t pitch2, int64_t bytes2);
+
 /* use_mcc for n grid points (host arrays in, host array out, synchronous).
  *   c1, r1        float pixel coordinates on image 1
  *   c2fg, r2fg    integer-valued first guess on image 2

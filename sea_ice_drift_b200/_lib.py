@@ -20,12 +20,13 @@ _i32p = C.POINTER(C.c_int)
 SID_TM_CCOEFF_NORMED = 5
 SID_HES_NORM, SID_HES_SMTH, SID_MCC_NORM = 1, 2, 4
 SID_SUBPIXEL = 8                # extension: sub-pixel c2 / r2 (include/sid_b200.h)
+SID_PT_VALID = 1                # point status of a valid row (sid_run*)
 
 EXPORTS = [
     "sid_version", "sid_create", "sid_destroy", "sid_last_error", "sid_set_stream", "sid_synchronize",
     "sid_set_pair", "sid_set_pair_device", "sid_pair_layout", "sid_adopt_pair_device", "sid_upload_rows", "sid_pm_epilogue_affine", "sid_first_guess", "sid_run", "sid_run_pair", "sid_run_device", "sid_map_layout", "sid_run_maps", "sid_launch_count", "sid_last_kernel_ms", "sid_last_kernel_name",
     "sid_rotate_and_match", "sid_get_template", "sid_match_template", "sid_get_hessian", "sid_knn_hamming2",
-    "sid_deformation",
+    "sid_deformation", "sid_downsample_pair",
 ]
 
 _lib = None
@@ -71,6 +72,8 @@ def load_library():
         lib.sid_pm_epilogue_affine.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64] + [C.c_void_p] * 6
         lib.sid_first_guess.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 4 + [C.c_int] + [C.c_void_p] * 2 + \
             [C.c_int64] + [C.c_void_p] * 6
+        lib.sid_downsample_pair.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_int64,
+                                            C.c_void_p, C.c_int64, C.c_int64]
         lib.sid_upload_rows.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_int]
         lib.sid_run.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 5 + \
             [C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_uint, C.c_int, C.c_void_p, C.c_void_p]
@@ -223,6 +226,15 @@ class Context(object):
             self._h, C.c_void_p(ptr1), shape1[0], shape1[1], pitch1, bytes1,
             C.c_void_p(ptr2), shape2[0], shape2[1], pitch2, bytes2))
         self._pair_key = None
+        return self
+
+    def downsample_pair(self, factor, buf1, buf2):
+        """k x k box downsampling (k = ``factor``) of the resident pair into caller-owned device buffers
+        (sid_downsample_pair), asynchronous on the context's stream.  ``buf1`` / ``buf2`` are ``(device pointer, pitch,
+        bytes)`` in the layout of ``pair_layout(rows // factor, cols // factor)`` of image 1 / 2."""
+        (p1, pitch1, bytes1), (p2, pitch2, bytes2) = buf1, buf2
+        self._check(self._lib.sid_downsample_pair(self._h, int(factor), C.c_void_p(int(p1)), int(pitch1), int(bytes1),
+                                                  C.c_void_p(int(p2)), int(pitch2), int(bytes2)))
         return self
 
     def pm_epilogue_affine(self, gpi, c2pm1, r2pm1, xy, ll, results=None):

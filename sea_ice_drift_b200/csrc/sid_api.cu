@@ -25,6 +25,7 @@
 #include "sid_knn_kernel.cuh"
 #include "sid_defor_kernel.cuh"
 #include "sid_fg_kernel.cuh"
+#include "sid_downsample_kernel.cuh"
 
 using namespace sid;
 
@@ -723,6 +724,34 @@ int sid_upload_rows(sid_ctx *ctx, uint8_t *d_dst, int64_t dst_pitch, const uint8
     if (!d_dst || !src || cols <= 0 || rows < 0 || dst_pitch < cols || src_pitch < cols) return fail(ctx, SID_EINVAL, "bad arguments");
     CU(cudaSetDevice(ctx->device));
     CU(cudaMemcpy2DAsync(d_dst, (size_t)dst_pitch, src, (size_t)src_pitch, (size_t)cols, (size_t)rows, cudaMemcpyHostToDevice, ctx->stream));
+    return SID_OK;
+}
+
+int sid_downsample_pair(sid_ctx *ctx, int factor, uint8_t *d_img1, int64_t pitch1, int64_t bytes1,
+                        uint8_t *d_img2, int64_t pitch2, int64_t bytes2) {
+    if (!ctx) return SID_EINVAL;
+    if (!ctx->have_pair) return fail(ctx, SID_ENOPAIR, "no image pair is resident");
+    if (factor < 2 || factor > 16) return fail(ctx, SID_EINVAL, "downsampling factor must be in [2, 16]");
+    const int r1 = ctx->rows1 / factor, c1 = ctx->cols1 / factor, r2 = ctx->rows2 / factor, c2 = ctx->cols2 / factor;
+    if (r1 < 1 || c1 < 1 || r2 < 1 || c2 < 1) return fail(ctx, SID_EINVAL, "downsampled image smaller than 1 x 1");
+    if (!d_img1 || !d_img2 || pitch1 < padded_pitch(c1) || pitch2 < padded_pitch(c2) || (pitch1 & 15) || (pitch2 & 15) ||
+        bytes1 < pitch1 * (int64_t)r1 + (int64_t)IMG_TAIL_SLACK || bytes2 < pitch2 * (int64_t)r2 + (int64_t)IMG_TAIL_SLACK)
+        return fail(ctx, SID_EINVAL, "output buffers need the layout of sid_pair_layout(rows / factor, cols / factor)");
+    CU(cudaSetDevice(ctx->device));
+    const DsImage im1{(const uint8_t *)ctx->img1.p, ctx->pitch1, d_img1, (long long)pitch1, r1, c1};
+    const DsImage im2{(const uint8_t *)ctx->img2.p, ctx->pitch2, d_img2, (long long)pitch2, r2, c2};
+    const int tile = ds_tile_out(factor), rows = ds_rows(factor);
+    const dim3 grid((unsigned)((std::max(r1, r2) + rows - 1) / rows), (unsigned)((std::max(c1, c2) + tile - 1) / tile), 2);
+    if (grid.y > 65535u) return fail(ctx, SID_EINVAL, "image too wide for sid_downsample_pair");
+    switch (factor) {       // one instantiation per factor: the loads and the division by 2 k^2 are unrolled / constant
+#define SID_DS_CASE(K) case K: downsample_kernel<K><<<grid, DS_THREADS, 0, ctx->stream>>>(im1, im2); break;
+        SID_DS_CASE(2) SID_DS_CASE(3) SID_DS_CASE(4) SID_DS_CASE(5) SID_DS_CASE(6) SID_DS_CASE(7) SID_DS_CASE(8)
+        SID_DS_CASE(9) SID_DS_CASE(10) SID_DS_CASE(11) SID_DS_CASE(12) SID_DS_CASE(13) SID_DS_CASE(14) SID_DS_CASE(15)
+        SID_DS_CASE(16)
+#undef SID_DS_CASE
+    }
+    ctx->launches += 1;
+    CU(cudaGetLastError());
     return SID_OK;
 }
 

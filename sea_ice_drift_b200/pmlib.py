@@ -12,6 +12,7 @@ the Nansat objects, the first-guess interpolation and the final re-gridding.
 """
 from __future__ import absolute_import, print_function
 
+import os
 import time
 
 import numpy as np
@@ -297,6 +298,159 @@ def prepare_first_guess(c2pm1, r2pm1, n1, c1, r1, n2, c2, r2, img_size,
     c2fg[outside_hull] = c2p2[outside_hull]
     r2fg[np.isnan(r2fg)] = r2p2[np.isnan(r2fg)]
     return c2fg, r2fg, border
+
+
+COARSE_DEFAULTS = dict(factor=4, step=32, img_size=35, max_drift=100.0, min_quality=4.0, angles=[-3, 0, 3], seed=0)
+
+
+def _incircle_zero(ax, ay, bx, by, cx, cy, dx, dy):
+    """True where d lies exactly on the circle through a, b, c (int64 coordinates, exact)."""
+    ax, ay, bx, by, cx, cy = ax - dx, ay - dy, bx - dx, by - dy, cx - dx, cy - dy
+    a2, b2, c2 = ax * ax + ay * ay, bx * bx + by * by, cx * cx + cy * cy
+    return ax * (by * c2 - b2 * cy) - ay * (bx * c2 - b2 * cx) + a2 * (bx * cy - by * cx) == 0
+
+
+def coarse_lattice(shape1, step, seed):
+    """Integer lattice ``step`` apart on a coarse image of ``shape1`` (rows, cols), every point moved by a seeded integer
+    jitter of at most ``step // 4`` per axis.  Returns int64 (c1, r1) in row-major lattice order.
+
+    On an exact lattice every Delaunay cell of the points is cocircular, so the triangulation that
+    :func:`prepare_first_guess` interpolates over is not unique and its ``'auto'`` mode takes the Qhull path.  With the
+    jitter, a cell can still be cocircular by chance (about one cell in 600 at ``step`` 16); the jitter of such a cell's
+    first corner is drawn again until no lattice cell is.  That is all the redraw guarantees: four points of different
+    cells (a sliver along the hull, a diamond across three rows) can still be cocircular -- none at ``step`` 16 and 32,
+    a few at ``step`` 8 in DESIGN.md section 8 -- and ``'auto'`` then takes the Qhull path, with the same result."""
+    if step < 4:
+        raise ValueError("step must be at least 4 coarse pixels")
+    rng = np.random.default_rng(seed)
+    amp = step // 4
+    xs = np.arange(step // 2, shape1[1], step, dtype=np.int64)
+    ys = np.arange(step // 2, shape1[0], step, dtype=np.int64)
+    gx, gy = np.meshgrid(xs, ys)
+    jx = rng.integers(-amp, amp + 1, gx.shape)
+    jy = rng.integers(-amp, amp + 1, gx.shape)
+    for _ in range(64):
+        c, r = gx + jx, gy + jy
+        bad = _incircle_zero(c[:-1, :-1], r[:-1, :-1], c[:-1, 1:], r[:-1, 1:], c[1:, 1:], r[1:, 1:], c[1:, :-1], r[1:, :-1])
+        if not bad.any():
+            break
+        iy, ix = np.nonzero(bad)
+        jx[iy, ix] = rng.integers(-amp, amp + 1, iy.size)
+        jy[iy, ix] = rng.integers(-amp, amp + 1, iy.size)
+    return (gx + jx).ravel(), (gy + jy).ravel()
+
+
+def coarse_inputs(n1, n2, shape1, shape2, factor, step, img_size, max_drift, seed=0):
+    """The coarse matching problem of :func:`coarse_tracking` on coarse images of ``shape1`` / ``shape2``: the lattice
+    points that pattern_matching's window rule keeps (in coarse pixels), their zero-drift first guess on coarse image 2
+    from the geolocation of ``n1`` / ``n2``, the coarse border and the initial rotation.  Returns
+    ``(c1, r1, c2fg, r2fg, border, alpha0)``; c1 ... border are float64 arrays, the border is
+    ``ceil(max_drift / factor) + 2`` everywhere."""
+    k = int(factor)
+    c1, r1 = coarse_lattice(shape1, step, seed)
+    c1, r1 = c1.astype(np.float64), r1.astype(np.float64)
+    off = (k - 1) / 2.
+    lon, lat = n1.transform_points(k * c1 + off, k * r1 + off)
+    x2, y2 = n2.transform_points(lon, lat, 1)
+    c2fg, r2fg = np.round((np.asarray(x2) - off) / k), np.round((np.asarray(y2) - off) / k)
+    border = float(np.ceil(max_drift / k) + 2)
+    hws = round(img_size / 2) + 1
+    hws_hypot = np.hypot(hws, hws)
+    with np.errstate(invalid='ignore'):
+        gpi = ((c2fg - border - hws > 0) & (r2fg - border - hws > 0) &
+               (c2fg + border + hws < shape2[1]) & (r2fg + border + hws < shape2[0]) &
+               (c1 - hws_hypot > 0) & (r1 - hws_hypot > 0) & (c1 + hws_hypot < shape1[1]) & (r1 + hws_hypot < shape1[0]))
+    return c1[gpi], r1[gpi], c2fg[gpi], r2fg[gpi], np.full(int(gpi.sum()), border), get_initial_rotation(n1, n2)
+
+
+def coarse_matches(table, status, c1, r1, factor, img_size, min_quality):
+    """Full-resolution matches ``(x1, y1, x2, y2)`` from the coarse table: rows with status valid, finite values and
+    ``r * h > min_quality``.  Template pixel ``int(s / 2) + 1`` samples coarse image 1 at (c1, r1) and lies at
+    ``c2 + 1`` in coarse image 2 for odd ``img_size`` s and at ``c2 + 1.5`` for even s; a coarse pixel j covers the
+    full-resolution pixels ``k * j ... k * j + k - 1``, centred on ``k * j + (k - 1) / 2``."""
+    k = int(factor)
+    table = np.asarray(table, dtype=np.float64).reshape(-1, 5)
+    with np.errstate(invalid='ignore'):
+        keep = (np.asarray(status) == _lib.SID_PT_VALID) & np.isfinite(table).all(axis=1) & \
+            (table[:, 3] * table[:, 4] > min_quality)
+    off = (k - 1) / 2.
+    delta = 1.0 if int(img_size) % 2 else 1.5
+    return (k * c1[keep] + off, k * r1[keep] + off,
+            k * (table[keep, 0] + delta) + off, k * (table[keep, 1] + delta) + off)
+
+
+_coarse_buffers = {}
+
+
+def _coarse_buffer(device, which, layout, nbytes):
+    """Device buffer of coarse image ``which`` (torch uint8, 256-byte aligned by the allocator): one per device and image,
+    grown when a call needs more bytes, so a process that sees many scene sizes keeps only the largest.  Zeroed when
+    ``layout`` (the coarse shape and factor) differs from its previous use, so the pitch padding is 0 as after an
+    upload.  The fill is queued on torch's current stream: the caller orders it before the context's work."""
+    import torch
+    buf, last = _coarse_buffers.get((device, which), (None, None))
+    if buf is None or buf.numel() < nbytes:
+        buf = torch.zeros(nbytes, dtype=torch.uint8, device=torch.device('cuda', device))
+    elif last != layout:
+        buf.zero_()
+    _coarse_buffers[(device, which)] = (buf, layout)
+    return buf
+
+
+_coarse_contexts = {}
+
+
+def coarse_tracking(n1, n2, **kwargs):
+    """Feature-tracking matches without feature tracking: ``(x1, y1, x2, y2)``, full-resolution pixel coordinates on
+    image 1 and image 2, what the reference's ``ftlib.feature_tracking`` returns, so they can go wherever its matches
+    go (``prepare_first_guess``, ``pattern_matching``, ``SeaIceDrift.get_drift_PM``).
+
+    The pair is made resident on the device and box-downsampled there by ``factor`` (``sid_downsample_pair``); a
+    private context adopts the coarse pair and matches a jittered lattice ``step`` coarse pixels apart
+    (:func:`coarse_lattice`) from the zero-drift first guess of the geolocation, border ``ceil(max_drift / factor) +
+    2``, templates of ``img_size`` coarse pixels, ``angles`` around the initial rotation, default flags.  Matches with
+    ``r * h > min_quality`` are mapped back to full resolution (:func:`coarse_matches`), in lattice order; their error
+    is about ``factor / 2`` px.  No image leaves the device.  Keywords and defaults: ``factor`` 4 (2 ... 16), ``step``
+    32 (the fastest whole drift call of steps 8 ... 32 on an EW-sized pair, DESIGN.md section 8), ``img_size`` 35, ``max_drift`` 100 (full-resolution px), ``min_quality`` 4.0, ``angles`` [-3, 0, 3], ``seed``
+    0 (the lattice jitter), ``device``."""
+    opts = dict(COARSE_DEFAULTS)
+    opts.update((key, kwargs[key]) for key in COARSE_DEFAULTS if key in kwargs)
+    k, s = int(opts['factor']), int(opts['img_size'])
+    if not 2 <= k <= 16 or k != opts['factor']:
+        raise ValueError("factor must be an integer in [2, 16]")
+    if not 2 <= s <= 128:
+        raise ValueError("img_size must be in [2, 128]")
+    img1, img2 = _lib.as_u8_image(n1[1]), _lib.as_u8_image(n2[1])
+    shape1 = (img1.shape[0] // k, img1.shape[1] // k)
+    shape2 = (img2.shape[0] // k, img2.shape[1] // k)
+    if min(shape1 + shape2) < s:
+        raise ValueError("a %d x downsampled image (%s, %s) is smaller than one %d x %d template"
+                         % (k, shape1, shape2, s, s))
+    c1, r1, c2fg, r2fg, border, alpha0 = coarse_inputs(n1, n2, shape1, shape2, k, int(opts['step']), s,
+                                                       float(opts['max_drift']), opts['seed'])
+    if c1.size == 0:
+        return tuple(np.zeros(0) for _ in range(4))
+    import torch
+    ctx = _ctx(kwargs)
+    ctx.set_pair(img1, img2)
+    bufs = []
+    for which, shape in enumerate((shape1, shape2)):
+        pitch, nbytes = _lib.pair_layout(*shape)
+        buf = _coarse_buffer(ctx.device, which, (shape, k), nbytes)
+        bufs.append((buf.data_ptr(), pitch, buf.numel()))
+    # the buffers' zero fill runs on torch's current stream, the downsampling on the context's own (non-blocking) stream
+    torch.cuda.current_stream(ctx.device).synchronize()
+    ctx.downsample_pair(k, bufs[0], bufs[1])
+    ctx.synchronize()                        # the private context's stream reads what the default one wrote
+    key = (os.getpid(), ctx.device)
+    coarse = _coarse_contexts.get(key)
+    if coarse is None:
+        coarse = _coarse_contexts[key] = _lib.Context(ctx.device)
+    (p1, pitch1, b1), (p2, pitch2, b2) = bufs
+    coarse.adopt_pair_device(p1, shape1, pitch1, b1, p2, shape2, pitch2, b2)
+    table, status = coarse.run(c1, r1, c2fg, r2fg, border, s, list(opts['angles']), alpha0, 0, _lib.SID_HES_NORM,
+                               want_status=True)
+    return coarse_matches(table, status, c1, r1, k, s, float(opts['min_quality']))
 
 
 def _nsr(srs):

@@ -1,8 +1,9 @@
 """``SeaIceDrift`` façade with the reference's interface (reference
 sea_ice_drift/seaicedrift.py:23-88).  Pattern matching runs on the GPU; opening
 Sentinel-1 files (Nansat/GDAL) and ORB feature tracking stay on the reference
-path and are delegated to the ``sea_ice_drift`` package when it is installed."""
-from .pmlib import pattern_matching
+path and are delegated to the ``sea_ice_drift`` package when it is installed;
+``get_drift_coarse`` gives first-guess matches without it, on the GPU."""
+from .pmlib import coarse_tracking, pattern_matching
 
 
 class SeaIceDrift(object):
@@ -31,6 +32,15 @@ class SeaIceDrift(object):
                               "stays on the reference path)") from e
         x1, y1, x2, y2 = feature_tracking(self.n1, self.n2, **kwargs)
         return get_drift_vectors(self.n1, x1, y1, self.n2, x2, y2, **kwargs)
+
+    def get_drift_coarse(self, **kwargs):
+        """Extension: the contract of get_drift_FT, ``(lon1, lat1, lon2, lat2)`` of matches on image 1 and image 2, from
+        pattern matching on a box-downsampled copy of the pair (:func:`pmlib.coarse_tracking`, keywords there) instead
+        of ORB feature tracking, so it needs neither the reference package nor host image processing."""
+        x1, y1, x2, y2 = coarse_tracking(self.n1, self.n2, **kwargs)
+        lon1, lat1 = self.n1.transform_points(x1, y1)
+        lon2, lat2 = self.n2.transform_points(x2, y2)
+        return lon1, lat1, lon2, lat2
 
     def get_drift_PM(self, lons, lats, lon1, lat1, lon2, lat2, **kwargs):
         """Same contract as the reference's get_drift_PM (seaicedrift.py:62-88):
