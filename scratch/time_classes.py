@@ -44,10 +44,6 @@ print("same table:", np.array_equal(a, bres, equal_nan=True))
 for cut in (28, 32, 36, 40):
     timed([np.nonzero(brd <= 20)[0], np.nonzero((brd > 20) & (brd <= cut))[0], np.nonzero(brd > cut)[0]], "three hand-made classes: <=20 | <=%d | rest" % cut, {"SID_PM_CLASSES": "0"})
 timed([np.nonzero(brd <= 20)[0], np.nonzero((brd > 20) & (brd <= 28))[0], np.nonzero((brd > 28) & (brd <= 38))[0], np.nonzero(brd > 38)[0]], "four hand-made classes: <=20 | <=28 | <=38 | rest", {"SID_PM_CLASSES": "0"})
-for kb in (64, 100):
-    r = timed([allp], "two classes, split tail up to %d KB of tail shared memory" % kb, {"SID_PM_TAIL_SMEM_KB": str(kb)})
-    print("same table:", np.array_equal(a, r, equal_nan=True))
-timed([np.nonzero(brd <= 20)[0], np.nonzero((brd > 20) & (brd <= 36))[0], np.nonzero(brd > 36)[0]], "three hand-made classes <=20 | <=36 | rest, split tail up to 100 KB", {"SID_PM_CLASSES": "0", "SID_PM_TAIL_SMEM_KB": "100"})
 for path in ("imma",):
     timed([np.nonzero(brd <= 20)[0]], "the <= 20 class alone", {"SID_PM_CLASSES": "0"})
     timed([np.nonzero(brd > 20)[0]], "the > 20 class alone", {"SID_PM_CLASSES": "0"})

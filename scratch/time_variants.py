@@ -21,7 +21,7 @@ flops = (len(angles) * 2.0 * s * s * (2 * b + 1 + (s % 2 == 0)) ** 2).sum()
 ref = None
 def run(label, env, reps=5):
     global ref
-    for k in ("SID_PM_THREADS", "SID_PM_GLOBAL_SCRATCH", "SID_PM_PATH", "SID_PM_TMA", "SID_PM_SPLIT_TAIL"): os.environ.pop(k, None)
+    for k in ("SID_PM_GLOBAL_SCRATCH", "SID_PM_PATH", "SID_PM_TMA", "SID_PM_SPLIT_TAIL"): os.environ.pop(k, None)
     os.environ.update(env)
     with torch.cuda.stream(stream):
         for _ in range(2): ctx.run_device(n, *ptrs, int(b.max()), s, angles, 0.0, d_out.data_ptr(), d_st.data_ptr())

@@ -30,9 +30,6 @@
 using namespace sid;
 
 namespace {
-#ifndef SID_WS_DEFAULT
-#define SID_WS_DEFAULT 1
-#endif
 
 constexpr size_t IMG_TAIL_SLACK = 4096;   // bytes readable past the last image row
 
@@ -112,19 +109,13 @@ struct sid_ctx {
     // per-call buffers
     DevBuf pts, order, out, status, angles, scratch, counter, misc, tail_maps, tail_recs, epi, fg;
     DevBuf maps, map_off, tpl;               // sid_run_maps: packed maps, their offsets, the templates
-    float *maps_out = nullptr;               // set for the duration of a sid_run_maps call (PmArgs::maps_out etc.)
-    const long long *map_off_dev = nullptr;
-    uint8_t *tpl_out = nullptr;
     void *pin = nullptr;
     size_t pin_cap = 0;
     cudaEvent_t k_ev[2] = {};                // bracket the last fused-kernel launch (sid_last_kernel_ms)
     bool k_ev_valid = false;
     const char *k_name = "";
-    bool k_ev_hold = false;                  // second launch of a two-class call: keep the start event of the first
     HostPool *pool = nullptr;                // staged upload of pageable images
-    size_t tail_region_stride = 0;           // floats per point of the tail-map regions of the current host call (0: the launch's own)
     long long table_n = -1;                  // rows of the result table the last sid_run / sid_run_pair left in `out`
-    long long tail_hint_n = 0;               // total points of the current host call (sizes the tail hand-off once)
     // staged upload of pageable host images (sid_run_pair): pinned double buffer + "slot free again" events
     void *stage = nullptr;
     size_t stage_cap = 0;
@@ -242,150 +233,107 @@ bool make_window_tensor_map(sid_ctx *ctx, CUtensorMap *map, int box_w, int box_h
     return r == CUDA_SUCCESS;
 }
 
-// shared launch path of sid_run / sid_run_device
-// Largest shared-memory footprint of pm_tail_kernel for which the tail is split off the correlation kernel
-// (SID_PM_TAIL_SMEM_KB overrides; 52 KB = at least 4 tail CTAs per SM)
-size_t tail_split_limit() {
-    if (const char *e = getenv("SID_PM_TAIL_SMEM_KB")) { const int kb = atoi(e); if (kb > 0) return (size_t)kb * 1024; }
-    return (size_t)52 * 1024;
+// ------------------------------------------------------------------ matching launches: plan, reserve, enqueue
+// Largest shared-memory footprint of pm_tail_kernel for which the tail is split off the correlation kernel: at least 4 tail
+// CTAs per SM; larger maps measured faster with the fused tail (cfg1: 1.10 vs 1.21 ms)
+constexpr size_t TAIL_SPLIT_SMEM = 52 * 1024;
+
+bool split_tail_fits(int max_rr, bool smth) {
+    if (const char *e = getenv("SID_PM_SPLIT_TAIL")) if (e[0] == '0') return false;
+    return pm_tail_smem_bytes(max_rr, smth) <= TAIL_SPLIT_SMEM;
 }
 
-// Words per work item of the tail hand-off regions of a two-class host call: the large class hands over float maps (when its
-// tail is split off), the small class is the one of pm_ws_kernel (three integer arrays per item)
-size_t tail_region_words(int rr_big, int rr_small, bool smth) {
-    const size_t big = pm_tail_smem_bytes(rr_big, smth) <= tail_split_limit() ? tail_item_words((rr_big + 3) & ~3, 0) : 0;
-    return std::max(big, tail_item_words((rr_small + 3) & ~3, 1));
+// SID_PM_PATH: unset = pm_ws_kernel where it fits, else pm_tc_kernel where two CTAs per SM fit, else mma.sync; "ws", "tc"
+// and "imma" force one of them where it fits (mma.sync otherwise), "dp4a" the integer-pipe kernel
+bool ws_wanted() {
+    const char *e = getenv("SID_PM_PATH");
+    return !e || strcmp(e, "ws") == 0;
 }
 
-int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1, const double *d_c2fg,
-              const double *d_r2fg, const double *d_border, const int *d_order, int max_border, int typ_border,
-              int img_size, int n_angles, const double *d_angles, const double *d_tab, int rot_order,
-              unsigned flags, double *d_out, int *d_status,
-              cudaStream_t st = nullptr, int slot = 0, long long tail_off = 0) {
-    if (!st) st = ctx->stream;
-    const int s = img_size;
+// pm_ws_kernel's shared-memory layout for borders up to `border` (typical map width rtyp, nstat sets of window statistics)
+// fits one CTA with `headroom` bytes to spare: the one rule the planner and ws_border_limit share
+bool ws_fits(const sid_ctx *ctx, int s, int border, int n_angles, int rtyp, int nstat, PmWsCfg &g, size_t headroom = 0) {
+    const int Wmax = 2 * (s / 2) + 2 * border + 1, Rmax = Wmax - s + 1;
+    return pm_ws_geometry(s, Rmax, Wmax, n_angles, Rmax * Rmax, g, rtyp, nstat) &&
+           (size_t)g.smem_bytes + 2048 + headroom <= (size_t)ctx->max_smem_optin;
+}
+
+enum PmKernel { PM_WS, PM_TC, PM_POINTS };
+
+// Everything a matching launch needs that does not depend on which points it takes: the kernel and its variant, its
+// configuration and tensor maps, the geometry fields of PmArgs, the CTA shape and that of the split tail
+struct PmPlan {
+    PmKernel kernel;
+    const void *kfn;
+    const char *name;                // sid_last_kernel_name
+    int kidx;                        // PM_TC / PM_POINTS: 8 + smem_scratch, or the index in the pm_points_kernel table
+    bool smem_scratch;               // PM_TC / PM_POINTS: per-point scratch in shared memory (else a global slab per CTA)
+    PmWsCfg wg;
+    PmTcCfg tg;
+    alignas(64) CUtensorMap tmap;    // image 2: the search windows
+    alignas(64) CUtensorMap tmap1;   // image 1 (PM_WS): the patch the templates of a point are sampled from
+    PmArgs args;                     // geometry only; the launch sets the pointers and the point count
+    size_t smem;
+    int threads, occ, occ_api;       // occ_api: what the occupancy API answered (SID_DEBUG)
+    int tail_threads;
+    size_t tail_smem;
+};
+
+// Kernel, variant and shape of a launch over points with borders up to max_border (typ_border: the typical point, which
+// sizes the CTA and pads pm_ws_kernel's layout).  Host queries only: nothing is allocated or enqueued.
+int plan_pm(sid_ctx *ctx, int s, int n_angles, unsigned flags, int max_border, int typ_border, PmPlan &p) {
+    p = PmPlan{};
     const int hws = s / 2;
     const int Wmax = 2 * hws + 2 * max_border + 1;
     const int Rmax = Wmax - s + 1;
     if (Rmax < 2) return fail(ctx, SID_EINVAL, "search window not larger than the template");
-    PmArgs a;
-    memset(&a, 0, sizeof a);
-    a.img1 = (const uint8_t *)ctx->img1.p; a.rows1 = ctx->rows1; a.cols1 = ctx->cols1; a.pitch1 = ctx->pitch1;
-    a.img2 = (const uint8_t *)ctx->img2.p; a.rows2 = ctx->rows2; a.cols2 = ctx->cols2; a.pitch2 = ctx->pitch2;
-    a.n = n;
-    a.c1 = d_c1; a.r1 = d_r1; a.c2fg = d_c2fg; a.r2fg = d_r2fg; a.border = d_border; a.order = d_order;
-    a.s = s; a.n_angles = n_angles; a.angles = d_angles; a.tab = d_tab;
-    a.rot_order = rot_order; a.flags = flags;
+    PmArgs &a = p.args;
+    a.s = s; a.n_angles = n_angles; a.flags = flags;
     const double area = (double)s * (double)s;
     a.inv_area = 1.0 / area;
     a.sqrt_inv_area = std::sqrt(a.inv_area);
     gaussian_weights(a.gw);
-    a.out = d_out; a.status = d_status;
-    a.maps_out = ctx->maps_out; a.map_off = ctx->map_off_dev; a.tpl_out = ctx->tpl_out;
     a.max_rr = Rmax * Rmax;
     a.max_hrw = Wmax * Rmax;
     // correlation path: tcgen05 tensor cores (default), legacy mma.sync (SID_PM_PATH=imma) or the integer pipe
     // (SID_PM_PATH=dp4a); all three give bit-identical results
     const char *path_env = getenv("SID_PM_PATH");
     const bool want_tc = !path_env || strcmp(path_env, "tc") == 0;
-    const bool want_ws = path_env ? strcmp(path_env, "ws") == 0 : SID_WS_DEFAULT != 0;
     const bool imma = !(path_env && strcmp(path_env, "dp4a") == 0);
     const bool smth = (flags & SID_HES_SMTH) != 0;
+    const bool global_scratch = getenv("SID_PM_GLOBAL_SCRATCH") != nullptr;
     // Split tail: peak statistics in a second, light kernel when the result map fits its shared memory
-    bool split_tail = pm_tail_smem_bytes(a.max_rr, smth) <= tail_split_limit();       // >= 4 tail CTAs per SM; larger maps measured
-                                                                             // faster with the fused tail (cfg1: 1.10 vs 1.21 ms)
-    if (const char *e = getenv("SID_PM_SPLIT_TAIL")) if (e[0] == '0') split_tail = false;
-    alignas(64) CUtensorMap tmap;
-    memset(&tmap, 0, sizeof tmap);
-    PmTcCfg tg;
-    memset(&tg, 0, sizeof tg);
-    bool use_tc = false;
-    // warp-specialised pipeline kernel (sid_pm_ws_kernel.cuh): small result maps (geometry: radius <= 24; its shared-memory layout fits 227 KB up to radius 20 at s = 35, 22 with two sets of window statistics), needs the split tail
-    PmWsCfg wg;
-    memset(&wg, 0, sizeof wg);
-    alignas(64) CUtensorMap tmap1;                  // image 1: the patch the templates of a point are sampled from
-    memset(&tmap1, 0, sizeof tmap1);
-    bool use_ws = false;
-    if (want_ws && split_tail) {
+    const bool split_tail = split_tail_fits(a.max_rr, smth);
+    a.split_tail = split_tail ? 1 : 0;
+    if (split_tail) a.tail_stride = (a.max_rr + 3) & ~3;
+    p.tail_threads = pm_tail_threads(a.max_rr);
+    p.tail_smem = pm_tail_smem_bytes(a.max_rr, smth);
+    if (split_tail)
+        if (int arc = allow_max_smem(ctx, (const void *)pm_tail_kernel)) return arc;
+    // warp-specialised pipeline kernel (sid_pm_ws_kernel.cuh): small result maps (geometry: radius <= 24; its shared-memory
+    // layout fits 227 KB up to radius 20 at s = 35, 22 with two sets of window statistics), needs the split tail
+    if (ws_wanted() && split_tail) {
         // three sets of window statistics where they fit the shared memory, else two (radius 21 ... 22 at img_size 35)
         const int rtyp = 2 * typ_border + (Wmax - 2 * max_border) - s + 1;
         bool fits = false;
-        for (int nstat = WS_NSTAT; nstat >= 2 && !fits; --nstat)
-            fits = pm_ws_geometry(s, Rmax, Wmax, n_angles, a.max_rr, wg, rtyp, nstat) && (size_t)wg.smem_bytes + 2048 <= (size_t)ctx->max_smem_optin;
-        if (fits && make_window_tensor_map(ctx, &tmap, 16, wg.load_rows) && make_window_tensor_map(ctx, &tmap1, wg.pbw, wg.pbh, 1))
-            use_ws = true;
-    }
-    if (use_ws) {
-        a.tma = 1; a.ab = wg.nab;
-        int rc = reserve(ctx, ctx->counter, 256);
-        if (rc) return rc;
-        a.counter = (unsigned int *)ctx->counter.p + 16 * slot;
-        CU(cudaMemsetAsync(a.counter, 0, sizeof(unsigned int), st));
-        a.split_tail = 1;
-        const size_t cap_n = (size_t)std::max<long long>(n + tail_off, ctx->tail_hint_n);
-        a.tail_stride = (a.max_rr + 3) & ~3;
-        // regions of concurrently running launches (bands, border classes) are laid out with ONE stride per host call;
-        // a work item of this kernel hands over three integer arrays (PmTailRec::mode 1)
-        const size_t region_stride = std::max(ctx->tail_region_stride, tail_item_words(a.tail_stride, 1));
-        if ((rc = reserve(ctx, ctx->tail_maps, cap_n * region_stride * sizeof(float)))) return rc;
-        if ((rc = reserve(ctx, ctx->tail_recs, cap_n * sizeof(PmTailRec)))) return rc;
-        a.tail_maps = (float *)ctx->tail_maps.p + (size_t)tail_off * region_stride;
-        a.tail_recs = (PmTailRec *)ctx->tail_recs.p + tail_off;
-        const void *kfn = (const void *)pm_ws_kernel;
-        if (int arc = allow_max_smem(ctx, kfn)) return arc;
-        long long grid = ctx->sm_count;
-        if (grid > n) grid = n;
-        if (grid < 1) grid = 1;
-        if (getenv("SID_DEBUG"))
-            fprintf(stderr, "[sid] launch: ws smem=%d nstat=%d nab=%d ks=%d npairs=%d nslots=%d slot_bytes=%d npanels=%d wrows=%d n16max=%d grid=%lld\n",
-                    wg.smem_bytes, wg.nstat, wg.nab, wg.ks, wg.npairs, wg.nslots, wg.slot_bytes, wg.npanels, wg.wrows, wg.n16max, grid);
-#ifdef SID_WS_PROF
-        if ((rc = reserve(ctx, ctx->scratch, (size_t)grid * 6 * 8 * 8))) return rc;
-        CU(cudaMemsetAsync(ctx->scratch.p, 0, (size_t)grid * 6 * 8 * 8, st));
-        a.scratch = (unsigned char *)ctx->scratch.p;
-#endif
-        void *params_ws[] = {(void *)&a, (void *)&wg, (void *)&tmap, (void *)&tmap1};
-        if (!ctx->k_ev[0]) { CU(cudaEventCreate(&ctx->k_ev[0])); CU(cudaEventCreate(&ctx->k_ev[1])); }
-        if (!ctx->k_ev_hold) CU(cudaEventRecord(ctx->k_ev[0], st));
-        CU(cudaLaunchKernel(kfn, dim3((unsigned)grid), dim3((unsigned)WS_THREADS), params_ws, (size_t)wg.smem_bytes, st));
-        CU(cudaEventRecord(ctx->k_ev[1], st));
-        ctx->k_ev_valid = true;
-        ctx->k_name = !ctx->k_ev_hold ? "sid::pm_ws_kernel"
-                      : strstr(ctx->k_name, "pm_tc_kernel") ? "sid::pm_tc_kernel + sid::pm_ws_kernel"
-                      : strstr(ctx->k_name, "pm_points_kernel") ? "sid::pm_points_kernel + sid::pm_ws_kernel" : "sid::pm_ws_kernel";
-        ctx->launches += 1;
-#ifdef SID_WS_PROF
-        {
-            std::vector<long long> h((size_t)grid * 48);
-            CU(cudaStreamSynchronize(st));
-            CU(cudaMemcpy(h.data(), ctx->scratch.p, h.size() * 8, cudaMemcpyDeviceToHost));
-            static const char *names[6] = {"control", "mma0", "gather0", "stats0", "epi0", "epi1"};
-            const double per_pt = (double)n / (double)grid;
-            for (int r = 0; r < 6; ++r) {
-                fprintf(stderr, "[ws prof] %-8s clk/point:", names[r]);
-                for (int k = 0; k < 8; ++k) {
-                    double sum = 0; for (long long c = 0; c < grid; ++c) sum += (double)h[((size_t)c * 6 + r) * 8 + k];
-                    fprintf(stderr, " %8.0f", sum / (double)grid / per_pt);
-                }
-                fprintf(stderr, "\n");
-            }
+        for (int nstat = WS_NSTAT; nstat >= 2 && !fits; --nstat) fits = ws_fits(ctx, s, max_border, n_angles, rtyp, nstat, p.wg);
+        if (fits && make_window_tensor_map(ctx, &p.tmap, 16, p.wg.load_rows) && make_window_tensor_map(ctx, &p.tmap1, p.wg.pbw, p.wg.pbh, 1)) {
+            p.kernel = PM_WS;
+            p.kfn = (const void *)pm_ws_kernel;
+            p.name = "sid::pm_ws_kernel";
+            a.tma = 1; a.ab = p.wg.nab;
+            p.smem = (size_t)p.wg.smem_bytes;
+            p.threads = WS_THREADS;
+            p.occ = 1;
+            return allow_max_smem(ctx, p.kfn);
         }
-#endif
-        const size_t tsm = pm_tail_smem_bytes(a.max_rr, smth);
-        if (int arc = allow_max_smem(ctx, (const void *)pm_tail_kernel)) return arc;
-        if (getenv("SID_DEBUG")) fprintf(stderr, "[sid] launch: tail threads=%d smem=%zu\n", pm_tail_threads(a.max_rr), tsm);
-        pm_tail_kernel<<<(unsigned)n, pm_tail_threads(a.max_rr), tsm, st>>>(a);
-        ctx->launches += 1;
-        CU(cudaGetLastError());
-        return SID_OK;
     }
-    if (want_tc && pm_tc_geometry(s, Rmax, Wmax, n_angles, tg) && make_window_tensor_map(ctx, &tmap, 16, tg.load_rows)) use_tc = true;
+    bool use_tc = want_tc && pm_tc_geometry(s, Rmax, Wmax, n_angles, p.tg) && make_window_tensor_map(ctx, &p.tmap, 16, p.tg.load_rows);
+    PmTcCfg &tg = p.tg;
     // Measured (profiles/r02_ab_tc_vs_imma.txt): with one CTA per SM (tensor memory > 256 columns: search radius ~100) the
     // latency-bound non-MAC phases make the tcgen05 kernel slower than the mma.sync kernel at three CTAs per SM, so the
     // default takes it only where two CTAs fit; SID_PM_PATH=tc forces it.
     if (use_tc && !path_env && tg.tmem_cols > 256) use_tc = false;
-    bool smem_scratch = false;
-    size_t smem = 0;
     int variant = 0;
     if (use_tc) {
         // window panels + four byte-shifted copies of the template rows (+ the per-point scratch when two CTAs
@@ -397,21 +345,20 @@ int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1,
         const size_t wsq_bytes = ((size_t)a.max_rr * 4 + 255) & ~(size_t)255;
         const size_t need = base + scratch + wsq_bytes;
         const size_t cap2 = 108 * 1024;
-        if (need <= cap2 && !getenv("SID_PM_GLOBAL_SCRATCH")) { smem_scratch = true; smem = need; }
-        else smem = base;
+        if (need <= cap2 && !global_scratch) { p.smem_scratch = true; p.smem = need; }
+        else p.smem = base;
         // window sums on the tensor cores: the two squares windows alias the result maps (dead until the first
         // epilogue), two accumulators of n16hmax columns + two A slots must fit the tensor-memory allocation
-        if (smem_scratch) {
+        if (p.smem_scratch) {
             const size_t maps_off = ((size_t)a.max_rr * 12 + 127) & ~(size_t)127;
             const size_t sq_bytes = 2 * (size_t)tg.npanels * (size_t)tg.wrows * 16;
             const bool fits_smem = maps_off + sq_bytes <= scratch;
             const bool fits_tmem = 2 * tg.n16hmax + 8 <= tg.nacc * tg.n16max + (tg.nslot - 2) * tg.slotc && tg.n16hmax <= tg.wrows;
-            const char *e = getenv("SID_TC_MMA_SUMS");
-            if (fits_smem && fits_tmem && !(e && e[0] == '0')) {
+            if (fits_smem && fits_tmem) {
                 tg.mma_sums = 1; tg.sq_off = (int)maps_off; tg.wsq_off = (int)scratch;
             }
         }
-        if (smem > (size_t)ctx->max_smem_optin - 4096 - (smem_scratch ? 0 : 8192)) use_tc = false;      // window too large: legacy kernels
+        if (p.smem > (size_t)ctx->max_smem_optin - 4096 - (p.smem_scratch ? 0 : 8192)) use_tc = false;      // window too large: legacy kernels
                                                                           // (the global-scratch variant has 8 KB more static shared memory)
     }
     const void *ktab[8] = {(const void *)pm_points_kernel<9, false, false>, (const void *)pm_points_kernel<13, false, false>,
@@ -423,13 +370,13 @@ int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1,
     if (!use_tc) {
     // window staging by TMA when the padded window (+15 bytes: the box must start 16-byte aligned) fits one
     // box of <= 256 x 256 bytes
-    memset(&tmap, 0, sizeof tmap);
+    memset(&p.tmap, 0, sizeof p.tmap);
     a.tma = 0;
     int wpw = pm_window_pitch_words(Wmax, imma);
     {
         const char *e = getenv("SID_PM_TMA");
         const int wpw_tma = pm_window_pitch_words(Wmax + 15, imma);
-        if (!(e && e[0] == '0') && make_window_tensor_map(ctx, &tmap, wpw_tma * 4, Wmax)) {
+        if (!(e && e[0] == '0') && make_window_tensor_map(ctx, &p.tmap, wpw_tma * 4, Wmax)) {
             a.tma = 1; a.tma_wpw = wpw_tma; a.tma_rows = Wmax;
             wpw = wpw_tma;
         }
@@ -451,15 +398,15 @@ int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1,
     // Shared memory: window + templates (+ the per-point scratch when it all fits in a third of an SM).
     const size_t smem_cap_fast = 75 * 1024;
     auto base_smem = [&](int ab) { return ((size_t)a.win_words + (size_t)ab * s * a.tpw) * 4; };
-    for (int ab = a.ab; ab >= 1 && !smem_scratch; --ab) {
+    for (int ab = a.ab; ab >= 1 && !p.smem_scratch; --ab) {
         const size_t need = base_smem(ab) + pm_scratch_bytes(a.max_rr, a.max_hrw, ab, smth, split_tail);
         // fewer resident templates only pays if it keeps all angles in <= the same number of batches
         if (need <= smem_cap_fast && (n_angles + ab - 1) / ab == (n_angles + a.ab - 1) / a.ab) {
-            smem_scratch = true; a.ab = ab; smem = need;
+            p.smem_scratch = true; a.ab = ab; p.smem = need;
         }
     }
-    if (getenv("SID_PM_GLOBAL_SCRATCH")) smem_scratch = false;
-    if (!smem_scratch) {
+    if (global_scratch) p.smem_scratch = false;
+    if (!p.smem_scratch) {
         // the kernel's static shared memory (PmShared, the window barrier: 1920 B as cudaFuncGetAttributes reports it) comes
         // out of the same per-block budget.  Without it a window that left less than that free was neither given fewer
         // angles per batch nor refused here, and failed the occupancy check below with SID_ECUDA instead (measured on a
@@ -467,11 +414,11 @@ int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1,
         cudaFuncAttributes fa;
         CU(cudaFuncGetAttributes(&fa, ktab[legacy_kidx(false)]));
         const size_t smem_max = (size_t)ctx->max_smem_optin - fa.sharedSizeBytes;
-        smem = base_smem(a.ab);
-        while (smem > smem_max && a.ab > 1) { --a.ab; smem = base_smem(a.ab); }
-        if (smem > smem_max) {
+        p.smem = base_smem(a.ab);
+        while (p.smem > smem_max && a.ab > 1) { --a.ab; p.smem = base_smem(a.ab); }
+        if (p.smem > smem_max) {
             if (getenv("SID_DEBUG"))
-                fprintf(stderr, "[sid] refuse: legacy smem=%zu limit=%zu static=%zu optin=%d\n", smem, smem_max,
+                fprintf(stderr, "[sid] refuse: legacy smem=%zu limit=%zu static=%zu optin=%d\n", p.smem, smem_max,
                         (size_t)fa.sharedSizeBytes, ctx->max_smem_optin);
             return fail(ctx, SID_EUNSUPPORTED, "search window too large for the fused kernel (border too big)");
         }
@@ -480,15 +427,15 @@ int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1,
 
     // CTA size: fill the CTA with thread tiles (dp4a) / warp tiles (IMMA) of a typical point
     const int Rt = 2 * typ_border + (Wmax - 2 * max_border) - s + 1;
-    int threads = PM_THREADS;
+    p.threads = PM_THREADS;
     if (use_tc) {
-        threads = TC_THREADS;
+        p.threads = TC_THREADS;
     } else if (imma) {
         const int warp_tiles = ((Rt + 15) / 16) * ((Rt + 23) / 24);
         double best_eff = -1.0;
         for (int w = 4; w <= PM_IMMA_THREADS / 32; ++w) {
             const double eff = (double)warp_tiles / (double)((warp_tiles + w - 1) / w * w);
-            if (eff >= best_eff - 1e-9) { best_eff = eff; threads = 32 * w; }
+            if (eff >= best_eff - 1e-9) { best_eff = eff; p.threads = 32 * w; }
         }
     } else {
         const int tx = pm_pick_tx(Rt);
@@ -499,83 +446,149 @@ int launch_pm(sid_ctx *ctx, long long n, const double *d_c1, const double *d_r1,
         double best_eff = -1.0;
         for (int bs = 128; bs <= PM_THREADS; bs += 32) {
             const double eff = (double)ntiles / (double)((ntiles + bs - 1) / bs * bs);
-            if (eff >= best_eff - 1e-9) { best_eff = eff; threads = bs; }
+            if (eff >= best_eff - 1e-9) { best_eff = eff; p.threads = bs; }
         }
     }
-    if (const char *e = use_tc ? nullptr : getenv("SID_PM_THREADS")) {
-        const int v = atoi(e);
-        if (v >= 32 && v <= (imma ? PM_IMMA_THREADS : PM_THREADS) && v % 32 == 0) threads = v;
-    }
 
-    const int kidx = use_tc ? (smem_scratch ? 9 : 8) : legacy_kidx(smem_scratch);
-    const void *kfn = use_tc ? (smem_scratch ? (const void *)pm_tc_kernel<true> : (const void *)pm_tc_kernel<false>) : ktab[kidx];
-    if (int arc = allow_max_smem(ctx, kfn)) return arc;
-    int occ = 0;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kfn, threads, smem));
-    if (occ < 1) {
+    p.kidx = use_tc ? (p.smem_scratch ? 9 : 8) : legacy_kidx(p.smem_scratch);
+    p.kfn = use_tc ? (p.smem_scratch ? (const void *)pm_tc_kernel<true> : (const void *)pm_tc_kernel<false>) : ktab[p.kidx];
+    if (int arc = allow_max_smem(ctx, p.kfn)) return arc;
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&p.occ, p.kfn, p.threads, p.smem));
+    if (p.occ < 1) {
         char msg[256];
         snprintf(msg, sizeof msg, "kernel does not fit on an SM (variant %d, %d threads, %zu B dynamic smem, img_size %d, max border %d, "
-                 "%d angles/batch, tma %d)", kidx, threads, smem, s, max_border, a.ab, a.tma);
+                 "%d angles/batch, tma %d)", p.kidx, p.threads, p.smem, s, max_border, a.ab, a.tma);
         return fail(ctx, SID_ECUDA, msg);
     }
-    if (getenv("SID_DEBUG"))
-        fprintf(stderr, "[sid] launch: tc=%d kidx=%d threads=%d smem=%zu occ(api)=%d tmem_cols=%d nab=%d ks=%d nacc=%d nb8=%d slotc=%d nslot=%d n16max=%d wrows=%d npanels=%d mma_sums=%d tma=%d nc=%d\n",
-                (int)use_tc, kidx, threads, smem, occ, tg.tmem_cols, tg.nab, tg.ks, tg.nacc, tg.nb8, tg.slotc, tg.nslot, tg.n16max, tg.wrows, tg.npanels, tg.mma_sums, a.tma, a.nc);
+    p.occ_api = p.occ;
     if (use_tc) {
         // The occupancy API answers 1 for a kernel that executes tcgen05.alloc with a run-time column count (it has to
         // assume all 512 columns); residency is really bounded by registers, shared memory and the columns we ask for.
         cudaFuncAttributes fa;
-        CU(cudaFuncGetAttributes(&fa, kfn));
+        CU(cudaFuncGetAttributes(&fa, p.kfn));
         int smem_sm = 0, regs_sm = 0;
         CU(cudaDeviceGetAttribute(&smem_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, ctx->device));
         CU(cudaDeviceGetAttribute(&regs_sm, cudaDevAttrMaxRegistersPerMultiprocessor, ctx->device));
-        const int by_smem = (int)((size_t)smem_sm / (smem + fa.sharedSizeBytes + 1024));
-        const int by_regs = regs_sm / std::max(1, fa.numRegs * threads);
-        occ = std::max(1, std::min(std::min(by_smem, by_regs), 512 / tg.tmem_cols));
+        const int by_smem = (int)((size_t)smem_sm / (p.smem + fa.sharedSizeBytes + 1024));
+        const int by_regs = regs_sm / std::max(1, fa.numRegs * p.threads);
+        p.occ = std::max(1, std::min(std::min(by_smem, by_regs), 512 / tg.tmem_cols));
     }
-    if (const char *e = getenv("SID_PM_OCC")) { const int v = atoi(e); if (v >= 1 && v <= occ) occ = v; }
-    long long grid = (long long)ctx->sm_count * occ;
-    if (grid > n) grid = n;
-    if (grid < 1) grid = 1;
-
     a.scratch_per_cta = pm_scratch_bytes(a.max_rr, a.max_hrw, a.ab, smth, split_tail);
-    int rc = SID_OK;
-    if (!smem_scratch) {
-        const size_t per_slot = (size_t)a.scratch_per_cta * (size_t)ctx->sm_count * (size_t)occ;
-        rc = reserve(ctx, ctx->scratch, per_slot * 2);
-        if (rc) return rc;
-        a.scratch = (unsigned char *)ctx->scratch.p + per_slot * (size_t)slot;
-    }
-    rc = reserve(ctx, ctx->counter, 256);
-    if (rc) return rc;
-    a.counter = (unsigned int *)ctx->counter.p + 16 * slot;
-    CU(cudaMemsetAsync(a.counter, 0, sizeof(unsigned int), st));
+    p.kernel = use_tc ? PM_TC : PM_POINTS;
+    p.name = use_tc ? "sid::pm_tc_kernel" : imma ? "sid::pm_points_kernel<imma>" : "sid::pm_points_kernel<dp4a>";
+    return SID_OK;
+}
 
-    a.split_tail = split_tail ? 1 : 0;
-    if (split_tail) {
-        const size_t cap_n = (size_t)std::max<long long>(n + tail_off, ctx->tail_hint_n);
-        a.tail_stride = (a.max_rr + 3) & ~3;
-        const size_t region_stride = std::max(ctx->tail_region_stride, (size_t)a.tail_stride);
-        if ((rc = reserve(ctx, ctx->tail_maps, cap_n * region_stride * sizeof(float)))) return rc;
-        if ((rc = reserve(ctx, ctx->tail_recs, cap_n * sizeof(PmTailRec)))) return rc;
-        a.tail_maps = (float *)ctx->tail_maps.p + (size_t)tail_off * region_stride;
+// What every matching launch of one sid_run / sid_run_pair / sid_run_device / sid_run_maps call shares
+struct PmCall {
+    const double *c1, *r1, *c2fg, *r2fg, *border;     // device point arrays
+    const double *angles, *tab;                        // device angle table
+    int rot_order;
+    double *out;
+    int *status;
+    float *maps_out;                 // sid_run_maps only (null otherwise), see PmArgs::maps_out
+    const long long *map_off;
+    uint8_t *tpl_out;
+    long long n;                     // points of the call: the tail hand-off regions are laid out for all of them
+    // set by reserve_call
+    size_t tail_stride;              // floats per point of the tail hand-off regions
+    size_t scratch_slot;             // bytes of global scratch per band stream
+};
+
+// The buffers the launches of a call share, reserved once before the first launch, so that none of them is reallocated
+// while a launch of the call is in flight.  Launches of different bands run concurrently on two streams: the tail hand-off
+// regions of all of them are laid out with ONE stride, and each stream has its own scratch slot and work counter.
+int reserve_call(sid_ctx *ctx, PmCall &call, const PmPlan *plans, int nplans) {
+    call.tail_stride = 0;
+    call.scratch_slot = 0;
+    for (int i = 0; i < nplans; ++i) {
+        const PmPlan &p = plans[i];
+        // a work item of pm_ws_kernel hands over three integer arrays (PmTailRec::mode 1), the others a float map
+        if (p.args.split_tail) call.tail_stride = std::max(call.tail_stride, tail_item_words(p.args.tail_stride, p.kernel == PM_WS));
+        if (p.kernel != PM_WS && !p.smem_scratch)
+            call.scratch_slot = std::max(call.scratch_slot, (size_t)p.args.scratch_per_cta * (size_t)ctx->sm_count * (size_t)p.occ);
+#ifdef SID_WS_PROF
+        if (p.kernel == PM_WS) call.scratch_slot = std::max(call.scratch_slot, (size_t)ctx->sm_count * 6 * 8 * 8);
+#endif
+    }
+    int rc = reserve(ctx, ctx->counter, 256);
+    if (rc) return rc;
+    if (call.scratch_slot && (rc = reserve(ctx, ctx->scratch, call.scratch_slot * 2))) return rc;
+    if (call.tail_stride) {
+        if ((rc = reserve(ctx, ctx->tail_maps, (size_t)call.n * call.tail_stride * sizeof(float)))) return rc;
+        if ((rc = reserve(ctx, ctx->tail_recs, (size_t)call.n * sizeof(PmTailRec)))) return rc;
+    }
+    return SID_OK;
+}
+
+// Enqueue one launch of a plan (and its split tail) on the buffers reserve_call reserved: points order[0 .. n) (null:
+// points 0 .. n - 1), their tail hand-off at point offset tail_off of the call's regions; `slot` picks the counter and
+// scratch of one of the two band streams.  `continues`: the second class of a two-class call, so the kernel-time events
+// bracket both launches.
+int enqueue_pm(sid_ctx *ctx, const PmCall &call, const PmPlan &p, long long n, const int *order, cudaStream_t st, int slot,
+               long long tail_off, bool continues) {
+    PmArgs a = p.args;
+    a.img1 = (const uint8_t *)ctx->img1.p; a.rows1 = ctx->rows1; a.cols1 = ctx->cols1; a.pitch1 = ctx->pitch1;
+    a.img2 = (const uint8_t *)ctx->img2.p; a.rows2 = ctx->rows2; a.cols2 = ctx->cols2; a.pitch2 = ctx->pitch2;
+    a.n = n;
+    a.c1 = call.c1; a.r1 = call.r1; a.c2fg = call.c2fg; a.r2fg = call.r2fg; a.border = call.border; a.order = order;
+    a.angles = call.angles; a.tab = call.tab; a.rot_order = call.rot_order;
+    a.out = call.out; a.status = call.status;
+    a.maps_out = call.maps_out; a.map_off = call.map_off; a.tpl_out = call.tpl_out;
+    a.counter = (unsigned int *)ctx->counter.p + 16 * slot;
+    a.scratch = (unsigned char *)ctx->scratch.p + call.scratch_slot * (size_t)slot;      // read by the global-scratch variants only
+    if (a.split_tail) {
+        a.tail_maps = (float *)ctx->tail_maps.p + (size_t)tail_off * call.tail_stride;
         a.tail_recs = (PmTailRec *)ctx->tail_recs.p + tail_off;
     }
-    void *params_legacy[] = {(void *)&a, (void *)&tmap};
-    void *params_tc[] = {(void *)&a, (void *)&tg, (void *)&tmap};
-    void **params = use_tc ? params_tc : params_legacy;
+    const long long grid = std::max(1LL, std::min((long long)ctx->sm_count * p.occ, n));
+    CU(cudaMemsetAsync(a.counter, 0, sizeof(unsigned int), st));
+    const bool debug = getenv("SID_DEBUG") != nullptr;
+    const PmWsCfg &wg = p.wg;
+    const PmTcCfg &tg = p.tg;
+    if (debug && p.kernel == PM_WS)
+        fprintf(stderr, "[sid] launch: ws smem=%d nstat=%d nab=%d ks=%d npairs=%d nslots=%d slot_bytes=%d npanels=%d wrows=%d n16max=%d grid=%lld\n",
+                wg.smem_bytes, wg.nstat, wg.nab, wg.ks, wg.npairs, wg.nslots, wg.slot_bytes, wg.npanels, wg.wrows, wg.n16max, grid);
+    else if (debug)
+        fprintf(stderr, "[sid] launch: tc=%d kidx=%d threads=%d smem=%zu occ(api)=%d tmem_cols=%d nab=%d ks=%d nacc=%d nb8=%d slotc=%d nslot=%d n16max=%d wrows=%d npanels=%d mma_sums=%d tma=%d nc=%d\n",
+                (int)(p.kernel == PM_TC), p.kidx, p.threads, p.smem, p.occ_api, tg.tmem_cols, tg.nab, tg.ks, tg.nacc, tg.nb8, tg.slotc, tg.nslot,
+                tg.n16max, tg.wrows, tg.npanels, tg.mma_sums, a.tma, a.nc);
+#ifdef SID_WS_PROF
+    if (p.kernel == PM_WS) CU(cudaMemsetAsync(a.scratch, 0, (size_t)grid * 6 * 8 * 8, st));
+#endif
+    void *params_ws[] = {(void *)&a, (void *)&p.wg, (void *)&p.tmap, (void *)&p.tmap1};
+    void *params_tc[] = {(void *)&a, (void *)&p.tg, (void *)&p.tmap};
+    void *params_points[] = {(void *)&a, (void *)&p.tmap};
+    void **params = p.kernel == PM_WS ? params_ws : p.kernel == PM_TC ? params_tc : params_points;
     if (!ctx->k_ev[0]) { CU(cudaEventCreate(&ctx->k_ev[0])); CU(cudaEventCreate(&ctx->k_ev[1])); }
-    if (!ctx->k_ev_hold) CU(cudaEventRecord(ctx->k_ev[0], st));
-    CU(cudaLaunchKernel(kfn, dim3((unsigned)grid), dim3((unsigned)threads), params, smem, st));
+    if (!continues) CU(cudaEventRecord(ctx->k_ev[0], st));
+    CU(cudaLaunchKernel(p.kfn, dim3((unsigned)grid), dim3((unsigned)p.threads), params, p.smem, st));
     CU(cudaEventRecord(ctx->k_ev[1], st));
     ctx->k_ev_valid = true;
-    ctx->k_name = use_tc ? "sid::pm_tc_kernel" : imma ? "sid::pm_points_kernel<imma>" : "sid::pm_points_kernel<dp4a>";
+    ctx->k_name = p.kernel != PM_WS || !continues ? p.name
+                  : strstr(ctx->k_name, "pm_tc_kernel") ? "sid::pm_tc_kernel + sid::pm_ws_kernel"
+                  : strstr(ctx->k_name, "pm_points_kernel") ? "sid::pm_points_kernel + sid::pm_ws_kernel" : p.name;
     ctx->launches += 1;
-    if (split_tail) {
-        const size_t tsm = pm_tail_smem_bytes(a.max_rr, smth);
-        if (int arc = allow_max_smem(ctx, (const void *)pm_tail_kernel)) return arc;
-        if (getenv("SID_DEBUG")) fprintf(stderr, "[sid] launch: tail threads=%d smem=%zu\n", pm_tail_threads(a.max_rr), tsm);
-        pm_tail_kernel<<<(unsigned)n, pm_tail_threads(a.max_rr), tsm, st>>>(a);
+#ifdef SID_WS_PROF
+    if (p.kernel == PM_WS) {             // role profile: cycles per bucket and point, averaged over the CTAs
+        std::vector<long long> h((size_t)grid * 48);
+        CU(cudaStreamSynchronize(st));
+        CU(cudaMemcpy(h.data(), a.scratch, h.size() * 8, cudaMemcpyDeviceToHost));
+        static const char *names[6] = {"control", "mma0", "gather0", "stats0", "epi0", "epi1"};
+        const double per_pt = (double)n / (double)grid;
+        for (int r = 0; r < 6; ++r) {
+            fprintf(stderr, "[ws prof] %-8s clk/point:", names[r]);
+            for (int k = 0; k < 8; ++k) {
+                double sum = 0; for (long long c = 0; c < grid; ++c) sum += (double)h[((size_t)c * 6 + r) * 8 + k];
+                fprintf(stderr, " %8.0f", sum / (double)grid / per_pt);
+            }
+            fprintf(stderr, "\n");
+        }
+    }
+#endif
+    if (a.split_tail) {
+        if (debug) fprintf(stderr, "[sid] launch: tail threads=%d smem=%zu\n", p.tail_threads, p.tail_smem);
+        pm_tail_kernel<<<(unsigned)n, p.tail_threads, p.tail_smem, st>>>(a);
         ctx->launches += 1;
         CU(cudaGetLastError());
     }
@@ -772,32 +785,41 @@ static int upload_angles(sid_ctx *ctx, int n_angles, const double *angles, const
 
 namespace {
 
-// Largest border (<= max_border) for which launch_pm would pick pm_ws_kernel (its geometry, its shared-memory layout and
-// the split tail all fit); -1 if none.  Used to send the points of a call to the kernels by border class.
+// Largest border (<= max_border) for which plan_pm would pick pm_ws_kernel (its geometry, its shared-memory layout and
+// the split tail all fit); -1 if none.
 int ws_border_limit(sid_ctx *ctx, int s, int n_angles, unsigned flags, int max_border) {
-    const char *path_env = getenv("SID_PM_PATH");
-    const bool want_ws = path_env ? strcmp(path_env, "ws") == 0 : SID_WS_DEFAULT != 0;
-    if (!want_ws) return -1;
-    if (const char *e = getenv("SID_PM_SPLIT_TAIL")) if (e[0] == '0') return -1;
+    if (!ws_wanted()) return -1;
     const bool smth = (flags & SID_HES_SMTH) != 0;
-    const int hws = s / 2;
     for (int b = std::min(max_border, 40); b >= 1; --b) {
-        const int Wmax = 2 * hws + 2 * b + 1, Rmax = Wmax - s + 1;
+        const int Rmax = 2 * (s / 2) + 2 * b + 1 - s + 1;
         if (Rmax < 2) break;
-        if (pm_tail_smem_bytes(Rmax * Rmax, smth) > tail_split_limit()) continue;
+        if (!split_tail_fits(Rmax * Rmax, smth)) continue;
         PmWsCfg g;
-        memset(&g, 0, sizeof g);
-        // the launch pads the angle planes for ITS typical map width (<= 31 words each): try the worst case, so that a
-        // border this function accepts is never refused by the launch
+        // the planner pads the angle planes for ITS typical map width (<= 31 words in each of 2 x 3 planes): where that may
+        // not fit, try every width, so that a border accepted here is never refused by the launch
         // (the smallest layout: two sets of window statistics)
-        bool ok = pm_ws_geometry(s, Rmax, Wmax, n_angles, Rmax * Rmax, g, 0, 2) && (size_t)g.smem_bytes + 2048 <= (size_t)ctx->max_smem_optin;
-        if (ok && (size_t)g.smem_bytes + 2048 + 31 * 4 * 2 * 3 > (size_t)ctx->max_smem_optin) {
-            for (int rt = 2; rt <= Rmax && ok; ++rt)
-                ok = pm_ws_geometry(s, Rmax, Wmax, n_angles, Rmax * Rmax, g, rt, 2) && (size_t)g.smem_bytes + 2048 <= (size_t)ctx->max_smem_optin;
-        }
+        bool ok = ws_fits(ctx, s, b, n_angles, 0, 2, g);
+        if (ok && !ws_fits(ctx, s, b, n_angles, 0, 2, g, 31 * 4 * 2 * 3))
+            for (int rt = 2; rt <= Rmax && ok; ++rt) ok = ws_fits(ctx, s, b, n_angles, rt, 2, g);
         if (ok) return b;
     }
     return -1;
+}
+
+// Border classes of a call with borders up to max_border: the points with borders up to the returned limit go to
+// pm_ws_kernel in launches of their own, the others to the kernels for larger maps; -1: one class (SID_PM_CLASSES=0, or
+// pm_ws_kernel takes all borders or none)
+int small_class_limit(sid_ctx *ctx, int s, int n_angles, unsigned flags, int max_border) {
+    const char *e = getenv("SID_PM_CLASSES");
+    if (e && e[0] == '0') return -1;
+    const int limit = ws_border_limit(ctx, s, n_angles, flags, max_border);
+    return limit < max_border ? limit : -1;
+}
+
+// A point's border in whole pixels (fractional borders: the window can be one pixel wider; not finite, negative or
+// >= 4096: 0)
+__host__ __device__ inline int border_pixels(double b) {
+    return isfinite(b) && b >= 0.0 && b < 4096.0 ? (int)ceil(b) : 0;
 }
 
 // Device-resident callers (sid_run_device): split the point indices by border class on the device
@@ -806,10 +828,7 @@ __global__ void partition_by_border_kernel(const double *__restrict__ border, in
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     bool small = false, valid = i < n;
     if (valid) {
-        const double b = border[i];
-        int v = 0;
-        if (isfinite(b) && b >= 0.0 && b < 4096.0) v = (int)ceil(b);
-        small = v <= limit;
+        small = border_pixels(border[i]) <= limit;
     }
     const unsigned m_small = __ballot_sync(0xffffffffu, valid && small), m_big = __ballot_sync(0xffffffffu, valid && !small);
     const int lane = threadIdx.x & 31;
@@ -878,12 +897,13 @@ struct HostPair {
 
 constexpr int MAX_BANDS = 16;
 
-// Body of sid_run and sid_run_pair.  With `pair` the images are uploaded in row bands on a second
+// Body of sid_run, sid_run_pair and sid_run_maps (maps_out, map_off, tpl_out: see PmArgs).  With `pair` the images are uploaded in row bands on a second
 // stream while the fused kernel already works on the points whose windows and templates lie
 // entirely inside the bands that have arrived (PCIe copy overlapped with compute).
 int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, const double *r1, const double *c2fg,
              const double *r2fg, const double *border, int img_size, int n_angles, const double *angles,
-             const double *angle_tab, int rot_order, unsigned flags, int mtype, double *out, int *status) {
+             const double *angle_tab, int rot_order, unsigned flags, int mtype, double *out, int *status,
+             float *maps_out, const long long *map_off, uint8_t *tpl_out) {
     int rc = check_common(ctx, img_size, n_angles, angle_tab, rot_order, mtype);
     if (rc) return rc;
     if (!pair && !ctx->have_pair) return fail(ctx, SID_ENOPAIR, "sid_set_pair has not been called");
@@ -1021,9 +1041,7 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
     const double ext = 0.5 * std::sqrt(2.0) * (img_size + 2) + 3.0;      // template reach around (c1, r1) incl. rounding
     const int hws = img_size / 2;
     for (int64_t i = 0; i < n; ++i) {
-        const double b = border[i];
-        int v = 0;
-        if (std::isfinite(b) && b >= 0.0 && b < 4096.0) v = (int)std::ceil(b);   // fractional borders: the window can be one pixel wider
+        const int v = border_pixels(border[i]);
         ib[(size_t)i] = v;
         max_border = std::max(max_border, v);
         if (nbands > 1) {
@@ -1055,17 +1073,14 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
     //      whose border fits pm_ws_kernel get their own launch per band, behind the larger ones (SID_PM_CLASSES=0: one launch).
     int small_max = -1, typ_small = 0, typ_big = typ_border;
     bool two_class = false;
-    {
-        const char *e = getenv("SID_PM_CLASSES");
-        const int limit = (e && e[0] == '0') ? -1 : ws_border_limit(ctx, img_size, n_angles, flags, max_border);
-        if (limit >= 0 && limit < max_border) {
-            long long n_small = 0;
-            for (int b = 0; b <= limit; ++b) if (per_b[(size_t)b]) { n_small += per_b[(size_t)b]; small_max = b; }
-            if (n_small >= 256 && small_max >= 1) {
-                two_class = true;
-                typ_small = median_border(0, small_max);
-                typ_big = median_border(limit + 1, max_border);
-            }
+    const int limit = small_class_limit(ctx, img_size, n_angles, flags, max_border);
+    if (limit >= 0) {
+        long long n_small = 0;
+        for (int b = 0; b <= limit; ++b) if (per_b[(size_t)b]) { n_small += per_b[(size_t)b]; small_max = b; }
+        if (n_small >= 256 && small_max >= 1) {
+            two_class = true;
+            typ_small = median_border(0, small_max);
+            typ_big = median_border(limit + 1, max_border);
         }
     }
     std::vector<int> band_mid((size_t)nbands, 0);           // first point of the small class inside each band's range
@@ -1107,15 +1122,12 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
         for (int k = 1; k < nbands; ++k) if ((rc = enqueue_band_copy(k))) return rc;
 
     const double *dp = (const double *)ctx->pts.p;
-    ctx->tail_hint_n = n;
-    ctx->tail_region_stride = 0;
-    if (two_class) {
-        // one stride for the tail-map regions of both classes (launches of different bands run concurrently)
-        auto rr_of = [&](int b) { const int R = 2 * (img_size / 2) + 2 * b + 1 - img_size + 1; return R * R; };
-        const bool smth = (flags & SID_HES_SMTH) != 0;
-        const int rr_big = rr_of(max_border), rr_small = rr_of(small_max);
-        ctx->tail_region_stride = tail_region_words(rr_big, rr_small, smth);
-    }
+    PmCall call{dp, dp + n, dp + 2 * n, dp + 3 * n, dp + 4 * n, d_angles, d_tab, rot_order, (double *)ctx->out.p,
+                (int *)ctx->status.p, maps_out, map_off, tpl_out, n, 0, 0};
+    PmPlan plans[2];            // the larger borders (all points when the call is not split into classes), the class of pm_ws_kernel
+    if ((rc = plan_pm(ctx, img_size, n_angles, flags, max_border, two_class ? typ_big : typ_border, plans[0]))) return rc;
+    if (two_class && (rc = plan_pm(ctx, img_size, n_angles, flags, small_max, typ_small, plans[1]))) return rc;
+    if ((rc = reserve_call(ctx, call, plans, two_class ? 2 : 1))) return rc;
     const bool two_streams = pair && nbands > 1;
     if (two_streams) {
         if (!ctx->band_stream[0])
@@ -1131,22 +1143,11 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
         if (pair) CU(cudaStreamWaitEvent(st, ctx->band_event[k], 0));
         const int lo = band_start[(size_t)k], hi = band_start[(size_t)k + 1], mid = band_mid[(size_t)k];
         if (hi <= lo) continue;
-        if (mid > lo) {         // the larger borders (all points when the call is not split into classes)
-            rc = launch_pm(ctx, mid - lo, dp, dp + n, dp + 2 * n, dp + 3 * n, dp + 4 * n, (const int *)ctx->order.p + lo,
-                           max_border, two_class ? typ_big : typ_border, img_size, n_angles, d_angles, d_tab, rot_order, flags,
-                           (double *)ctx->out.p, (int *)ctx->status.p, st, two_streams ? (k & 1) : 0, lo);
-            if (rc) { ctx->tail_region_stride = 0; return rc; }
-        }
-        if (hi > mid) {         // the class of pm_ws_kernel
-            ctx->k_ev_hold = mid > lo;
-            rc = launch_pm(ctx, hi - mid, dp, dp + n, dp + 2 * n, dp + 3 * n, dp + 4 * n, (const int *)ctx->order.p + mid,
-                           small_max, typ_small, img_size, n_angles, d_angles, d_tab, rot_order, flags,
-                           (double *)ctx->out.p, (int *)ctx->status.p, st, two_streams ? (k & 1) : 0, mid);
-            ctx->k_ev_hold = false;
-            if (rc) { ctx->tail_region_stride = 0; return rc; }
-        }
+        const int slot = two_streams ? (k & 1) : 0;
+        const int *order = (const int *)ctx->order.p;
+        if (mid > lo && (rc = enqueue_pm(ctx, call, plans[0], mid - lo, order + lo, st, slot, lo, false))) return rc;
+        if (hi > mid && (rc = enqueue_pm(ctx, call, plans[1], hi - mid, order + mid, st, slot, mid, mid > lo))) return rc;
     }
-    ctx->tail_region_stride = 0;
     if (two_streams) {
         for (int k = 0; k < 2; ++k) {
             CU(cudaEventRecord(ctx->slot_event[1 + k], ctx->band_stream[k]));
@@ -1172,7 +1173,7 @@ int sid_run(sid_ctx *ctx, int64_t n, const double *c1, const double *r1, const d
             const double *r2fg, const double *border, int img_size, int n_angles, const double *angles,
             const double *angle_tab, int rot_order, unsigned flags, int mtype, double *out, int *status) {
     return run_host(ctx, nullptr, n, c1, r1, c2fg, r2fg, border, img_size, n_angles, angles, angle_tab, rot_order,
-                    flags, mtype, out, status);
+                    flags, mtype, out, status, nullptr, nullptr, nullptr);
 }
 
 int sid_run_pair(sid_ctx *ctx, const uint8_t *img1, int rows1, int cols1, int64_t pitch1,
@@ -1183,7 +1184,7 @@ int sid_run_pair(sid_ctx *ctx, const uint8_t *img1, int rows1, int cols1, int64_
     if (!ctx) return SID_EINVAL;
     HostPair hp{img1, img2, rows1, cols1, rows2, cols2, (long long)pitch1, (long long)pitch2};
     return run_host(ctx, &hp, n, c1, r1, c2fg, r2fg, border, img_size, n_angles, angles, angle_tab, rot_order,
-                    flags, mtype, out, status);
+                    flags, mtype, out, status, nullptr, nullptr, nullptr);
 }
 
 int sid_run_device(sid_ctx *ctx, int64_t n, const double *d_c1, const double *d_r1, const double *d_c2fg,
@@ -1202,15 +1203,15 @@ int sid_run_device(sid_ctx *ctx, int64_t n, const double *d_c1, const double *d_
         CU(cudaMemcpyAsync(hb.data(), d_border, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));
         CU(cudaStreamSynchronize(ctx->stream));
         max_border = 1;
-        for (double b : hb) if (std::isfinite(b) && b >= 0.0 && b < 4096.0) max_border = std::max(max_border, (int)std::ceil(b));
+        for (double b : hb) max_border = std::max(max_border, border_pixels(b));
     }
     const double *d_angles, *d_tab;
     if ((rc = upload_angles(ctx, n_angles, angles, angle_tab, &d_angles, &d_tab))) return rc;
-    ctx->tail_region_stride = 0;
+    PmCall call{d_c1, d_r1, d_c2fg, d_r2fg, d_border, d_angles, d_tab, rot_order, d_out, d_status, nullptr, nullptr, nullptr, n, 0, 0};
+    PmPlan plans[2];
     // border classes as in sid_run (see run_host): the indices are split on the device, one 8-byte read-back sizes the launches
-    const char *ce = getenv("SID_PM_CLASSES");
-    const int limit = (ce && ce[0] == '0') || n < 512 ? -1 : ws_border_limit(ctx, img_size, n_angles, flags, max_border);
-    if (limit >= 0 && limit < max_border) {
+    const int limit = n < 512 ? -1 : small_class_limit(ctx, img_size, n_angles, flags, max_border);
+    if (limit >= 0) {
         if ((rc = reserve(ctx, ctx->order, (size_t)n * 2 * sizeof(int) + 64))) return rc;
         int *d_small = (int *)ctx->order.p, *d_big = d_small + n;
         unsigned *d_counts = (unsigned *)(d_big + n);
@@ -1223,26 +1224,17 @@ int sid_run_device(sid_ctx *ctx, int64_t n, const double *d_c1, const double *d_
         CU(cudaGetLastError());
         const long long n_small = counts[0], n_big = counts[1];
         if (n_small >= 256 && n_big > 0) {
-            auto rr_of = [&](int b) { const int R = 2 * (img_size / 2) + 2 * b + 1 - img_size + 1; return R * R; };
-            const bool smth = (flags & SID_HES_SMTH) != 0;
-            ctx->tail_region_stride = tail_region_words(rr_of(max_border), rr_of(limit), smth);
-            ctx->tail_hint_n = n;
-            rc = launch_pm(ctx, n_big, d_c1, d_r1, d_c2fg, d_r2fg, d_border, d_big, max_border, max_border, img_size,
-                           n_angles, d_angles, d_tab, rot_order, flags, d_out, d_status, nullptr, 0, 0);
-            if (!rc) {
-                ctx->k_ev_hold = true;
-                rc = launch_pm(ctx, n_small, d_c1, d_r1, d_c2fg, d_r2fg, d_border, d_small, limit, limit, img_size,
-                               n_angles, d_angles, d_tab, rot_order, flags, d_out, d_status, nullptr, 0, n_big);
-                ctx->k_ev_hold = false;
-            }
-            ctx->tail_region_stride = 0;
-            ctx->tail_hint_n = 0;
-            return rc;
+            if ((rc = plan_pm(ctx, img_size, n_angles, flags, max_border, max_border, plans[0]))) return rc;
+            if ((rc = plan_pm(ctx, img_size, n_angles, flags, limit, limit, plans[1]))) return rc;
+            if ((rc = reserve_call(ctx, call, plans, 2))) return rc;
+            if ((rc = enqueue_pm(ctx, call, plans[0], n_big, d_big, ctx->stream, 0, 0, false))) return rc;
+            return enqueue_pm(ctx, call, plans[1], n_small, d_small, ctx->stream, 0, n_big, true);
         }
         if (n_big == 0) max_border = limit;              // every point fits the pipeline kernel
     }
-    return launch_pm(ctx, n, d_c1, d_r1, d_c2fg, d_r2fg, d_border, nullptr, max_border, max_border, img_size,
-                     n_angles, d_angles, d_tab, rot_order, flags, d_out, d_status);
+    if ((rc = plan_pm(ctx, img_size, n_angles, flags, max_border, max_border, plans[0]))) return rc;
+    if ((rc = reserve_call(ctx, call, plans, 1))) return rc;
+    return enqueue_pm(ctx, call, plans[0], n, nullptr, ctx->stream, 0, 0, false);
 }
 
 // ------------------------------------------------------------------ winning maps and templates (sid_run_maps)
@@ -1300,12 +1292,9 @@ int sid_run_maps(sid_ctx *ctx, int64_t n, const double *c1, const double *r1, co
     CU(cudaMemsetAsync(ctx->maps.p, 0xff, (size_t)total * sizeof(float), ctx->stream));
     if (templates) CU(cudaMemsetAsync(ctx->tpl.p, 0, tpl_bytes, ctx->stream));
     CU(cudaMemcpyAsync(ctx->map_off.p, off.data(), (size_t)n * sizeof(long long), cudaMemcpyHostToDevice, ctx->stream));
-    ctx->maps_out = (float *)ctx->maps.p;
-    ctx->map_off_dev = (const long long *)ctx->map_off.p;
-    ctx->tpl_out = templates ? (uint8_t *)ctx->tpl.p : nullptr;
     rc = run_host(ctx, nullptr, n, c1, r1, c2fg, r2fg, border, img_size, n_angles, angles, angle_tab, rot_order,
-                  flags, mtype, out, status);
-    ctx->maps_out = nullptr; ctx->map_off_dev = nullptr; ctx->tpl_out = nullptr;
+                  flags, mtype, out, status, (float *)ctx->maps.p, (const long long *)ctx->map_off.p,
+                  templates ? (uint8_t *)ctx->tpl.p : nullptr);
     if (rc) return rc;
     if (total > 0) CU(cudaMemcpy(maps, ctx->maps.p, (size_t)total * sizeof(float), cudaMemcpyDeviceToHost));
     if (templates) CU(cudaMemcpy(templates, ctx->tpl.p, tpl_bytes, cudaMemcpyDeviceToHost));

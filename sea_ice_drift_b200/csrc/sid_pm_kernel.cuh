@@ -840,9 +840,8 @@ __global__ void __launch_bounds__(PM_TAIL_MAX_THREADS) pm_tail_kernel(const PmAr
     }
 }
 // CTA size of pm_tail_kernel by map size: a large map in shared memory leaves room for only two CTAs per SM, so each gets
-// more warps (SID_PM_TAIL_THREADS overrides; 128 / 256 / 512 take peak_statistics' fast path)
+// more warps (128 / 256 / 512 take peak_statistics' fast path)
 inline int pm_tail_threads(int max_rr) {
-    if (const char *e = getenv("SID_PM_TAIL_THREADS")) { const int v = atoi(e); if (v == 128 || v == 256 || v == 512) return v; }
     return max_rr <= 2560 ? 128 : (max_rr <= 6144 ? 256 : 512);
 }
 inline size_t pm_tail_smem_bytes(int max_rr, bool smth) { return (size_t)((max_rr + 3) & ~3) * 4 * (2 + (smth ? 2 : 0)) + 2048 * 4; }

@@ -265,7 +265,7 @@ def point_band(lo, need):
 
 
 def predicted_launches(lo, pts, s, limit):
-    """The (band, class) pairs run_host launches: one launch_pm per non-empty pair; the small class (borders <= the
+    """The (band, class) pairs run_host launches: one launch per non-empty pair; the small class (borders <= the
     pm_ws_kernel limit) is split off only when it has >= 256 points, one border >= 1 and a larger border exists."""
     c1, r1, c2, r2, b = pts
     ib = [int(math.ceil(x)) if np.isfinite(x) and 0.0 <= x < 4096.0 else 0 for x in b]

@@ -1,6 +1,6 @@
 """Every matching kernel over the whole img_size range (2 ... 128) and on both sides of each dispatch boundary.
 
-``launch_pm`` picks a kernel and its variant from shared-memory and tensor-memory arithmetic on (img_size, largest
+``plan_pm`` picks a kernel and its variant from shared-memory and tensor-memory arithmetic on (img_size, largest
 border, angles per batch, flags): pm_ws_kernel with three or two sets of window statistics, pm_tc_kernel with shared or
 global scratch, window sums on the tensor cores or not, 128 / 256 tensor-memory columns and a split or fused tail,
 pm_points_kernel<imma> with TMA or plain window loads and 1 ... 5 K chunks.  Each row of ``ROWS`` names the launch its
@@ -494,7 +494,7 @@ def largest_accepted_border(ctx, pts, s, angles, lo, hi):
     return lo
 
 
-# The largest border launch_pm takes at each size (1 angle, or 3 angles in batches of one): the legacy kernels with the
+# The largest border plan_pm takes at each size (1 angle, or 3 angles in batches of one): the legacy kernels with the
 # window in shared memory; the next is refused on the host with SID_EUNSUPPORTED.  Measured on a B200 (232448 B of opt-in
 # shared memory per block, 1920 B of it the kernels' static shared memory by cudaFuncGetAttributes).
 # Regression: the shared-memory check used to leave out that static part, so a window just below the limit was neither
