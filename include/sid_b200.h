@@ -64,11 +64,24 @@ typedef struct sid_ctx sid_ctx;
  * and the same down the column for dy and r2.  |dx|, |dy| <= 0.5; a peak on the first or last column (row) leaves c2
  * (r2) exactly as without the flag.  Angle, r, h, the NaN rows and status are bit-identical to the call without it. */
 #define SID_SUBPIXEL 8u
+/* SID_MASKED (extension, not in the reference): match the rows the reference returns as NaN because some angle's template
+ * holds a 0 pixel (land, no-data, samples outside image 1) by the Pearson correlation over the template's valid pixels.
+ * For one angle's template T (s x s): M = (T > 0), n = sum M, St = sum T, Stt = sum T^2; at map position p over the
+ * window patch W (window pixels are data, zeros included; only the template is masked):
+ *   C = sum T W, Sw = sum M W, Sww = sum M W^2;  num = n C - St Sw, vt = n Stt - St^2, vw = n Sww - Sw^2   (exact int64)
+ *   r = (double)num / (sqrt((double)vt) * sqrt((double)vw)) in IEEE double without contraction, clamped to [-1, 1],
+ *   rounded to float32;  r = 0 where vw = 0
+ * (cv2.matchTemplate(image, T, TM_CCOEFF_NORMED, mask=(T > 0))).  A row is re-matched this way, every angle masked, when
+ * the call without the flag gives it SID_PT_NAN, every angle's template has at least ceil(s^2 / 2) valid pixels and
+ * vt > 0 for every angle; its status is SID_PT_MASKED.  Winner, h, mcc_norm, hes_smth and SID_SUBPIXEL follow the usual
+ * rules on the masked float maps.  Every other row is bit-identical to the call without the flag. */
+#define SID_MASKED 16u
 
 /* point status written by sid_run* (optional output) */
 #define SID_PT_VALID 1
 #define SID_PT_NAN 0         /* zero pixel in a template -> NaN row              */
 #define SID_PT_REJECTED (-1) /* window not inside image 2 / too small            */
+#define SID_PT_MASKED 2      /* SID_MASKED: matched by the masked rule          */
 
 const char *sid_version(void);
 
@@ -146,7 +159,7 @@ int sid_downsample_pair(sid_ctx *ctx, int factor,
                         uint8_t *d_img1, int64_t pitch1, int64_t bytes1,
                         uint8_t *d_img2, int64_t pitch2, int64_t bytes2);
 
-/* use_mcc for n grid points (host arrays in, host array out, synchronous).
+/* use_mcc for n grid points (host arrays in, host array out, synchronous).  All sid_run* honour SID_MASKED.
  *   c1, r1        float pixel coordinates on image 1
  *   c2fg, r2fg    integer-valued first guess on image 2
  *   border        integer-valued search radius per point
@@ -207,9 +220,10 @@ int sid_map_layout(sid_ctx *ctx, int64_t n,
  * computed from them).
  *   maps        maps_capacity floats: the maps of sid_map_layout packed in point order.  For a valid row, the raw
  *               float32 NCC map of the winning angle (the first of equal peaks; hes_smth and mcc_norm do not touch
- *               it; a flat template gives all 1.0).  Segments of rows that are not valid are NaN.
- *   templates   optional (may be NULL), n x img_size x img_size bytes: the winning angle's template; 0 for rows
- *               that are not valid.
+ *               it; a flat template gives all 1.0); for a SID_PT_MASKED row its masked map.  Segments of rows that
+ *               are neither are NaN.
+ *   templates   optional (may be NULL), n x img_size x img_size bytes: the winning angle's template (zeros
+ *               included for a SID_PT_MASKED row); 0 for rows that are neither valid nor masked.
  * maps_capacity below sid_map_layout's total -> SID_EINVAL before anything is launched. */
 int sid_run_maps(sid_ctx *ctx, int64_t n,
                  const double *c1, const double *r1,
@@ -233,7 +247,8 @@ const char *sid_last_kernel_name(const sid_ctx *ctx);
  * (host pointers).  Outputs: *valid (0 -> the reference returns 7 x NaN),
  * dc, dr, best_angle_idx (index into the angle list), best_r, best_h, and
  * optionally the best NCC map ((H-s+1) x (W-s+1) floats) and template (s x s).
- * SID_SUBPIXEL adds the sub-pixel offsets of sid_run to *dc / *dr; best_result is the unrefined map. */
+ * SID_SUBPIXEL adds the sub-pixel offsets of sid_run to *dc / *dr; best_result is the unrefined map.
+ * SID_MASKED applies the masked rule to any window size; *valid = 2 (SID_PT_MASKED) for a point it matched. */
 int sid_rotate_and_match(sid_ctx *ctx,
                          const uint8_t *img1, int rows1, int cols1, int64_t pitch1,
                          double c1, double r1, int img_size,

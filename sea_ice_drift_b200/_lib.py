@@ -20,7 +20,9 @@ _i32p = C.POINTER(C.c_int)
 SID_TM_CCOEFF_NORMED = 5
 SID_HES_NORM, SID_HES_SMTH, SID_MCC_NORM = 1, 2, 4
 SID_SUBPIXEL = 8                # extension: sub-pixel c2 / r2 (include/sid_b200.h)
+SID_MASKED = 16                 # extension: masked correlation for templates with 0 pixels (include/sid_b200.h)
 SID_PT_VALID = 1                # point status of a valid row (sid_run*)
+SID_PT_MASKED = 2               # point status of a row matched by the masked rule (SID_MASKED)
 
 EXPORTS = [
     "sid_version", "sid_create", "sid_destroy", "sid_last_error", "sid_set_stream", "sid_synchronize",
@@ -132,16 +134,17 @@ def pair_layout(rows, cols):
     return int(pitch.value), int(nbytes.value)
 
 
-def flags_from_kwargs(hes_norm=True, hes_smth=False, mcc_norm=False, subpixel=False):
+def flags_from_kwargs(hes_norm=True, hes_smth=False, mcc_norm=False, subpixel=False, masked=False):
     return (SID_HES_NORM if hes_norm else 0) | (SID_HES_SMTH if hes_smth else 0) | (SID_MCC_NORM if mcc_norm else 0) | \
-        (SID_SUBPIXEL if subpixel else 0)
+        (SID_SUBPIXEL if subpixel else 0) | (SID_MASKED if masked else 0)
 
 
 def flags_from_options(kwargs):
     """The sid_run* flags of a kwargs dict of the drop-in API: ``hes_norm`` (default True), ``hes_smth``, ``mcc_norm``
-    and the extension ``subpixel`` (default False), so every entry point maps its keyword arguments the same way."""
+    and the extensions ``subpixel`` and ``masked`` (default False), so every entry point maps its keyword arguments the
+    same way."""
     return flags_from_kwargs(kwargs.get('hes_norm', True), kwargs.get('hes_smth', False), kwargs.get('mcc_norm', False),
-                             kwargs.get('subpixel', False))
+                             kwargs.get('subpixel', False), kwargs.get('masked', False))
 
 
 class Context(object):
@@ -299,8 +302,8 @@ class Context(object):
                  mtype=SID_TM_CCOEFF_NORMED, want_status=False):
         """:meth:`run` on the resident pair that also returns every valid row's winning NCC map and template
         (``rotate_and_match(...)[5]`` / ``[6]``, sid_run_maps): ``(table, maps, templates[, status])``.  ``maps`` is a
-        list of N float32 2-D views into one contiguous buffer (point order), None where the row is not valid;
-        ``templates`` an (N, img_size, img_size) uint8 array, 0 where the row is not valid."""
+        list of N float32 2-D views into one contiguous buffer (point order), None where the row is neither valid nor
+        masked (SID_MASKED); ``templates`` an (N, img_size, img_size) uint8 array, 0 where the row is neither."""
         arrs = [np.ascontiguousarray(np.atleast_1d(x), dtype=np.float64) for x in (c1, r1, c2fg, r2fg, border)]
         n = arrs[0].size
         if any(a.size != n for a in arrs):
@@ -320,7 +323,7 @@ class Context(object):
             tab.ctypes.data, int(rot_order), int(flags), int(mtype), out.ctypes.data, status.ctypes.data,
             buf.size, buf.ctypes.data, templates.ctypes.data))
         ends = np.cumsum(shape[:, 0].astype(np.int64) * shape[:, 1])
-        maps = [buf[e - h * w:e].reshape(h, w) if st == 1 else None
+        maps = [buf[e - h * w:e].reshape(h, w) if st in (SID_PT_VALID, SID_PT_MASKED) else None
                 for (h, w), e, st in zip(shape.tolist(), ends.tolist(), status.tolist())]
         return (out, maps, templates, status) if want_status else (out, maps, templates)
 

@@ -26,6 +26,7 @@
 #include "sid_defor_kernel.cuh"
 #include "sid_fg_kernel.cuh"
 #include "sid_downsample_kernel.cuh"
+#include "sid_pm_masked_kernel.cuh"
 
 using namespace sid;
 
@@ -109,6 +110,7 @@ struct sid_ctx {
     // per-call buffers
     DevBuf pts, order, out, status, angles, scratch, counter, misc, tail_maps, tail_recs, epi, fg;
     DevBuf maps, map_off, tpl;               // sid_run_maps: packed maps, their offsets, the templates
+    DevBuf cand;                             // SID_MASKED: the candidate rows of the masked pass
     void *pin = nullptr;
     size_t pin_cap = 0;
     cudaEvent_t k_ev[2] = {};                // bracket the last fused-kernel launch (sid_last_kernel_ms)
@@ -258,7 +260,7 @@ bool ws_fits(const sid_ctx *ctx, int s, int border, int n_angles, int rtyp, int 
            (size_t)g.smem_bytes + 2048 + headroom <= (size_t)ctx->max_smem_optin;
 }
 
-enum PmKernel { PM_WS, PM_TC, PM_POINTS };
+enum PmKernel { PM_WS, PM_TC, PM_POINTS, PM_MASKED };
 
 // Everything a matching launch needs that does not depend on which points it takes: the kernel and its variant, its
 // configuration and tensor maps, the geometry fields of PmArgs, the CTA shape and that of the split tail
@@ -280,8 +282,9 @@ struct PmPlan {
 };
 
 // Kernel, variant and shape of a launch over points with borders up to max_border (typ_border: the typical point, which
-// sizes the CTA and pads pm_ws_kernel's layout).  Host queries only: nothing is allocated or enqueued.
-int plan_pm(sid_ctx *ctx, int s, int n_angles, unsigned flags, int max_border, int typ_border, PmPlan &p) {
+// sizes the CTA and pads pm_ws_kernel's layout).  `masked`: the masked pass of SID_MASKED (pm_masked_kernel, any border,
+// its own tail).  Host queries only: nothing is allocated or enqueued.
+int plan_pm(sid_ctx *ctx, int s, int n_angles, unsigned flags, int max_border, int typ_border, PmPlan &p, bool masked = false) {
     p = PmPlan{};
     const int hws = s / 2;
     const int Wmax = 2 * hws + 2 * max_border + 1;
@@ -295,6 +298,17 @@ int plan_pm(sid_ctx *ctx, int s, int n_angles, unsigned flags, int max_border, i
     gaussian_weights(a.gw);
     a.max_rr = Rmax * Rmax;
     a.max_hrw = Wmax * Rmax;
+    if (masked) {
+        p.kernel = PM_MASKED;
+        p.kfn = (const void *)pm_masked_kernel;
+        p.name = "sid::pm_masked_kernel";
+        p.threads = PM_MASKED_THREADS;
+        a.scratch_per_cta = pm_masked_scratch_bytes(a.max_rr);
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&p.occ, p.kfn, p.threads, 0));
+        if (p.occ < 1) return fail(ctx, SID_ECUDA, "pm_masked_kernel does not fit on an SM");
+        p.occ_api = p.occ;
+        return SID_OK;
+    }
     // correlation path: tcgen05 tensor cores (default), legacy mma.sync (SID_PM_PATH=imma) or the integer pipe
     // (SID_PM_PATH=dp4a); all three give bit-identical results
     const char *path_env = getenv("SID_PM_PATH");
@@ -490,6 +504,7 @@ struct PmCall {
     const long long *map_off;
     uint8_t *tpl_out;
     long long n;                     // points of the call: the tail hand-off regions are laid out for all of them
+    int *cand;                       // set by reserve_call for a masked pass: its candidate rows (n) and their count
     // set by reserve_call
     size_t tail_stride;              // floats per point of the tail hand-off regions
     size_t scratch_slot;             // bytes of global scratch per band stream
@@ -501,10 +516,12 @@ struct PmCall {
 int reserve_call(sid_ctx *ctx, PmCall &call, const PmPlan *plans, int nplans) {
     call.tail_stride = 0;
     call.scratch_slot = 0;
+    bool masked = false;
     for (int i = 0; i < nplans; ++i) {
         const PmPlan &p = plans[i];
         // a work item of pm_ws_kernel hands over three integer arrays (PmTailRec::mode 1), the others a float map
         if (p.args.split_tail) call.tail_stride = std::max(call.tail_stride, tail_item_words(p.args.tail_stride, p.kernel == PM_WS));
+        if (p.kernel == PM_MASKED) masked = true;
         if (p.kernel != PM_WS && !p.smem_scratch)
             call.scratch_slot = std::max(call.scratch_slot, (size_t)p.args.scratch_per_cta * (size_t)ctx->sm_count * (size_t)p.occ);
 #ifdef SID_WS_PROF
@@ -518,13 +535,23 @@ int reserve_call(sid_ctx *ctx, PmCall &call, const PmPlan *plans, int nplans) {
         if ((rc = reserve(ctx, ctx->tail_maps, (size_t)call.n * call.tail_stride * sizeof(float)))) return rc;
         if ((rc = reserve(ctx, ctx->tail_recs, (size_t)call.n * sizeof(PmTailRec)))) return rc;
     }
+    if (masked) {
+        // the masked pass finds its rows by their status: a call without a status array gets the context's
+        if (!call.status) {
+            if ((rc = reserve(ctx, ctx->status, (size_t)call.n * sizeof(int)))) return rc;
+            call.status = (int *)ctx->status.p;
+        }
+        if ((rc = reserve(ctx, ctx->cand, (size_t)call.n * sizeof(int)))) return rc;
+        call.cand = (int *)ctx->cand.p;
+    }
     return SID_OK;
 }
 
 // Enqueue one launch of a plan (and its split tail) on the buffers reserve_call reserved: points order[0 .. n) (null:
 // points 0 .. n - 1), their tail hand-off at point offset tail_off of the call's regions; `slot` picks the counter and
-// scratch of one of the two band streams.  `continues`: the second class of a two-class call, so the kernel-time events
-// bracket both launches.
+// scratch of one of the two band streams.  `continues`: the second class of a two-class call, or the masked pass, so the
+// kernel-time events bracket every launch of the call.  The masked pass (PM_MASKED) runs after every other launch of the
+// call: it gathers the rows they left with status 0 on the device (masked_candidates_kernel) and takes those.
 int enqueue_pm(sid_ctx *ctx, const PmCall &call, const PmPlan &p, long long n, const int *order, cudaStream_t st, int slot,
                long long tail_off, bool continues) {
     PmArgs a = p.args;
@@ -543,10 +570,20 @@ int enqueue_pm(sid_ctx *ctx, const PmCall &call, const PmPlan &p, long long n, c
     }
     const long long grid = std::max(1LL, std::min((long long)ctx->sm_count * p.occ, n));
     CU(cudaMemsetAsync(a.counter, 0, sizeof(unsigned int), st));
+    unsigned *n_cand = (unsigned *)ctx->counter.p + 32;
+    if (p.kernel == PM_MASKED) {
+        a.order = call.cand;
+        CU(cudaMemsetAsync(n_cand, 0, sizeof(unsigned), st));
+        masked_candidates_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(call.status, n, call.cand, n_cand);
+        ctx->launches += 1;
+        CU(cudaGetLastError());
+    }
     const bool debug = getenv("SID_DEBUG") != nullptr;
     const PmWsCfg &wg = p.wg;
     const PmTcCfg &tg = p.tg;
-    if (debug && p.kernel == PM_WS)
+    if (debug && p.kernel == PM_MASKED)
+        fprintf(stderr, "[sid] launch: masked threads=%d occ=%d scratch=%llu grid=%lld\n", p.threads, p.occ, a.scratch_per_cta, grid);
+    else if (debug && p.kernel == PM_WS)
         fprintf(stderr, "[sid] launch: ws smem=%d nstat=%d nab=%d ks=%d npairs=%d nslots=%d slot_bytes=%d npanels=%d wrows=%d n16max=%d grid=%lld\n",
                 wg.smem_bytes, wg.nstat, wg.nab, wg.ks, wg.npairs, wg.nslots, wg.slot_bytes, wg.npanels, wg.wrows, wg.n16max, grid);
     else if (debug)
@@ -559,13 +596,16 @@ int enqueue_pm(sid_ctx *ctx, const PmCall &call, const PmPlan &p, long long n, c
     void *params_ws[] = {(void *)&a, (void *)&p.wg, (void *)&p.tmap, (void *)&p.tmap1};
     void *params_tc[] = {(void *)&a, (void *)&p.tg, (void *)&p.tmap};
     void *params_points[] = {(void *)&a, (void *)&p.tmap};
-    void **params = p.kernel == PM_WS ? params_ws : p.kernel == PM_TC ? params_tc : params_points;
+    void *params_masked[] = {(void *)&a, (void *)&n_cand};
+    void **params = p.kernel == PM_WS ? params_ws : p.kernel == PM_TC ? params_tc : p.kernel == PM_MASKED ? params_masked : params_points;
     if (!ctx->k_ev[0]) { CU(cudaEventCreate(&ctx->k_ev[0])); CU(cudaEventCreate(&ctx->k_ev[1])); }
     if (!continues) CU(cudaEventRecord(ctx->k_ev[0], st));
     CU(cudaLaunchKernel(p.kfn, dim3((unsigned)grid), dim3((unsigned)p.threads), params, p.smem, st));
     CU(cudaEventRecord(ctx->k_ev[1], st));
     ctx->k_ev_valid = true;
-    ctx->k_name = p.kernel != PM_WS || !continues ? p.name
+    // the masked pass keeps the name of the correlation kernel of the call
+    ctx->k_name = p.kernel == PM_MASKED ? ctx->k_name
+                  : p.kernel != PM_WS || !continues ? p.name
                   : strstr(ctx->k_name, "pm_tc_kernel") ? "sid::pm_tc_kernel + sid::pm_ws_kernel"
                   : strstr(ctx->k_name, "pm_points_kernel") ? "sid::pm_points_kernel + sid::pm_ws_kernel" : p.name;
     ctx->launches += 1;
@@ -629,7 +669,7 @@ void sid_destroy(sid_ctx *ctx) {
     cudaStreamSynchronize(ctx->stream);
     DevBuf *bufs[] = {&ctx->img1, &ctx->img2, &ctx->pts, &ctx->order, &ctx->out, &ctx->status,
                       &ctx->angles, &ctx->scratch, &ctx->counter, &ctx->misc, &ctx->tail_maps, &ctx->tail_recs, &ctx->epi, &ctx->fg,
-                      &ctx->maps, &ctx->map_off, &ctx->tpl};
+                      &ctx->maps, &ctx->map_off, &ctx->tpl, &ctx->cand};
     for (DevBuf *b : bufs) if (b->p && b->owned) cudaFree(b->p);
     if (ctx->pin) cudaFreeHost(ctx->pin);
     if (ctx->stage) cudaFreeHost(ctx->stage);
@@ -1124,10 +1164,14 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
     const double *dp = (const double *)ctx->pts.p;
     PmCall call{dp, dp + n, dp + 2 * n, dp + 3 * n, dp + 4 * n, d_angles, d_tab, rot_order, (double *)ctx->out.p,
                 (int *)ctx->status.p, maps_out, map_off, tpl_out, n, 0, 0};
-    PmPlan plans[2];            // the larger borders (all points when the call is not split into classes), the class of pm_ws_kernel
+    // the larger borders (all points when the call is not split into classes), the class of pm_ws_kernel, the masked pass
+    PmPlan plans[3];
+    const bool masked = (flags & SID_MASKED) != 0;
+    const int nplans = two_class ? 2 : 1;
     if ((rc = plan_pm(ctx, img_size, n_angles, flags, max_border, two_class ? typ_big : typ_border, plans[0]))) return rc;
     if (two_class && (rc = plan_pm(ctx, img_size, n_angles, flags, small_max, typ_small, plans[1]))) return rc;
-    if ((rc = reserve_call(ctx, call, plans, two_class ? 2 : 1))) return rc;
+    if (masked && (rc = plan_pm(ctx, img_size, n_angles, flags, max_border, typ_border, plans[nplans], true))) return rc;
+    if ((rc = reserve_call(ctx, call, plans, nplans + (masked ? 1 : 0)))) return rc;
     const bool two_streams = pair && nbands > 1;
     if (two_streams) {
         if (!ctx->band_stream[0])
@@ -1154,6 +1198,8 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
             CU(cudaStreamWaitEvent(ctx->stream, ctx->slot_event[1 + k], 0));
         }
     }
+    // every band has arrived and every row has its status
+    if (masked && (rc = enqueue_pm(ctx, call, plans[nplans], n, nullptr, ctx->stream, 0, 0, true))) return rc;
     if (pair) ctx->have_pair = true;
     double *hout = (double *)((char *)ctx->pin + pts_bytes + ord_bytes);
     int *hst = (int *)((char *)hout + out_bytes);
@@ -1208,7 +1254,8 @@ int sid_run_device(sid_ctx *ctx, int64_t n, const double *d_c1, const double *d_
     const double *d_angles, *d_tab;
     if ((rc = upload_angles(ctx, n_angles, angles, angle_tab, &d_angles, &d_tab))) return rc;
     PmCall call{d_c1, d_r1, d_c2fg, d_r2fg, d_border, d_angles, d_tab, rot_order, d_out, d_status, nullptr, nullptr, nullptr, n, 0, 0};
-    PmPlan plans[2];
+    PmPlan plans[3];                 // [0], [1]: the border classes; the masked pass behind them
+    const bool masked = (flags & SID_MASKED) != 0;
     // border classes as in sid_run (see run_host): the indices are split on the device, one 8-byte read-back sizes the launches
     const int limit = n < 512 ? -1 : small_class_limit(ctx, img_size, n_angles, flags, max_border);
     if (limit >= 0) {
@@ -1226,15 +1273,19 @@ int sid_run_device(sid_ctx *ctx, int64_t n, const double *d_c1, const double *d_
         if (n_small >= 256 && n_big > 0) {
             if ((rc = plan_pm(ctx, img_size, n_angles, flags, max_border, max_border, plans[0]))) return rc;
             if ((rc = plan_pm(ctx, img_size, n_angles, flags, limit, limit, plans[1]))) return rc;
-            if ((rc = reserve_call(ctx, call, plans, 2))) return rc;
+            if (masked && (rc = plan_pm(ctx, img_size, n_angles, flags, max_border, max_border, plans[2], true))) return rc;
+            if ((rc = reserve_call(ctx, call, plans, masked ? 3 : 2))) return rc;
             if ((rc = enqueue_pm(ctx, call, plans[0], n_big, d_big, ctx->stream, 0, 0, false))) return rc;
-            return enqueue_pm(ctx, call, plans[1], n_small, d_small, ctx->stream, 0, n_big, true);
+            if ((rc = enqueue_pm(ctx, call, plans[1], n_small, d_small, ctx->stream, 0, n_big, true))) return rc;
+            return masked ? enqueue_pm(ctx, call, plans[2], n, nullptr, ctx->stream, 0, 0, true) : SID_OK;
         }
         if (n_big == 0) max_border = limit;              // every point fits the pipeline kernel
     }
     if ((rc = plan_pm(ctx, img_size, n_angles, flags, max_border, max_border, plans[0]))) return rc;
-    if ((rc = reserve_call(ctx, call, plans, 1))) return rc;
-    return enqueue_pm(ctx, call, plans[0], n, nullptr, ctx->stream, 0, 0, false);
+    if (masked && (rc = plan_pm(ctx, img_size, n_angles, flags, max_border, max_border, plans[1], true))) return rc;
+    if ((rc = reserve_call(ctx, call, plans, masked ? 2 : 1))) return rc;
+    if ((rc = enqueue_pm(ctx, call, plans[0], n, nullptr, ctx->stream, 0, 0, false))) return rc;
+    return masked ? enqueue_pm(ctx, call, plans[1], n, nullptr, ctx->stream, 0, 0, true) : SID_OK;
 }
 
 // ------------------------------------------------------------------ winning maps and templates (sid_run_maps)
@@ -1715,6 +1766,23 @@ int sid_rotate_and_match(sid_ctx *ctx, const uint8_t *img1, int rows1, int cols1
     CU(cudaGetLastError());
     *valid = 1;
     for (int a = 0; a < n_angles; ++a) if (hstats[(size_t)a * 3 + 2]) *valid = 0;
+    // SID_MASKED: a template holds a 0 pixel; the masked rule takes the point when every template qualifies
+    std::vector<long long> mstat;                                     // n, St, Stt per angle
+    if (!*valid && (flags & SID_MASKED)) {
+        std::vector<uint8_t> htpl((size_t)n_angles * s * s);
+        CU(cudaMemcpy(htpl.data(), d_tpl, htpl.size(), cudaMemcpyDeviceToHost));
+        mstat.resize((size_t)n_angles * 3);
+        bool ok = true;
+        for (int a = 0; a < n_angles; ++a) {
+            long long cnt = 0;
+            for (int k = 0; k < s * s; ++k) cnt += htpl[(size_t)a * s * s + k] != 0;
+            long long *m = &mstat[(size_t)a * 3];
+            m[0] = cnt; m[1] = hstats[(size_t)a * 3]; m[2] = hstats[(size_t)a * 3 + 1];
+            ok = ok && masked_template_ok(s, m[0], m[1], m[2]);
+        }
+        if (ok) *valid = 2;
+        else mstat.clear();
+    }
     if (!*valid) {
         *dc = NAN; *dr = NAN; *best_angle_idx = -1; *best_r = NAN; *best_h = NAN;
         return SID_OK;
@@ -1723,9 +1791,18 @@ int sid_rotate_and_match(sid_ctx *ctx, const uint8_t *img1, int rows1, int cols1
     // angle order, like the reference loop pmlib.py:155-166)
     for (int a = 0; a < n_angles; ++a) {
         float *d_map = d_maps + (size_t)a * mstride;
-        rc = match_on_device(ctx, (const uint8_t *)ctx->img2.p, H, W, dp2, d_tpl + (size_t)a * s * s, s, s, s,
-                             d_isum, d_isq, a > 0, d_ts, d_map);
-        if (rc) return rc;
+        if (!mstat.empty()) {
+            const long long *m = &mstat[(size_t)a * 3];
+            const unsigned grid = (unsigned)std::min<size_t>((rr + 255) / 256, (size_t)ctx->sm_count * 8);
+            masked_map_kernel<<<grid, 256, 0, ctx->stream>>>((const uint8_t *)ctx->img2.p, H, W, dp2, d_tpl + (size_t)a * s * s, s,
+                                                           m[0], m[1], m[2], d_map);
+            ctx->launches += 1;
+            CU(cudaGetLastError());
+        } else {
+            rc = match_on_device(ctx, (const uint8_t *)ctx->img2.p, H, W, dp2, d_tpl + (size_t)a * s * s, s, s, s,
+                                 d_isum, d_isq, a > 0, d_ts, d_map);
+            if (rc) return rc;
+        }
         argmax_kernel<<<1, 1024, 0, ctx->stream>>>(d_map, (int)rr, d_key + a);
         ctx->launches += 1;
     }

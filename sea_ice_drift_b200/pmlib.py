@@ -82,11 +82,16 @@ def rotate_and_match(img1, c1, r1, img_size, image2, alpha0,
 
     ``subpixel=True`` (extension): ``dc`` / ``dr`` refined to sub-pixel precision by a parabola through the peak of
     ``best_result`` and its two neighbours per axis (``SID_SUBPIXEL``, include/sid_b200.h); needs the built-in
-    matcher."""
+    matcher.
+
+    ``masked=True`` (extension): where a template holds a 0 pixel, match by the Pearson correlation over the
+    templates' valid pixels instead of returning NaNs, when every angle's template has at least half its pixels valid
+    and is not flat (``SID_MASKED``, include/sid_b200.h); needs the built-in matcher."""
     rot_order = kwargs.get('rot_order', 0)
-    if kwargs.get('subpixel') and not _is_builtin_matcher(template_matcher):
-        raise ValueError("subpixel=True needs the built-in matcher (template_matcher None, match_template or "
-                         "cv2.matchTemplate)")
+    for option in ('subpixel', 'masked'):
+        if kwargs.get(option) and not _is_builtin_matcher(template_matcher):
+            raise ValueError("%s=True needs the built-in matcher (template_matcher None, match_template or "
+                             "cv2.matchTemplate)" % option)
     flags = flags_from_options(dict(kwargs, mcc_norm=mcc_norm))
     ctx = _ctx(kwargs)
     if _is_builtin_matcher(template_matcher):
@@ -129,10 +134,15 @@ def use_mcc_batch(c1, r1, c2fg, r2fg, border, img1, img2, img_size, alpha0, **kw
 
     ``subpixel=True`` (extension): ``c2`` / ``r2`` refined to sub-pixel precision on the device by a parabola through
     the peak of the winning map and its two neighbours per axis (``SID_SUBPIXEL``, include/sid_b200.h); the other
-    columns, the NaN rows and the maps of ``return_maps`` are unchanged.  Needs the built-in matcher."""
+    columns, the NaN rows and the maps of ``return_maps`` are unchanged.  Needs the built-in matcher.
+
+    ``masked=True`` (extension): rows that are NaN because a template holds a 0 pixel (land, no-data) are matched by
+    the Pearson correlation over the templates' valid pixels where every angle's template has at least
+    ``ceil(img_size**2 / 2)`` valid pixels and is not flat (``SID_MASKED``, include/sid_b200.h); ``return_maps`` then
+    gives their masked maps and templates.  Every other row is unchanged.  Needs the built-in matcher."""
     matcher = kwargs.get('template_matcher')
     return_maps = kwargs.get('return_maps', False)
-    for option in ('return_maps', 'subpixel'):
+    for option in ('return_maps', 'subpixel', 'masked'):
         if kwargs.get(option) and not _is_builtin_matcher(matcher):
             raise ValueError("%s=True needs the built-in matcher (template_matcher None, match_template or "
                              "cv2.matchTemplate)" % option)
@@ -470,7 +480,9 @@ def pattern_matching(lon_pm1, lat_pm1, n1, c1, r1, n2, c2, r2,
     compatibility and ignored: all grid points go through one GPU launch (or one
     launch per rank when ``torch.distributed`` is initialised, see sharding.py).
 
-    ``subpixel=True`` (extension): sub-pixel drift vectors (see :func:`use_mcc_batch`)."""
+    ``subpixel=True`` (extension): sub-pixel drift vectors (see :func:`use_mcc_batch`).
+    ``masked=True`` (extension): vectors next to land and no-data from the masked correlation (see
+    :func:`use_mcc_batch`)."""
     t0 = time.time()
     img1, img2 = n1[1], n2[1]
     dst_shape = lon_pm1.shape
