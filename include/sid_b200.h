@@ -76,6 +76,21 @@ typedef struct sid_ctx sid_ctx;
  * vt > 0 for every angle; its status is SID_PT_MASKED.  Winner, h, mcc_norm, hes_smth and SID_SUBPIXEL follow the usual
  * rules on the masked float maps.  Every other row is bit-identical to the call without the flag. */
 #define SID_MASKED 16u
+/* SID_PEAKS (extension, not in the reference): also record, for every row, the SID_N_PEAKS next-best peaks of its winning
+ * map, for the outlier filter (sid_filter_outliers).  m is the row's RAW float32 winning-angle map, RH x RW (the map
+ * sid_run_maps returns), flat index f(i, j) = i RW + j.  p is a PEAK when every in-map 8-neighbour q has m[q] < m[p] if
+ * f(q) < f(p) and m[q] <= m[p] if f(q) > f(p): a plateau counts once, at its first index (np.argmax's rule; the primary
+ * peak is always one).  The SECONDARY peaks are all peaks but the primary, by m descending, ties by f ascending; the first
+ * SID_N_PEAKS are kept, each as four doubles c2, r2, r, h computed exactly as the row computes its own:
+ *   c2 = c2fg + (j - (W - s) / 2), r2 = r2fg + (i - (H - s) / 2), plus peak_offsets at (i, j) with SID_SUBPIXEL;
+ *   r = m[p], or (m[p] - median m) / std m under mcc_norm, in float32 as the row's r;
+ *   h = get_hessian(m, hes_norm, hes_smth)[p], normalised with the median and std that normalised the row's h.
+ * Missing peaks (fewer than SID_N_PEAKS; a flat template's all-1.0 map has none) and rows that are neither SID_PT_VALID nor
+ * SID_PT_MASKED get NaN records.  Every sid_run* honours it; the table, status and maps are bit-identical to the call
+ * without it; sid_get_peaks copies the records out, and sid_filter_outliers reads them on the device.
+ * sid_rotate_and_match refuses it (SID_EUNSUPPORTED). */
+#define SID_PEAKS 32u
+#define SID_N_PEAKS 3
 
 /* point status written by sid_run* (optional output) */
 #define SID_PT_VALID 1
@@ -142,6 +157,31 @@ int sid_pm_epilogue_affine(sid_ctx *ctx, int64_t n_valid, const int32_t *grid_in
                            const double *c2pm1, const double *r2pm1, const double *results,
                            const double *xy, const double *ll, double *out);
 
+/* SID_PEAKS records of the previous sid_run* call: out = n x SID_N_PEAKS x 4 doubles (c2, r2, r, h per peak, rank order,
+ * NaN where missing), host pointer, synchronous.  SID_EINVAL (context stays usable) when that call did not set SID_PEAKS
+ * or had a different n. */
+int sid_get_peaks(sid_ctx *ctx, int64_t n, double *out);
+
+/* Normalised median test (Westerweel & Scarano 2005, "universal outlier detection") over the grid of a result table, with
+ * replacement by a secondary peak (SID_PEAKS), on the device.  Every operation is an IEEE double op without contraction.
+ *   grid_rows x grid_cols  the grid; n_valid, grid_index, c2pm1, r2pm1 as for sid_pm_epilogue_affine (n_grid = rows x cols)
+ *   results, peaks         host (n_valid, 5) table and (n_valid, SID_N_PEAKS, 4) records, or both NULL: what the previous
+ *                          sid_run / sid_run_pair / sid_run_maps left on the device (it must have set SID_PEAKS)
+ *   out                    host (n_valid, 5) filtered table; NULL (device-resident inputs only) updates the device table
+ *                          in place, so that sid_pm_epilogue_affine(results = NULL) reads the filtered table
+ *   flag                   optional host n_valid ints (below)
+ * Rule, decided on the unfiltered table in one pass.  Displacement of a row at grid position g:
+ * d = (c2 - rint(c2pm1[g]), r2 - rint(r2pm1[g])) (rint: ties to even).  Neighbours: the in-grid 8-neighbours of g whose row
+ * has a finite c2.  With k < 3 neighbours the row is kept, flag -2.  Per axis: m = median of the neighbours' d ((a + b) *
+ * 0.5 of the middle two for even k), r_m = median of |d_i - m|, e = |d0 - m| / (r_m + eps).  The row is an outlier iff
+ * e_x^2 + e_y^2 > threshold^2; it then takes the first finite secondary peak, in rank order, that passes the same test
+ * against the same m and r_m (its c2, r2, r, h; angle unchanged; flag = its rank 1 ... SID_N_PEAKS), else it becomes a NaN
+ * row, flag -1.  Kept rows: flag 0; NaN rows: flag -3.  Suggested eps 1.0 px, threshold 2.0. */
+int sid_filter_outliers(sid_ctx *ctx, int grid_rows, int grid_cols, int64_t n_valid, const int32_t *grid_index,
+                        const double *c2pm1, const double *r2pm1,
+                        const double *results, const double *peaks,
+                        double eps, double threshold, double *out, int32_t *flag);
+
 /* Asynchronous 2-D host -> device copy of `rows` image rows on the context's stream (a rank's row slab of the
  * pair, before the all-gather that completes the adopted buffers). */
 int sid_upload_rows(sid_ctx *ctx, uint8_t *d_dst, int64_t dst_pitch, const uint8_t *src, int64_t src_pitch, int cols, int rows);
@@ -159,7 +199,7 @@ int sid_downsample_pair(sid_ctx *ctx, int factor,
                         uint8_t *d_img1, int64_t pitch1, int64_t bytes1,
                         uint8_t *d_img2, int64_t pitch2, int64_t bytes2);
 
-/* use_mcc for n grid points (host arrays in, host array out, synchronous).  All sid_run* honour SID_MASKED.
+/* use_mcc for n grid points (host arrays in, host array out, synchronous).  All sid_run* honour SID_MASKED and SID_PEAKS.
  *   c1, r1        float pixel coordinates on image 1
  *   c2fg, r2fg    integer-valued first guess on image 2
  *   border        integer-valued search radius per point

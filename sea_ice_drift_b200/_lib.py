@@ -21,6 +21,8 @@ SID_TM_CCOEFF_NORMED = 5
 SID_HES_NORM, SID_HES_SMTH, SID_MCC_NORM = 1, 2, 4
 SID_SUBPIXEL = 8                # extension: sub-pixel c2 / r2 (include/sid_b200.h)
 SID_MASKED = 16                 # extension: masked correlation for templates with 0 pixels (include/sid_b200.h)
+SID_PEAKS = 32                  # extension: the secondary peaks of every row's winning map (include/sid_b200.h)
+SID_N_PEAKS = 3                 # secondary peaks recorded per row
 SID_PT_VALID = 1                # point status of a valid row (sid_run*)
 SID_PT_MASKED = 2               # point status of a row matched by the masked rule (SID_MASKED)
 
@@ -28,7 +30,7 @@ EXPORTS = [
     "sid_version", "sid_create", "sid_destroy", "sid_last_error", "sid_set_stream", "sid_synchronize",
     "sid_set_pair", "sid_set_pair_device", "sid_pair_layout", "sid_adopt_pair_device", "sid_upload_rows", "sid_pm_epilogue_affine", "sid_first_guess", "sid_run", "sid_run_pair", "sid_run_device", "sid_map_layout", "sid_run_maps", "sid_launch_count", "sid_last_kernel_ms", "sid_last_kernel_name",
     "sid_rotate_and_match", "sid_get_template", "sid_match_template", "sid_get_hessian", "sid_knn_hamming2",
-    "sid_deformation", "sid_downsample_pair",
+    "sid_deformation", "sid_downsample_pair", "sid_get_peaks", "sid_filter_outliers",
 ]
 
 _lib = None
@@ -96,6 +98,9 @@ def load_library():
         lib.sid_knn_hamming2.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
         lib.sid_get_hessian.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_uint, C.c_void_p]
         lib.sid_deformation.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 4 + [C.c_int] + [C.c_void_p] * 7
+        lib.sid_get_peaks.argtypes = [C.c_void_p, C.c_int64, C.c_void_p]
+        lib.sid_filter_outliers.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int64] + [C.c_void_p] * 5 + \
+            [C.c_double, C.c_double, C.c_void_p, C.c_void_p]
         _lib = lib
         return lib
 
@@ -256,6 +261,45 @@ class Context(object):
             self._h, idx.size, idx.ctypes.data, gpi.size, c.ctypes.data, r.ctypes.data,
             None if res is None else res.ctypes.data, xy.ctypes.data, ll.ctypes.data, out.ctypes.data))
         return out
+
+    def peaks(self, n):
+        """The SID_PEAKS records of the previous run (sid_get_peaks): an (n, SID_N_PEAKS, 4) float64 array of c2, r2,
+        r, h per secondary peak, rank order, NaN where missing."""
+        out = np.empty((int(n), SID_N_PEAKS, 4), dtype=np.float64)
+        self._check(self._lib.sid_get_peaks(self._h, int(n), out.ctypes.data))
+        return out
+
+    def filter_outliers(self, grid_shape, gpi, c2pm1, r2pm1, results=None, peaks=None, eps=1.0, threshold=2.0,
+                        in_place=False):
+        """Normalised median test with secondary-peak replacement (sid_filter_outliers) on a ``grid_shape`` (rows,
+        cols) grid whose valid points are ``gpi`` (flat or grid-shaped, table order = row-major order of the True
+        positions).  ``results`` / ``peaks`` None: the table and peaks the previous run left on the device.  Returns
+        ``(table, flags)``; with ``in_place`` (device-resident inputs only) the device table is updated and ``table`` is
+        None."""
+        rows, cols = (int(v) for v in grid_shape)
+        gpi = np.asarray(gpi, dtype=bool).ravel()
+        if gpi.size != rows * cols:
+            raise ValueError("gpi must have grid_shape's number of elements")
+        idx = np.ascontiguousarray(np.flatnonzero(gpi), dtype=np.int32)
+        c = np.ascontiguousarray(c2pm1, dtype=np.float64).ravel()
+        r = np.ascontiguousarray(r2pm1, dtype=np.float64).ravel()
+        if c.size != gpi.size or r.size != gpi.size:
+            raise ValueError("c2pm1 / r2pm1 must have one value per grid point")
+        if (results is None) != (peaks is None):
+            raise ValueError("pass both results and peaks, or neither")
+        res = pk = None
+        if results is not None:
+            res = np.ascontiguousarray(results, dtype=np.float64).reshape(-1, 5)
+            pk = np.ascontiguousarray(peaks, dtype=np.float64).reshape(-1, SID_N_PEAKS, 4)
+            if res.shape[0] != idx.size or pk.shape[0] != idx.size:
+                raise ValueError("results / peaks need one row per valid grid point")
+        out = None if in_place else np.empty((idx.size, 5), dtype=np.float64)
+        flags = np.empty(idx.size, dtype=np.int32)
+        self._check(self._lib.sid_filter_outliers(
+            self._h, rows, cols, idx.size, idx.ctypes.data, c.ctypes.data, r.ctypes.data,
+            None if res is None else res.ctypes.data, None if pk is None else pk.ctypes.data, float(eps),
+            float(threshold), None if out is None else out.ctypes.data, flags.ctypes.data))
+        return out, flags
 
     def first_guess(self, sx, sy, vx, vy, kx, ky, qx, qy):
         """Delaunay-linear interpolation of (vx, vy) from the sources (sx, sy) onto (qx, qy) and the distance of every

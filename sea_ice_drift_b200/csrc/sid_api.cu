@@ -111,6 +111,10 @@ struct sid_ctx {
     DevBuf pts, order, out, status, angles, scratch, counter, misc, tail_maps, tail_recs, epi, fg;
     DevBuf maps, map_off, tpl;               // sid_run_maps: packed maps, their offsets, the templates
     DevBuf cand;                             // SID_MASKED: the candidate rows of the masked pass
+    DevBuf peaks;                            // SID_PEAKS: n x SID_N_PEAKS x 4 doubles of the last sid_run* call
+    long long peaks_n = -1;                  // its n, or -1 when the last sid_run* call did not set SID_PEAKS
+    bool peaks_of_table = false;             // that call was the sid_run / sid_run_pair / sid_run_maps that left `out`
+    DevBuf filt;                             // sid_filter_outliers
     void *pin = nullptr;
     size_t pin_cap = 0;
     cudaEvent_t k_ev[2] = {};                // bracket the last fused-kernel launch (sid_last_kernel_ms)
@@ -300,7 +304,7 @@ int plan_pm(sid_ctx *ctx, int s, int n_angles, unsigned flags, int max_border, i
     a.max_hrw = Wmax * Rmax;
     if (masked) {
         p.kernel = PM_MASKED;
-        p.kfn = (const void *)pm_masked_kernel;
+        p.kfn = (flags & SID_PEAKS) ? (const void *)pm_masked_kernel<true> : (const void *)pm_masked_kernel<false>;
         p.name = "sid::pm_masked_kernel";
         p.threads = PM_MASKED_THREADS;
         a.scratch_per_cta = pm_masked_scratch_bytes(a.max_rr);
@@ -323,7 +327,8 @@ int plan_pm(sid_ctx *ctx, int s, int n_angles, unsigned flags, int max_border, i
     p.tail_threads = pm_tail_threads(a.max_rr);
     p.tail_smem = pm_tail_smem_bytes(a.max_rr, smth);
     if (split_tail)
-        if (int arc = allow_max_smem(ctx, (const void *)pm_tail_kernel)) return arc;
+        if (int arc = allow_max_smem(ctx, (flags & SID_PEAKS) ? (const void *)pm_tail_kernel<true> : (const void *)pm_tail_kernel<false>))
+            return arc;
     // warp-specialised pipeline kernel (sid_pm_ws_kernel.cuh): small result maps (geometry: radius <= 24; its shared-memory
     // layout fits 227 KB up to radius 20 at s = 35, 22 with two sets of window statistics), needs the split tail
     if (ws_wanted() && split_tail) {
@@ -375,10 +380,16 @@ int plan_pm(sid_ctx *ctx, int s, int n_angles, unsigned flags, int max_border, i
         if (p.smem > (size_t)ctx->max_smem_optin - 4096 - (p.smem_scratch ? 0 : 8192)) use_tc = false;      // window too large: legacy kernels
                                                                           // (the global-scratch variant has 8 KB more static shared memory)
     }
-    const void *ktab[8] = {(const void *)pm_points_kernel<9, false, false>, (const void *)pm_points_kernel<13, false, false>,
-                           (const void *)pm_points_kernel<0, false, false>, (const void *)pm_points_kernel<9, true, false>,
-                           (const void *)pm_points_kernel<13, true, false>, (const void *)pm_points_kernel<0, true, false>,
-                           (const void *)pm_points_kernel<0, false, true>, (const void *)pm_points_kernel<0, true, true>};
+    // [8 ... 15]: the same kernels with SID_PEAKS
+    const void *ktab[16] = {(const void *)pm_points_kernel<9, false, false, false>, (const void *)pm_points_kernel<13, false, false, false>,
+                            (const void *)pm_points_kernel<0, false, false, false>, (const void *)pm_points_kernel<9, true, false, false>,
+                            (const void *)pm_points_kernel<13, true, false, false>, (const void *)pm_points_kernel<0, true, false, false>,
+                            (const void *)pm_points_kernel<0, false, true, false>, (const void *)pm_points_kernel<0, true, true, false>,
+                            (const void *)pm_points_kernel<9, false, false, true>, (const void *)pm_points_kernel<13, false, false, true>,
+                            (const void *)pm_points_kernel<0, false, false, true>, (const void *)pm_points_kernel<9, true, false, true>,
+                            (const void *)pm_points_kernel<13, true, false, true>, (const void *)pm_points_kernel<0, true, false, true>,
+                            (const void *)pm_points_kernel<0, false, true, true>, (const void *)pm_points_kernel<0, true, true, true>};
+    const int kpeaks = (flags & SID_PEAKS) ? 8 : 0;
     // the legacy kernel of this launch in ktab: mma.sync (imma) or a dp4a specialisation, per-point scratch in shared or global memory
     auto legacy_kidx = [&](bool smem_scr) { return imma ? (smem_scr ? 7 : 6) : variant + (smem_scr ? 3 : 0); };
     if (!use_tc) {
@@ -426,7 +437,7 @@ int plan_pm(sid_ctx *ctx, int s, int n_angles, unsigned flags, int max_border, i
         // angles per batch nor refused here, and failed the occupancy check below with SID_ECUDA instead (measured on a
         // B200: img_size 35, 3 angles, borders 206, 207, 209 and 210; img_size 128, 3 angles, borders 124 and 125)
         cudaFuncAttributes fa;
-        CU(cudaFuncGetAttributes(&fa, ktab[legacy_kidx(false)]));
+        CU(cudaFuncGetAttributes(&fa, ktab[kpeaks + legacy_kidx(false)]));
         const size_t smem_max = (size_t)ctx->max_smem_optin - fa.sharedSizeBytes;
         p.smem = base_smem(a.ab);
         while (p.smem > smem_max && a.ab > 1) { --a.ab; p.smem = base_smem(a.ab); }
@@ -465,7 +476,7 @@ int plan_pm(sid_ctx *ctx, int s, int n_angles, unsigned flags, int max_border, i
     }
 
     p.kidx = use_tc ? (p.smem_scratch ? 9 : 8) : legacy_kidx(p.smem_scratch);
-    p.kfn = use_tc ? (p.smem_scratch ? (const void *)pm_tc_kernel<true> : (const void *)pm_tc_kernel<false>) : ktab[p.kidx];
+    p.kfn = use_tc ? (p.smem_scratch ? (const void *)pm_tc_kernel<true> : (const void *)pm_tc_kernel<false>) : ktab[kpeaks + p.kidx];
     if (int arc = allow_max_smem(ctx, p.kfn)) return arc;
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&p.occ, p.kfn, p.threads, p.smem));
     if (p.occ < 1) {
@@ -508,6 +519,7 @@ struct PmCall {
     // set by reserve_call
     size_t tail_stride;              // floats per point of the tail hand-off regions
     size_t scratch_slot;             // bytes of global scratch per band stream
+    double *peaks = nullptr;         // SID_PEAKS only, see PmArgs::peaks
 };
 
 // The buffers the launches of a call share, reserved once before the first launch, so that none of them is reallocated
@@ -562,6 +574,7 @@ int enqueue_pm(sid_ctx *ctx, const PmCall &call, const PmPlan &p, long long n, c
     a.angles = call.angles; a.tab = call.tab; a.rot_order = call.rot_order;
     a.out = call.out; a.status = call.status;
     a.maps_out = call.maps_out; a.map_off = call.map_off; a.tpl_out = call.tpl_out;
+    a.peaks = call.peaks;
     a.counter = (unsigned int *)ctx->counter.p + 16 * slot;
     a.scratch = (unsigned char *)ctx->scratch.p + call.scratch_slot * (size_t)slot;      // read by the global-scratch variants only
     if (a.split_tail) {
@@ -628,7 +641,8 @@ int enqueue_pm(sid_ctx *ctx, const PmCall &call, const PmPlan &p, long long n, c
 #endif
     if (a.split_tail) {
         if (debug) fprintf(stderr, "[sid] launch: tail threads=%d smem=%zu\n", p.tail_threads, p.tail_smem);
-        pm_tail_kernel<<<(unsigned)n, p.tail_threads, p.tail_smem, st>>>(a);
+        if (a.peaks) pm_tail_kernel<true><<<(unsigned)n, p.tail_threads, p.tail_smem, st>>>(a);
+        else pm_tail_kernel<false><<<(unsigned)n, p.tail_threads, p.tail_smem, st>>>(a);
         ctx->launches += 1;
         CU(cudaGetLastError());
     }
@@ -946,6 +960,8 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
              float *maps_out, const long long *map_off, uint8_t *tpl_out) {
     int rc = check_common(ctx, img_size, n_angles, angle_tab, rot_order, mtype);
     if (rc) return rc;
+    ctx->peaks_n = -1;
+    ctx->peaks_of_table = false;
     if (!pair && !ctx->have_pair) return fail(ctx, SID_ENOPAIR, "sid_set_pair has not been called");
     if (n < 0 || (n > 0 && (!c1 || !r1 || !c2fg || !r2fg || !border)) || !angles)
         return fail(ctx, SID_EINVAL, "null point array");
@@ -955,10 +971,18 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
         if (!pair->img1 || !pair->img2 || pair->rows1 <= 0 || pair->cols1 <= 0 || pair->rows2 <= 0 || pair->cols2 <= 0 ||
             pair->pitch1 < pair->cols1 || pair->pitch2 < pair->cols2)
             return fail(ctx, SID_EINVAL, "bad image arguments");
-        if (n == 0) return sid_set_pair(ctx, pair->img1, pair->rows1, pair->cols1, pair->pitch1, pair->img2, pair->rows2,
-                                        pair->cols2, pair->pitch2);
+        if (n == 0) {
+            if ((rc = sid_set_pair(ctx, pair->img1, pair->rows1, pair->cols1, pair->pitch1, pair->img2, pair->rows2,
+                                   pair->cols2, pair->pitch2)))
+                return rc;
+            ctx->peaks_n = (flags & SID_PEAKS) ? 0 : -1;
+            return SID_OK;
+        }
     }
-    if (n == 0) return SID_OK;
+    if (n == 0) {
+        ctx->peaks_n = (flags & SID_PEAKS) ? 0 : -1;
+        return SID_OK;
+    }
 
     // ---- bands (upload granularity); a single band means "everything is already resident".  The bands TAPER: while the
     //      upload runs the kernels of band k hide behind the copy of band k + 1, but the kernels of the LAST band run after
@@ -1138,6 +1162,7 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
     if ((rc = reserve(ctx, ctx->order, ord_bytes))) return rc;
     if ((rc = reserve(ctx, ctx->out, out_bytes))) return rc;
     if ((rc = reserve(ctx, ctx->status, st_bytes))) return rc;
+    if ((flags & SID_PEAKS) && (rc = reserve(ctx, ctx->peaks, (size_t)n * SID_N_PEAKS * 4 * sizeof(double)))) return rc;
 
     double *hp = (double *)ctx->pin;
     memcpy(hp, c1, (size_t)n * 8); memcpy(hp + n, r1, (size_t)n * 8); memcpy(hp + 2 * n, c2fg, (size_t)n * 8);
@@ -1154,6 +1179,8 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
     CU(cudaMemcpyAsync(ctx->order.p, hord, ord_bytes, cudaMemcpyHostToDevice, up));
     const double *d_angles, *d_tab;
     if ((rc = upload_angles(ctx, n_angles, angles, angle_tab, &d_angles, &d_tab, up))) return rc;
+    // rows that end up neither valid nor masked keep NaN (all bits set) peak records
+    if (flags & SID_PEAKS) CU(cudaMemsetAsync(ctx->peaks.p, 0xff, (size_t)n * SID_N_PEAKS * 4 * sizeof(double), up));
     if (!ctx->slot_event[0])
         for (int k = 0; k < 3; ++k) CU(cudaEventCreateWithFlags(&ctx->slot_event[k], cudaEventDisableTiming));
     CU(cudaEventRecord(ctx->slot_event[0], up));                       // point / angle uploads are enqueued
@@ -1164,6 +1191,7 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
     const double *dp = (const double *)ctx->pts.p;
     PmCall call{dp, dp + n, dp + 2 * n, dp + 3 * n, dp + 4 * n, d_angles, d_tab, rot_order, (double *)ctx->out.p,
                 (int *)ctx->status.p, maps_out, map_off, tpl_out, n, 0, 0};
+    if (flags & SID_PEAKS) call.peaks = (double *)ctx->peaks.p;
     // the larger borders (all points when the call is not split into classes), the class of pm_ws_kernel, the masked pass
     PmPlan plans[3];
     const bool masked = (flags & SID_MASKED) != 0;
@@ -1210,6 +1238,7 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
     CU(cudaGetLastError());
     if (out) memcpy(out, hout, out_bytes);
     if (status) memcpy(status, hst, st_bytes);
+    if (flags & SID_PEAKS) { ctx->peaks_n = n; ctx->peaks_of_table = true; }
     return SID_OK;
 }
 
@@ -1239,10 +1268,15 @@ int sid_run_device(sid_ctx *ctx, int64_t n, const double *d_c1, const double *d_
                    double *d_out, int *d_status) {
     int rc = check_common(ctx, img_size, n_angles, angle_tab, rot_order, mtype);
     if (rc) return rc;
+    ctx->peaks_n = -1;
+    ctx->peaks_of_table = false;
     if (!ctx->have_pair) return fail(ctx, SID_ENOPAIR, "sid_set_pair has not been called");
     if (n < 0 || (n > 0 && (!d_c1 || !d_r1 || !d_c2fg || !d_r2fg || !d_border || !d_out)) || !angles)
         return fail(ctx, SID_EINVAL, "null point array");
-    if (n == 0) return SID_OK;
+    if (n == 0) {
+        ctx->peaks_n = (flags & SID_PEAKS) ? 0 : -1;
+        return SID_OK;
+    }
     CU(cudaSetDevice(ctx->device));
     if (max_border <= 0) {
         std::vector<double> hb((size_t)n);
@@ -1254,6 +1288,12 @@ int sid_run_device(sid_ctx *ctx, int64_t n, const double *d_c1, const double *d_
     const double *d_angles, *d_tab;
     if ((rc = upload_angles(ctx, n_angles, angles, angle_tab, &d_angles, &d_tab))) return rc;
     PmCall call{d_c1, d_r1, d_c2fg, d_r2fg, d_border, d_angles, d_tab, rot_order, d_out, d_status, nullptr, nullptr, nullptr, n, 0, 0};
+    if (flags & SID_PEAKS) {
+        const size_t b = (size_t)n * SID_N_PEAKS * 4 * sizeof(double);
+        if ((rc = reserve(ctx, ctx->peaks, b))) return rc;
+        CU(cudaMemsetAsync(ctx->peaks.p, 0xff, b, ctx->stream));
+        call.peaks = (double *)ctx->peaks.p;
+    }
     PmPlan plans[3];                 // [0], [1]: the border classes; the masked pass behind them
     const bool masked = (flags & SID_MASKED) != 0;
     // border classes as in sid_run (see run_host): the indices are split on the device, one 8-byte read-back sizes the launches
@@ -1277,7 +1317,9 @@ int sid_run_device(sid_ctx *ctx, int64_t n, const double *d_c1, const double *d_
             if ((rc = reserve_call(ctx, call, plans, masked ? 3 : 2))) return rc;
             if ((rc = enqueue_pm(ctx, call, plans[0], n_big, d_big, ctx->stream, 0, 0, false))) return rc;
             if ((rc = enqueue_pm(ctx, call, plans[1], n_small, d_small, ctx->stream, 0, n_big, true))) return rc;
-            return masked ? enqueue_pm(ctx, call, plans[2], n, nullptr, ctx->stream, 0, 0, true) : SID_OK;
+            if (masked && (rc = enqueue_pm(ctx, call, plans[2], n, nullptr, ctx->stream, 0, 0, true))) return rc;
+            if (flags & SID_PEAKS) ctx->peaks_n = n;
+            return SID_OK;
         }
         if (n_big == 0) max_border = limit;              // every point fits the pipeline kernel
     }
@@ -1285,7 +1327,9 @@ int sid_run_device(sid_ctx *ctx, int64_t n, const double *d_c1, const double *d_
     if (masked && (rc = plan_pm(ctx, img_size, n_angles, flags, max_border, max_border, plans[1], true))) return rc;
     if ((rc = reserve_call(ctx, call, plans, masked ? 2 : 1))) return rc;
     if ((rc = enqueue_pm(ctx, call, plans[0], n, nullptr, ctx->stream, 0, 0, false))) return rc;
-    return masked ? enqueue_pm(ctx, call, plans[1], n, nullptr, ctx->stream, 0, 0, true) : SID_OK;
+    if (masked && (rc = enqueue_pm(ctx, call, plans[1], n, nullptr, ctx->stream, 0, 0, true))) return rc;
+    if (flags & SID_PEAKS) ctx->peaks_n = n;
+    return SID_OK;
 }
 
 // ------------------------------------------------------------------ winning maps and templates (sid_run_maps)
@@ -1326,6 +1370,8 @@ int sid_run_maps(sid_ctx *ctx, int64_t n, const double *c1, const double *r1, co
                  int64_t maps_capacity, float *maps, uint8_t *templates) {
     int rc = check_common(ctx, img_size, n_angles, angle_tab, rot_order, mtype);
     if (rc) return rc;
+    ctx->peaks_n = -1;
+    ctx->peaks_of_table = false;
     if (!angles) return fail(ctx, SID_EINVAL, "null point array");
     if (n > 0x7fffffffLL) return fail(ctx, SID_EINVAL, "too many points");
     std::vector<long long> off;
@@ -1333,7 +1379,10 @@ int sid_run_maps(sid_ctx *ctx, int64_t n, const double *c1, const double *r1, co
     if ((rc = map_layout(ctx, n, c1, r1, c2fg, r2fg, border, img_size, nullptr, &off, &total))) return rc;
     if (maps_capacity < total) return fail(ctx, SID_EINVAL, "maps_capacity below the total of sid_map_layout");
     if (total > 0 && !maps) return fail(ctx, SID_EINVAL, "null maps buffer");
-    if (n == 0) return SID_OK;
+    if (n == 0) {
+        ctx->peaks_n = (flags & SID_PEAKS) ? 0 : -1;
+        return SID_OK;
+    }
     CU(cudaSetDevice(ctx->device));
     const size_t tpl_bytes = (size_t)n * img_size * img_size;
     if ((rc = reserve(ctx, ctx->maps, (size_t)std::max<int64_t>(total, 1) * sizeof(float)))) return rc;
@@ -1410,6 +1459,150 @@ int sid_pm_epilogue_affine(sid_ctx *ctx, int64_t n_valid, const int32_t *grid_in
     ctx->launches += n_valid ? 2 : 1;
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(out, d_out, b_out, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    return SID_OK;
+}
+
+int sid_get_peaks(sid_ctx *ctx, int64_t n, double *out) {
+    if (!ctx) return SID_EINVAL;
+    if (n < 0 || ctx->peaks_n != n) return fail(ctx, SID_EINVAL, "the previous sid_run* call did not set SID_PEAKS for n points");
+    if (n > 0 && !out) return fail(ctx, SID_EINVAL, "null output pointer");
+    if (n == 0) return SID_OK;
+    CU(cudaSetDevice(ctx->device));
+    CU(cudaMemcpyAsync(out, ctx->peaks.p, (size_t)n * SID_N_PEAKS * 4 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    return SID_OK;
+}
+
+// ------------------------------------------------------------------ outlier filter (normalised median test)
+namespace {
+__global__ void outlier_index_kernel(long long n_valid, const int *gidx, int *inv) {
+    const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k < n_valid) inv[gidx[k]] = (int)k;
+}
+// median of v[0 .. k) (k <= 8), sorted in place; np.median's (a + b) * 0.5 of the middle two for even k
+__device__ __forceinline__ double median_small(double (&v)[8], int k) {
+    for (int i = 1; i < k; ++i) {
+        const double x = v[i];
+        int j = i - 1;
+        while (j >= 0 && v[j] > x) { v[j + 1] = v[j]; --j; }
+        v[j + 1] = x;
+    }
+    return (k & 1) ? v[k / 2] : __dmul_rn(__dadd_rn(v[k / 2 - 1], v[k / 2]), 0.5);
+}
+// e_x^2 + e_y^2 > threshold^2 against the neighbours' medians m and median residuals rm
+__device__ __forceinline__ bool outlier_test(double dx, double dy, const double (&m)[2], const double (&rm)[2], double eps,
+                                             double thr2) {
+    const double ex = __ddiv_rn(fabs(__dsub_rn(dx, m[0])), __dadd_rn(rm[0], eps));
+    const double ey = __ddiv_rn(fabs(__dsub_rn(dy, m[1])), __dadd_rn(rm[1], eps));
+    return __dadd_rn(__dmul_rn(ex, ex), __dmul_rn(ey, ey)) > thr2;
+}
+// One thread per table row: the rule of sid_filter_outliers (include/sid_b200.h).  Reads res / peaks, writes out / flag.
+__global__ void outlier_filter_kernel(long long n_valid, int grid_rows, int grid_cols, const int *gidx, const int *inv,
+                                      const double *c2pm1, const double *r2pm1, const double *res, const double *peaks,
+                                      double eps, double thr2, double *out, int *flag) {
+    const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n_valid) return;
+    const double *row = res + 5 * k;
+    double *o = out + 5 * k;
+    for (int c = 0; c < 5; ++c) o[c] = row[c];
+    if (!isfinite(row[0])) { flag[k] = -3; return; }
+    const int g = gidx[k], gr = g / grid_cols, gc = g - gr * grid_cols;
+    const double cg = rint(c2pm1[g]), rg = rint(r2pm1[g]);
+    double dx[8], dy[8];
+    int nn = 0;
+    for (int di = -1; di <= 1; ++di) {
+        for (int dj = -1; dj <= 1; ++dj) {
+            const int y = gr + di, x = gc + dj;
+            if ((di == 0 && dj == 0) || y < 0 || y >= grid_rows || x < 0 || x >= grid_cols) continue;
+            const int q = inv[y * grid_cols + x];
+            if (q < 0 || !isfinite(res[5 * (long long)q])) continue;
+            const int gq = y * grid_cols + x;
+            dx[nn] = __dsub_rn(res[5 * (long long)q], rint(c2pm1[gq]));
+            dy[nn] = __dsub_rn(res[5 * (long long)q + 1], rint(r2pm1[gq]));
+            ++nn;
+        }
+    }
+    if (nn < 3) { flag[k] = -2; return; }
+    double m[2], rm[2];
+    m[0] = median_small(dx, nn);
+    m[1] = median_small(dy, nn);
+    for (int i = 0; i < nn; ++i) { dx[i] = fabs(__dsub_rn(dx[i], m[0])); dy[i] = fabs(__dsub_rn(dy[i], m[1])); }
+    rm[0] = median_small(dx, nn);
+    rm[1] = median_small(dy, nn);
+    if (!outlier_test(__dsub_rn(row[0], cg), __dsub_rn(row[1], rg), m, rm, eps, thr2)) { flag[k] = 0; return; }
+    for (int r = 0; r < SID_N_PEAKS; ++r) {
+        const double *pk = peaks + (12 * k + 4 * r);
+        if (!isfinite(pk[0])) continue;
+        if (outlier_test(__dsub_rn(pk[0], cg), __dsub_rn(pk[1], rg), m, rm, eps, thr2)) continue;
+        o[0] = pk[0]; o[1] = pk[1]; o[3] = pk[2]; o[4] = pk[3];
+        flag[k] = r + 1;
+        return;
+    }
+    for (int c = 0; c < 5; ++c) o[c] = nan("");
+    flag[k] = -1;
+}
+}  // namespace
+
+int sid_filter_outliers(sid_ctx *ctx, int grid_rows, int grid_cols, int64_t n_valid, const int32_t *grid_index,
+                        const double *c2pm1, const double *r2pm1, const double *results, const double *peaks,
+                        double eps, double threshold, double *out, int32_t *flag) {
+    if (!ctx) return SID_EINVAL;
+    const long long n_grid = (long long)grid_rows * (long long)grid_cols;
+    if (grid_rows <= 0 || grid_cols <= 0 || n_grid > 0x7fffffffLL || n_valid < 0 || n_valid > n_grid ||
+        (n_valid > 0 && !grid_index) || !c2pm1 || !r2pm1)
+        return fail(ctx, SID_EINVAL, "bad outlier filter arguments");
+    if (!(eps >= 0.0) || !(threshold >= 0.0) || !std::isfinite(eps) || !std::isfinite(threshold))
+        return fail(ctx, SID_EINVAL, "eps and threshold must be finite and >= 0");
+    const bool resident = !results && !peaks;
+    if (!resident && (!results || !peaks)) return fail(ctx, SID_EINVAL, "pass both results and peaks, or neither");
+    if (resident && (ctx->table_n != n_valid || ctx->peaks_n != n_valid || !ctx->peaks_of_table))
+        return fail(ctx, SID_EINVAL, "no device table with SID_PEAKS of that length (run sid_run / sid_run_pair with SID_PEAKS first)");
+    if (!out && !resident) return fail(ctx, SID_EINVAL, "out may be NULL only with the device-resident inputs");
+    {   // every grid position once, inside the grid: the scatter below must not race or write out of bounds
+        std::vector<unsigned char> seen((size_t)n_grid, 0);
+        for (int64_t k = 0; k < n_valid; ++k) {
+            const int32_t g = grid_index[k];
+            if (g < 0 || g >= n_grid || seen[(size_t)g]) return fail(ctx, SID_EINVAL, "grid_index out of range or repeated");
+            seen[(size_t)g] = 1;
+        }
+    }
+    CU(cudaSetDevice(ctx->device));
+    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t b_inv = al((size_t)n_grid * 4), b_idx = al((size_t)n_valid * 4), b_grid = al((size_t)n_grid * 8);
+    const size_t b_res = resident ? 0 : al((size_t)n_valid * 40), b_pk = resident ? 0 : al((size_t)n_valid * 96);
+    const size_t b_out = al((size_t)n_valid * 40), b_flag = al((size_t)n_valid * 4);
+    int rc = reserve(ctx, ctx->filt, b_inv + b_idx + 2 * b_grid + b_res + b_pk + b_out + b_flag);
+    if (rc) return rc;
+    char *base = (char *)ctx->filt.p;
+    int *d_inv = (int *)base;
+    int *d_idx = (int *)(base + b_inv);
+    double *d_c = (double *)(base + b_inv + b_idx), *d_r = (double *)(base + b_inv + b_idx + b_grid);
+    char *p = base + b_inv + b_idx + 2 * b_grid;
+    double *d_res = resident ? (double *)ctx->out.p : (double *)p;
+    double *d_pk = resident ? (double *)ctx->peaks.p : (double *)(p + b_res);
+    double *d_out = (double *)(p + b_res + b_pk);
+    int *d_flag = (int *)(p + b_res + b_pk + b_out);
+    CU(cudaMemsetAsync(d_inv, 0xff, (size_t)n_grid * 4, ctx->stream));                // -1: no table row
+    if (n_valid) CU(cudaMemcpyAsync(d_idx, grid_index, (size_t)n_valid * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(d_c, c2pm1, (size_t)n_grid * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(d_r, r2pm1, (size_t)n_grid * 8, cudaMemcpyHostToDevice, ctx->stream));
+    if (!resident && n_valid) {
+        CU(cudaMemcpyAsync(d_res, results, (size_t)n_valid * 40, cudaMemcpyHostToDevice, ctx->stream));
+        CU(cudaMemcpyAsync(d_pk, peaks, (size_t)n_valid * 96, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    if (n_valid) {
+        const unsigned blocks = (unsigned)((n_valid + 255) / 256);
+        outlier_index_kernel<<<blocks, 256, 0, ctx->stream>>>(n_valid, d_idx, d_inv);
+        outlier_filter_kernel<<<blocks, 256, 0, ctx->stream>>>(n_valid, grid_rows, grid_cols, d_idx, d_inv, d_c, d_r, d_res,
+                                                               d_pk, eps, threshold * threshold, d_out, d_flag);
+        ctx->launches += 2;
+        CU(cudaGetLastError());
+        // decisions read the unfiltered table only: the filtered one is written to a second buffer and copied back
+        if (out) CU(cudaMemcpyAsync(out, d_out, (size_t)n_valid * 40, cudaMemcpyDeviceToHost, ctx->stream));
+        else CU(cudaMemcpyAsync(ctx->out.p, d_out, (size_t)n_valid * 40, cudaMemcpyDeviceToDevice, ctx->stream));
+        if (flag) CU(cudaMemcpyAsync(flag, d_flag, (size_t)n_valid * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    }
     CU(cudaStreamSynchronize(ctx->stream));
     return SID_OK;
 }
@@ -1727,6 +1920,7 @@ int sid_rotate_and_match(sid_ctx *ctx, const uint8_t *img1, int rows1, int cols1
     int rc = check_common(ctx, img_size, n_angles, angle_tab, rot_order, mtype);
     if (rc) return rc;
     if (!valid || !dc || !dr || !best_angle_idx || !best_r || !best_h) return fail(ctx, SID_EINVAL, "null output pointer");
+    if (flags & SID_PEAKS) return fail(ctx, SID_EUNSUPPORTED, "SID_PEAKS is for the batched sid_run* calls");
     const int s = img_size;
     if (!img1 || !image2 || H < s + 1 || W < s + 1)
         return fail(ctx, SID_EINVAL, "search window must exceed the template by at least one pixel in each axis");

@@ -510,9 +510,10 @@ __device__ __forceinline__ void fast_rank_search(const uint32_t *__restrict__ hi
     __syncthreads();
 }
 
-// `hist`: 2048 words of shared memory (any contents).  Returns (hes[peak] - median(hes)) / std(hes); every thread calls it.
+// `hist`: 2048 words of shared memory (any contents).  Returns (hes[peak] - median(hes)) / std(hes) and the median and std
+// it used; every thread calls it.
 __device__ float hes_norm_fast(const float *__restrict__ map, int rows, int cols, int peak_idx, float *__restrict__ hes,
-                               uint32_t *__restrict__ hist, BlockScratch &bs) {
+                               uint32_t *__restrict__ hist, BlockScratch &bs, float &med_out, float &sd_out) {
     const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, warp = tid >> 5, nw = nt >> 5, n = rows * cols;
     for (int k = tid; k < 512; k += nt) reinterpret_cast<uint4 *>(hist)[k] = make_uint4(0u, 0u, 0u, 0u);
     __syncthreads();
@@ -605,13 +606,17 @@ __device__ float hes_norm_fast(const float *__restrict__ map, int rows, int cols
     } else {
         med = block_select_wide(hes, n, n / 2, hist, bs);          // many values share 20 bits (flat maps): the general select
     }
+    med_out = med;
+    sd_out = sd;
     return __fdiv_rn(__fsub_rn(hes[peak_idx], med), sd);
 }
 
 // Tail of rotate_and_match (reference pmlib.py:167-172): Hessian at the peak and the
 // optional normalisations.  `best` is the winning NCC map; tmp_a/tmp_b/hes are scratch
-// maps of the same size.  Every thread of the CTA calls this; results valid in all.
-struct PeakStats { float h; float r; };
+// maps of the same size.  Every thread of the CTA calls this; results valid in all.  On return `best` is unchanged and
+// `hes` holds the Hessian map (of the smoothed map with hes_smth) before normalisation; hmed / hsd (hes_norm) and rmed /
+// rsd (mcc_norm) are the median and std that normalised h and r, so SID_PEAKS normalises its secondary peaks with them.
+struct PeakStats { float h; float r; float hmed, hsd, rmed, rsd; };
 __device__ PeakStats peak_statistics(const float *__restrict__ best, int rows, int cols, int peak_idx, float peak_r,
                                      unsigned flags, const double *gw,
                                      float *__restrict__ tmp_a, float *__restrict__ tmp_b, float *__restrict__ hes,
@@ -620,7 +625,8 @@ __device__ PeakStats peak_statistics(const float *__restrict__ best, int rows, i
     if ((flags & 7u) == 1u && wide_hist != nullptr && rows >= 5 && cols >= 5 && (n & 1) && (nt == 128 || nt == 256 || nt == 512)) {
         PeakStats fast;
         fast.r = peak_r;
-        fast.h = hes_norm_fast(best, rows, cols, peak_idx, hes, wide_hist, bs);
+        fast.h = hes_norm_fast(best, rows, cols, peak_idx, hes, wide_hist, bs, fast.hmed, fast.hsd);
+        fast.rmed = 0.0f; fast.rsd = 1.0f;
         return fast;
     }
     const int y_first = tid / cols, x_first = tid - y_first * cols, dy = nt / cols, dx = nt - dy * cols;
@@ -671,15 +677,18 @@ __device__ PeakStats peak_statistics(const float *__restrict__ best, int rows, i
     PeakStats ps;
     ps.h = hes[peak_idx];
     ps.r = peak_r;
+    ps.hmed = 0.0f; ps.hsd = 1.0f; ps.rmed = 0.0f; ps.rsd = 1.0f;
     if (flags & 1u) {               // hes_norm
         const float med = block_median(hes, n, bs, wide_hist);
         const float sd = block_std(hes, n, bs);
         ps.h = __fdiv_rn(__fsub_rn(ps.h, med), sd);
+        ps.hmed = med; ps.hsd = sd;
     }
     if (flags & 4u) {               // mcc_norm
         const float med = block_median(best, n, bs, wide_hist);
         const float sd = block_std(best, n, bs);
         ps.r = __fdiv_rn(__fsub_rn(peak_r, med), sd);
+        ps.rmed = med; ps.rsd = sd;
     }
     return ps;
 }
@@ -743,6 +752,75 @@ __device__ __forceinline__ unsigned long long warp_max_u64(unsigned long long k)
         k = other > k ? other : k;
     }
     return k;
+}
+
+// Secondary peaks (SID_PEAKS, rule in include/sid_b200.h): the SID_N_PEAKS best local maxima of the raw winning map other
+// than the primary (flat index peak_idx), and their records c2, r2, r, h, computed as the row computes its own.  One sweep
+// over the map; every thread keeps a sorted top 3 of peak_key()s (value, then lowest index), then three rounds of a
+// block-wide maximum pop the best ones.  `hes` and ps: what peak_statistics left.  (c2fg, r2fg): the point's first guess;
+// H x W: its window.  Every thread of the CTA calls this after peak_statistics; thread 0 writes the 3 x 4 doubles at dst
+// (NaN records where fewer peaks exist).  bs.red is reused.
+constexpr int N_PEAKS = 3;
+__device__ __noinline__ void store_secondary_peaks(double *dst, const float *map, const float *hes, int rows, int cols,
+                                                   int peak_idx, const PeakStats ps, unsigned flags, double c2fg,
+                                                   double r2fg, int H, int W, int s, BlockScratch &bs) {
+    const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, warp = tid >> 5, nw = (nt + 31) >> 5, n = rows * cols;
+    unsigned long long t0 = 0ull, t1 = 0ull, t2 = 0ull;
+    for (int p = tid; p < n; p += nt) {
+        if (p == peak_idx) continue;
+        const int i = p / cols, j = p - i * cols;
+        const float v = map[p];
+        // lower flat index (row above, left neighbour): strictly smaller; higher (right neighbour, row below): not larger
+        bool pk = true;
+        if (j > 0) pk = pk && map[p - 1] < v;
+        if (j < cols - 1) pk = pk && map[p + 1] <= v;
+        if (i > 0) {
+            const float *u = map + p - cols;
+            pk = pk && u[0] < v && (j == 0 || u[-1] < v) && (j == cols - 1 || u[1] < v);
+        }
+        if (i < rows - 1) {
+            const float *d = map + p + cols;
+            pk = pk && d[0] <= v && (j == 0 || d[-1] <= v) && (j == cols - 1 || d[1] <= v);
+        }
+        if (!pk) continue;
+        const unsigned long long k = peak_key(v, (uint32_t)p);
+        if (k > t2) {
+            if (k > t1) { t2 = t1; if (k > t0) { t1 = t0; t0 = k; } else t1 = k; }
+            else t2 = k;
+        }
+    }
+    unsigned long long *red = reinterpret_cast<unsigned long long *>(bs.red);
+    unsigned long long top[N_PEAKS];
+#pragma unroll
+    for (int r = 0; r < N_PEAKS; ++r) {
+        const unsigned long long m = warp_max_u64(t0);
+        __syncthreads();                                   // the previous reads of bs.red are done
+        if (lane == 0) red[warp] = m;
+        __syncthreads();
+        unsigned long long best = 0ull;
+        for (int w = 0; w < nw; ++w) best = red[w] > best ? red[w] : best;
+        if (best != 0ull && t0 == best) { t0 = t1; t1 = t2; t2 = 0ull; }     // keys are unique: one thread pops
+        top[r] = best;
+    }
+    if (tid != 0) return;
+#pragma unroll
+    for (int r = 0; r < N_PEAKS; ++r) {
+        double *o = dst + 4 * r;
+        if (top[r] == 0ull) { o[0] = o[1] = o[2] = o[3] = nan(""); continue; }
+        const int p = (int)(0xffffffffu - (uint32_t)(top[r] & 0xffffffffull));
+        const int i = p / cols, j = p - i * cols;
+        double c2 = c2fg + ((double)j - (double)(W - s) / 2.0);
+        double r2 = r2fg + ((double)i - (double)(H - s) / 2.0);
+        if (flags & 8u) {                                  // SID_SUBPIXEL: p > 0 and q >= 0 as for the primary
+            const PeakOffsets d = peak_offsets(map, rows, cols, i, j);
+            c2 = __dadd_rn(c2, d.dx);
+            r2 = __dadd_rn(r2, d.dy);
+        }
+        float rv = map[p], hv = hes[p];
+        if (flags & 4u) rv = __fdiv_rn(__fsub_rn(rv, ps.rmed), ps.rsd);
+        if (flags & 1u) hv = __fdiv_rn(__fsub_rn(hv, ps.hmed), ps.hsd);
+        o[0] = c2; o[1] = r2; o[2] = (double)rv; o[3] = (double)hv;
+    }
 }
 
 }  // namespace sid

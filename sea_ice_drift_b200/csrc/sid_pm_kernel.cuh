@@ -90,6 +90,8 @@ struct PmArgs {
     float *maps_out;
     const long long *map_off;
     uint8_t *tpl_out;
+    // SID_PEAKS only (null otherwise): the secondary peaks of point pt go to peaks + 12 * pt (store_secondary_peaks)
+    double *peaks;
 };
 
 __host__ __device__ inline int pm_window_pitch_words(int W, bool imma = false) {
@@ -450,8 +452,9 @@ __host__ __device__ inline size_t pm_scratch_bytes(int max_rr, int max_hrw, int 
 
 // SMEM_SCRATCH: the per-point scratch sits in shared memory behind the templates (small search
 // windows: no L2 round trips in the statistics / epilogue / Hessian / median phases); otherwise
-// in this CTA's global slab (any window size).
-template <int NW, bool SMEM_SCRATCH, bool IMMA>
+// in this CTA's global slab (any window size).  PEAKS: SID_PEAKS (store_secondary_peaks after the row), a separate
+// instantiation so that the kernels without it keep their registers.
+template <int NW, bool SMEM_SCRATCH, bool IMMA, bool PEAKS>
 __global__ void __launch_bounds__(IMMA ? PM_IMMA_THREADS : PM_THREADS, 3)
 pm_points_kernel(const PmArgs a, const __grid_constant__ CUtensorMap tmap2) {
     extern __shared__ __align__(128) unsigned char pm_smem[];
@@ -772,14 +775,17 @@ pm_points_kernel(const PmArgs a, const __grid_constant__ CUtensorMap tmap2) {
             o[4] = (double)ps.h;
             if (a.status) a.status[pt] = 1;
         }
+        if constexpr (PEAKS) store_secondary_peaks(a.peaks + 12 * pt, best, hes, RH, RW, best_idx, ps, a.flags, c2, r2, H, W, s, S.bs);
         if (a.tpl_out) pm_store_template(a, pt, S.best_a);
     }
 }
 
 // Peak statistics of one work item per CTA (reference pmlib.py:167-172, 209-210) on the map the fused kernel
-// handed over.  Light on registers and shared memory, so ~10 CTAs are resident per SM.
+// handed over.  Light on registers and shared memory, so ~10 CTAs are resident per SM.  PEAKS: SID_PEAKS, as in
+// pm_points_kernel.
 constexpr int PM_TAIL_THREADS = 128;            // small maps; 256 / 512 for larger ones (pm_tail_threads)
 constexpr int PM_TAIL_MAX_THREADS = 512;
+template <bool PEAKS>
 __global__ void __launch_bounds__(PM_TAIL_MAX_THREADS) pm_tail_kernel(const PmArgs a) {
     extern __shared__ __align__(16) unsigned char tail_smem[];
     __shared__ BlockScratch bs;
@@ -838,6 +844,9 @@ __global__ void __launch_bounds__(PM_TAIL_MAX_THREADS) pm_tail_kernel(const PmAr
         o[4] = (double)ps.h;
         if (a.status) a.status[rec.pt] = 1;
     }
+    if constexpr (PEAKS)
+        store_secondary_peaks(a.peaks + 12 * (long long)rec.pt, map, hes, rec.RH, rec.RW, rec.best_idx, ps, a.flags,
+                              a.c2fg[rec.pt], a.r2fg[rec.pt], rec.H, rec.W, a.s, bs);
 }
 // CTA size of pm_tail_kernel by map size: a large map in shared memory leaves room for only two CTAs per SM, so each gets
 // more warps (128 / 256 / 512 take peak_statistics' fast path)

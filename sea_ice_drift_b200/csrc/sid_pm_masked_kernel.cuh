@@ -108,6 +108,8 @@ struct PmMaskedShared {
 // One candidate row per CTA (work stealing over a.order[0 .. *n_cand)).  The winning angle's float map goes through the
 // existing peak_statistics / peak_offsets / pm_store_map / pm_store_template.  Per-CTA global scratch: two map slots (the
 // best so far and the current angle), the Hessian map and a smoothing temporary, max_rr floats each.
+// PEAKS: SID_PEAKS, a separate instantiation as for pm_points_kernel.
+template <bool PEAKS>
 __global__ void __launch_bounds__(PM_MASKED_THREADS) pm_masked_kernel(const PmArgs a, const unsigned *__restrict__ n_cand) {
     __shared__ PmMaskedShared S;
     const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, s = a.s;
@@ -193,6 +195,7 @@ __global__ void __launch_bounds__(PM_MASKED_THREADS) pm_masked_kernel(const PmAr
             o[4] = (double)ps.h;
             if (a.status) a.status[pt] = 2;                 // SID_PT_MASKED
         }
+        if constexpr (PEAKS) store_secondary_peaks(a.peaks + 12 * pt, best, hes, RH, RW, best_idx, ps, a.flags, c2, r2, H, W, s, S.bs);
         if (a.tpl_out) pm_store_template(a, pt, best_a);
     }
 }

@@ -819,6 +819,7 @@ pm_tc_kernel(const PmArgs a, const PmTcCfg g, const __grid_constant__ CUtensorMa
             o[4] = (double)ps.h;
             if (a.status) a.status[pt] = 1;
         }
+        if (a.peaks) store_secondary_peaks(a.peaks + 12 * pt, best, hes, RH, RW, best_idx, ps, a.flags, c2, r2, H, W, s, S.bs);
         if (a.tpl_out) pm_store_template(a, pt, S.best_a);
     }
     // a window requested for a work item that never ran (the list ended) must land before the CTA exits

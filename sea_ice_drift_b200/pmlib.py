@@ -139,10 +139,16 @@ def use_mcc_batch(c1, r1, c2fg, r2fg, border, img1, img2, img_size, alpha0, **kw
     ``masked=True`` (extension): rows that are NaN because a template holds a 0 pixel (land, no-data) are matched by
     the Pearson correlation over the templates' valid pixels where every angle's template has at least
     ``ceil(img_size**2 / 2)`` valid pixels and is not flat (``SID_MASKED``, include/sid_b200.h); ``return_maps`` then
-    gives their masked maps and templates.  Every other row is unchanged.  Needs the built-in matcher."""
+    gives their masked maps and templates.  Every other row is unchanged.  Needs the built-in matcher.
+
+    ``peaks=True`` (extension): also return the three next-best peaks of every row's winning map (``SID_PEAKS``,
+    include/sid_b200.h) as an (N, 3, 4) float64 array of c2, r2, r, h per peak, NaN where missing, appended to what the
+    call returns: ``(table, peaks)`` or ``(table, maps, templates, peaks)``.  The table is unchanged.  Needs the
+    built-in matcher."""
     matcher = kwargs.get('template_matcher')
     return_maps = kwargs.get('return_maps', False)
-    for option in ('return_maps', 'subpixel', 'masked'):
+    want_peaks = kwargs.get('peaks', False)
+    for option in ('return_maps', 'subpixel', 'masked', 'peaks'):
         if kwargs.get(option) and not _is_builtin_matcher(matcher):
             raise ValueError("%s=True needs the built-in matcher (template_matcher None, match_template or "
                              "cv2.matchTemplate)" % option)
@@ -151,7 +157,7 @@ def use_mcc_batch(c1, r1, c2fg, r2fg, border, img1, img2, img_size, alpha0, **kw
                 for a, b, c, d, e in zip(c1, r1, c2fg, r2fg, border)]
         return np.array(rows, dtype=np.float64).reshape(-1, 5)
     ctx = _ctx(kwargs)
-    flags = flags_from_options(kwargs)
+    flags = flags_from_options(kwargs) | (_lib.SID_PEAKS if want_peaks else 0)
     args = (c1, r1, c2fg, r2fg, border, img_size, list(kwargs.get('angles', [-3, 0, 3])), alpha0,
             kwargs.get('rot_order', 0), flags, kwargs.get('mtype', TM_CCOEFF_NORMED))
     # The pair is uploaded on EVERY call (overlapped with the matching, so it costs ~1.5 ms per EW pair) unless
@@ -162,12 +168,17 @@ def use_mcc_batch(c1, r1, c2fg, r2fg, border, img1, img2, img_size, alpha0, **kw
         if not (kwargs.get('resident') and ctx._pair_key is not None):
             ctx.set_pair(img1, img2)
             ctx._pair_key = (np.shape(img1), np.shape(img2))
-        return ctx.run_maps(*args)
-    if kwargs.get('resident') and ctx._pair_key is not None:
-        return ctx.run(*args)
-    out = ctx.run_pair(img1, img2, *args)
-    ctx._pair_key = (np.shape(img1), np.shape(img2))
-    return out
+        out = ctx.run_maps(*args)
+    elif kwargs.get('resident') and ctx._pair_key is not None:
+        out = ctx.run(*args)
+    else:
+        out = ctx.run_pair(img1, img2, *args)
+        ctx._pair_key = (np.shape(img1), np.shape(img2))
+    if not want_peaks:
+        return out
+    if return_maps:
+        return out + (ctx.peaks(len(out[0])),)
+    return out, ctx.peaks(len(out))
 
 
 def use_mcc(c1, r1, c2fg, r2fg, border, img1, img2, img_size, alpha0, **kwargs):
@@ -463,6 +474,31 @@ def coarse_tracking(n1, n2, **kwargs):
     return coarse_matches(table, status, c1, r1, k, s, float(opts['min_quality']))
 
 
+OUTLIER_EPS, OUTLIER_THRESHOLD = 1.0, 2.0
+
+
+def _grid_shape(shape):
+    """(rows, cols) of a grid of ``shape``: a 1-D grid is one row."""
+    shape = tuple(int(v) for v in shape)
+    if len(shape) == 1:
+        return 1, shape[0]
+    if len(shape) != 2:
+        raise ValueError("the grid must be 1-D or 2-D")
+    return shape
+
+
+def filter_outliers(table, peaks, gpi, c2pm1, r2pm1, eps=OUTLIER_EPS, threshold=OUTLIER_THRESHOLD, **kwargs):
+    """Normalised median test (Westerweel & Scarano 2005) with replacement by secondary peaks, on the device
+    (``sid_filter_outliers``, include/sid_b200.h), for callers with their own grid.  ``table``: the (N, 5) table of
+    :func:`use_mcc_batch` for the True positions of the grid-shaped boolean ``gpi`` in row-major order; ``peaks``: its
+    (N, 3, 4) ``peaks=True`` records; ``c2pm1`` / ``r2pm1``: the grid's image-2 pixel coordinates.  Every row is
+    compared with its 8 grid neighbours' displacements ``(c2, r2) - round(c2pm1, r2pm1)``; an outlier takes its first
+    secondary peak that passes the test, else becomes NaN.  Returns ``(table, flags)``: flags 0 kept, 1 ... 3 replaced
+    by that peak, -1 rejected, -2 fewer than 3 neighbours (kept), -3 NaN row."""
+    gpi = np.asarray(gpi, dtype=bool)
+    return _ctx(kwargs).filter_outliers(_grid_shape(gpi.shape), gpi, c2pm1, r2pm1, table, peaks, eps, threshold)
+
+
 def _nsr(srs):
     try:
         from nansat import NSR
@@ -482,7 +518,24 @@ def pattern_matching(lon_pm1, lat_pm1, n1, c1, r1, n2, c2, r2,
 
     ``subpixel=True`` (extension): sub-pixel drift vectors (see :func:`use_mcc_batch`).
     ``masked=True`` (extension): vectors next to land and no-data from the masked correlation (see
-    :func:`use_mcc_batch`)."""
+    :func:`use_mcc_batch`).
+    ``outliers=True`` (extension): repair outlier vectors before the post-processing with the normalised median test
+    over the grid and the three secondary peaks of every point (see :func:`filter_outliers`; ``outlier_eps`` default
+    1.0 px, ``outlier_threshold`` default 2.0): replaced vectors come back in place, rejected ones as NaN.  Needs the
+    built-in matcher and one GPU (no process group of more than one rank).  With ``return_flags=True`` an eighth grid
+    (int32) holds every point's flag of :func:`filter_outliers`, and -4 where the point was not matched (outside the
+    image or its search window)."""
+    from .sharding import use_mcc_batch_sharded, _dist
+    outliers = kwargs.get('outliers', False)
+    if outliers and not _is_builtin_matcher(kwargs.get('template_matcher')):
+        raise ValueError("outliers=True needs the built-in matcher (template_matcher None, match_template or "
+                         "cv2.matchTemplate)")
+    if outliers and _dist() is not None:
+        raise ValueError("outliers=True runs on one GPU: it is not supported under a process group of more than one rank")
+    eps, threshold = kwargs.get('outlier_eps', OUTLIER_EPS), kwargs.get('outlier_threshold', OUTLIER_THRESHOLD)
+    return_flags = kwargs.get('return_flags', False)
+    if return_flags and not outliers:
+        raise ValueError("return_flags=True needs outliers=True")
     t0 = time.time()
     img1, img2 = n1[1], n2[1]
     dst_shape = lon_pm1.shape
@@ -506,8 +559,16 @@ def pattern_matching(lon_pm1, lat_pm1, n1, c1, r1, n2, c2, r2,
            (c1pm1i + hws_hypot + margin < shape1[1]) *
            (r1pm1i + hws_hypot + margin < shape1[0]))
     alpha0 = get_initial_rotation(n1, n2)
+    grid_shape = _grid_shape(dst_shape)
+    flag_grid = np.full(dst_shape, -4, np.int32)
 
-    from .sharding import use_mcc_batch_sharded, _dist
+    def finish(grids, flags=None):
+        if return_flags:
+            if flags is not None:
+                flag_grid.ravel()[np.flatnonzero(gpi)] = flags
+            return tuple(grids) + (flag_grid,)
+        return tuple(grids)
+
     # Affine geolocation (an object exposing ``affine_maps(srs) -> (pixel->x/y, pixel->lon/lat)`` 2 x 3 matrices, e.g.
     # synthetic.ArrayDomain): the post-processing below (reference pmlib.py:462-497) runs on the device too, on the
     # table the kernels left there -- the (N, 5) table never visits the host.  Real Nansat objects (GDAL, possibly
@@ -517,20 +578,31 @@ def pattern_matching(lon_pm1, lat_pm1, n1, c1, r1, n2, c2, r2,
             and _is_builtin_matcher(kwargs.get('template_matcher'))):
         xy, ll = affine(srs)
         ctx = _ctx(kwargs)
-        flags = flags_from_options(kwargs)
+        flags = flags_from_options(kwargs) | (_lib.SID_PEAKS if outliers else 0)
         ctx.run_pair(img1, img2, c1pm1i[gpi], r1pm1i[gpi], c2fg[gpi], r2fg[gpi], brd2[gpi], img_size,
                      list(kwargs.get('angles', [-3, 0, 3])), alpha0, kwargs.get('rot_order', 0), flags,
                      kwargs.get('mtype', TM_CCOEFF_NORMED), keep_on_device=True)
+        out_flags = None
+        if outliers:
+            out_flags = ctx.filter_outliers(grid_shape, gpi, c2pm1, r2pm1, eps=eps, threshold=threshold, in_place=True)[1]
         grids = ctx.pm_epilogue_affine(gpi, c2pm1, r2pm1, xy, ll)
         print('\n', 'Pattern matching - OK! (%3.0f sec)' % (time.time() - t0))
-        return tuple(grid.reshape(dst_shape) for grid in grids)
-    results = use_mcc_batch_sharded(c1pm1i[gpi], r1pm1i[gpi], c2fg[gpi], r2fg[gpi], brd2[gpi],
-                                    img1, img2, img_size, alpha0, **kwargs)
+        return finish((grid.reshape(dst_shape) for grid in grids), out_flags)
+    out_flags = None
+    if outliers:
+        results, peaks = use_mcc_batch(c1pm1i[gpi], r1pm1i[gpi], c2fg[gpi], r2fg[gpi], brd2[gpi],
+                                       img1, img2, img_size, alpha0, **dict(kwargs, peaks=True))
+        if len(results):
+            results, out_flags = _ctx(kwargs).filter_outliers(grid_shape, gpi, c2pm1, r2pm1, results, peaks, eps,
+                                                              threshold)
+    else:
+        results = use_mcc_batch_sharded(c1pm1i[gpi], r1pm1i[gpi], c2fg[gpi], r2fg[gpi], brd2[gpi],
+                                        img1, img2, img_size, alpha0, **kwargs)
 
     print('\n', 'Pattern matching - OK! (%3.0f sec)' % (time.time() - t0))
     if len(results) == 0:
         nan_grid = np.zeros(dst_shape) + np.nan
-        return tuple(nan_grid.copy() for _ in range(7))
+        return finish(nan_grid.copy() for _ in range(7))
 
     c2pm2 = results[:, 0] + (c2pm1 - c2pm1i)[gpi]
     r2pm2 = results[:, 1] + (r2pm1 - r2pm1i)[gpi]
@@ -543,5 +615,4 @@ def pattern_matching(lon_pm1, lat_pm1, n1, c1, r1, n2, c2, r2,
     a = _fill_gpi(dst_shape, gpi, results[:, 2])
     r = _fill_gpi(dst_shape, gpi, results[:, 3])
     h = _fill_gpi(dst_shape, gpi, results[:, 4])
-    return (u, v, a, r, h,
-            _fill_gpi(dst_shape, gpi, lon_pm2), _fill_gpi(dst_shape, gpi, lat_pm2))
+    return finish((u, v, a, r, h, _fill_gpi(dst_shape, gpi, lon_pm2), _fill_gpi(dst_shape, gpi, lat_pm2)), out_flags)
