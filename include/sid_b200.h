@@ -91,6 +91,32 @@ typedef struct sid_ctx sid_ctx;
  * sid_rotate_and_match refuses it (SID_EUNSUPPORTED). */
 #define SID_PEAKS 32u
 #define SID_N_PEAKS 3
+/* SID_UNCERT (extension, not in the reference): also record, for every row, the covariance of the sub-pixel offsets
+ * (dx, dy) that SID_SUBPIXEL added to c2 and r2 -- three doubles var_c, var_r, cov_cr in image-2 pixels^2 -- by correlation
+ * statistics (Wieneke 2015, Meas. Sci. Technol. 26, 074002).  Valid only with SID_SUBPIXEL: without it every sid_run*
+ * returns SID_EINVAL before any launch.  For a SID_PT_VALID or SID_PT_MASKED row: T the winning angle's template (s x s,
+ * the bytes sid_run_maps returns), W_P the window patch at map position P (the kernels' window rule), m the RAW float32
+ * winning map (RH x RW) and (bi, bj) its primary integer peak.  M_k = 1 (VALID) or (T_k > 0) (MASKED), and
+ *   n = sum M_k, St = sum M_k T_k, t_k = M_k (n T_k - St), Vt = sum t_k^2                                 (exact int64)
+ *   Sw(P) = sum M_k W_P,k, w_k(P) = M_k (n W_P,k - Sw(P)), A(P) = sum t_k w_k(P), V(P) = sum w_k(P)^2     (exact int64:
+ *   |t|, |w| < 2^22 for s <= 128), S(P, Q) = sum t_k^2 w_k(P) w_k(Q)  (exact 128-bit: |S| < 2^102 at s = 128)
+ *   K(P, Q) = D(n S(P, Q) - A(P) A(Q)) / (((D(n) D(Vt)) sqrt(D(V(P)))) sqrt(D(V(Q))))
+ * with D the correctly rounded (ties to even) integer -> double conversion of the exact numerator (|.| < 2^117) and every
+ * operation IEEE double, round to nearest, without contraction.  The per-pixel contributions
+ * x_k(P) = t_k w_k(P) / (sqrt(Vt) sqrt(V(P))) sum to the Pearson correlation at P; K is n times their population
+ * covariance over the n pixels, i.e. the covariance of the correlation values at P and Q when pixels are independent.
+ * Positions, in this order: P0 = (bi, bj), X- / X+ = (bi, bj -+ 1), Y- / Y+ = (bi -+ 1, bj); K is evaluated
+ * once per unordered pair, P the earlier of the two in that order.  With a, b, c = m at X-, P0, X+ widened to double,
+ * p = b - a, q = b - c, w = (p + q) (p + q) and g = (-q / w, (q - p) / w, p / w) (the gradient of the vertex
+ * d = (p - q) / (2 (p + q)) in (a, b, c)); g' the same down the column (Y-, P0, Y+):
+ *   var_c = (g0 h0 + g1 h1) + g2 h2,  h_u = (K(u, X-) g0 + K(u, P0) g1) + K(u, X+) g2,  u = X-, P0, X+
+ *   var_r the same with g' over Y-, P0, Y+;  cov_cr with g on the left over (X-, P0, X+), g' on the right over (Y-, P0, Y+).
+ * NaN: a peak on the first or last map column makes var_c and cov_cr NaN (that axis is not refined), one on the first or
+ * last row var_r and cov_cr; V(P) = 0 at a position an axis uses makes that axis' variance and cov_cr NaN; rows that are
+ * neither VALID nor MASKED get three NaN.  mcc_norm and hes_smth do not enter.  The pass is one extra launch behind every
+ * other launch of the call; the table, status, maps, templates and peaks are bit-identical to the call without the flag.
+ * sid_get_uncertainty copies the records out; sid_rotate_and_match refuses the flag (SID_EUNSUPPORTED). */
+#define SID_UNCERT 64u
 
 /* point status written by sid_run* (optional output) */
 #define SID_PT_VALID 1
@@ -162,6 +188,10 @@ int sid_pm_epilogue_affine(sid_ctx *ctx, int64_t n_valid, const int32_t *grid_in
  * or had a different n. */
 int sid_get_peaks(sid_ctx *ctx, int64_t n, double *out);
 
+/* SID_UNCERT records of the previous sid_run* call: out = n x 3 doubles (var_c, var_r, cov_cr), host pointer,
+ * synchronous.  SID_EINVAL (context stays usable) when that call did not set SID_UNCERT or had a different n. */
+int sid_get_uncertainty(sid_ctx *ctx, int64_t n, double *out);
+
 /* Normalised median test (Westerweel & Scarano 2005, "universal outlier detection") over the grid of a result table, with
  * replacement by a secondary peak (SID_PEAKS), on the device.  Every operation is an IEEE double op without contraction.
  *   grid_rows x grid_cols  the grid; n_valid, grid_index, c2pm1, r2pm1 as for sid_pm_epilogue_affine (n_grid = rows x cols)
@@ -199,7 +229,7 @@ int sid_downsample_pair(sid_ctx *ctx, int factor,
                         uint8_t *d_img1, int64_t pitch1, int64_t bytes1,
                         uint8_t *d_img2, int64_t pitch2, int64_t bytes2);
 
-/* use_mcc for n grid points (host arrays in, host array out, synchronous).  All sid_run* honour SID_MASKED and SID_PEAKS.
+/* use_mcc for n grid points (host arrays in, host array out, synchronous).  All sid_run* honour SID_MASKED, SID_PEAKS and SID_UNCERT.
  *   c1, r1        float pixel coordinates on image 1
  *   c2fg, r2fg    integer-valued first guess on image 2
  *   border        integer-valued search radius per point

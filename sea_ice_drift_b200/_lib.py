@@ -23,6 +23,7 @@ SID_SUBPIXEL = 8                # extension: sub-pixel c2 / r2 (include/sid_b200
 SID_MASKED = 16                 # extension: masked correlation for templates with 0 pixels (include/sid_b200.h)
 SID_PEAKS = 32                  # extension: the secondary peaks of every row's winning map (include/sid_b200.h)
 SID_N_PEAKS = 3                 # secondary peaks recorded per row
+SID_UNCERT = 64                 # extension: covariance of every row's sub-pixel offsets (include/sid_b200.h)
 SID_PT_VALID = 1                # point status of a valid row (sid_run*)
 SID_PT_MASKED = 2               # point status of a row matched by the masked rule (SID_MASKED)
 
@@ -30,7 +31,7 @@ EXPORTS = [
     "sid_version", "sid_create", "sid_destroy", "sid_last_error", "sid_set_stream", "sid_synchronize",
     "sid_set_pair", "sid_set_pair_device", "sid_pair_layout", "sid_adopt_pair_device", "sid_upload_rows", "sid_pm_epilogue_affine", "sid_first_guess", "sid_run", "sid_run_pair", "sid_run_device", "sid_map_layout", "sid_run_maps", "sid_launch_count", "sid_last_kernel_ms", "sid_last_kernel_name",
     "sid_rotate_and_match", "sid_get_template", "sid_match_template", "sid_get_hessian", "sid_knn_hamming2",
-    "sid_deformation", "sid_downsample_pair", "sid_get_peaks", "sid_filter_outliers",
+    "sid_deformation", "sid_downsample_pair", "sid_get_peaks", "sid_filter_outliers", "sid_get_uncertainty",
 ]
 
 _lib = None
@@ -99,6 +100,7 @@ def load_library():
         lib.sid_get_hessian.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_uint, C.c_void_p]
         lib.sid_deformation.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 4 + [C.c_int] + [C.c_void_p] * 7
         lib.sid_get_peaks.argtypes = [C.c_void_p, C.c_int64, C.c_void_p]
+        lib.sid_get_uncertainty.argtypes = [C.c_void_p, C.c_int64, C.c_void_p]
         lib.sid_filter_outliers.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int64] + [C.c_void_p] * 5 + \
             [C.c_double, C.c_double, C.c_void_p, C.c_void_p]
         _lib = lib
@@ -139,17 +141,20 @@ def pair_layout(rows, cols):
     return int(pitch.value), int(nbytes.value)
 
 
-def flags_from_kwargs(hes_norm=True, hes_smth=False, mcc_norm=False, subpixel=False, masked=False):
+def flags_from_kwargs(hes_norm=True, hes_smth=False, mcc_norm=False, subpixel=False, masked=False, uncertainty=False):
+    if uncertainty and not subpixel:
+        raise ValueError("uncertainty=True needs subpixel=True: it is the covariance of the sub-pixel offsets")
     return (SID_HES_NORM if hes_norm else 0) | (SID_HES_SMTH if hes_smth else 0) | (SID_MCC_NORM if mcc_norm else 0) | \
-        (SID_SUBPIXEL if subpixel else 0) | (SID_MASKED if masked else 0)
+        (SID_SUBPIXEL if subpixel else 0) | (SID_MASKED if masked else 0) | (SID_UNCERT if uncertainty else 0)
 
 
 def flags_from_options(kwargs):
     """The sid_run* flags of a kwargs dict of the drop-in API: ``hes_norm`` (default True), ``hes_smth``, ``mcc_norm``
-    and the extensions ``subpixel`` and ``masked`` (default False), so every entry point maps its keyword arguments the
-    same way."""
+    and the extensions ``subpixel``, ``masked`` and ``uncertainty`` (default False), so every entry point maps its
+    keyword arguments the same way.  ``uncertainty`` without ``subpixel`` raises ValueError."""
     return flags_from_kwargs(kwargs.get('hes_norm', True), kwargs.get('hes_smth', False), kwargs.get('mcc_norm', False),
-                             kwargs.get('subpixel', False), kwargs.get('masked', False))
+                             kwargs.get('subpixel', False), kwargs.get('masked', False),
+                             kwargs.get('uncertainty', False))
 
 
 class Context(object):
@@ -267,6 +272,13 @@ class Context(object):
         r, h per secondary peak, rank order, NaN where missing."""
         out = np.empty((int(n), SID_N_PEAKS, 4), dtype=np.float64)
         self._check(self._lib.sid_get_peaks(self._h, int(n), out.ctypes.data))
+        return out
+
+    def uncertainty(self, n):
+        """The SID_UNCERT records of the previous run (sid_get_uncertainty): an (n, 3) float64 array of var_c, var_r,
+        cov_cr, the covariance of every row's sub-pixel offsets in image-2 pixels^2, NaN where undefined."""
+        out = np.empty((int(n), 3), dtype=np.float64)
+        self._check(self._lib.sid_get_uncertainty(self._h, int(n), out.ctypes.data))
         return out
 
     def filter_outliers(self, grid_shape, gpi, c2pm1, r2pm1, results=None, peaks=None, eps=1.0, threshold=2.0,

@@ -27,6 +27,7 @@
 #include "sid_fg_kernel.cuh"
 #include "sid_downsample_kernel.cuh"
 #include "sid_pm_masked_kernel.cuh"
+#include "sid_uncert_kernel.cuh"
 
 using namespace sid;
 
@@ -115,6 +116,8 @@ struct sid_ctx {
     long long peaks_n = -1;                  // its n, or -1 when the last sid_run* call did not set SID_PEAKS
     bool peaks_of_table = false;             // that call was the sid_run / sid_run_pair / sid_run_maps that left `out`
     DevBuf filt;                             // sid_filter_outliers
+    DevBuf uncert;                           // SID_UNCERT: n x 3 doubles of the last sid_run* call
+    long long uncert_n = -1;                 // its n, or -1 when the last sid_run* call did not set SID_UNCERT
     void *pin = nullptr;
     size_t pin_cap = 0;
     cudaEvent_t k_ev[2] = {};                // bracket the last fused-kernel launch (sid_last_kernel_ms)
@@ -211,6 +214,12 @@ int check_common(sid_ctx *ctx, int img_size, int n_angles, const double *angle_t
     return SID_OK;
 }
 
+// SID_UNCERT propagates through the sub-pixel estimator, so it needs SID_SUBPIXEL
+int check_uncert(sid_ctx *ctx, unsigned flags) {
+    if ((flags & SID_UNCERT) && !(flags & SID_SUBPIXEL)) return fail(ctx, SID_EINVAL, "SID_UNCERT needs SID_SUBPIXEL");
+    return SID_OK;
+}
+
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
                                   const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -264,7 +273,10 @@ bool ws_fits(const sid_ctx *ctx, int s, int border, int n_angles, int rtyp, int 
            (size_t)g.smem_bytes + 2048 + headroom <= (size_t)ctx->max_smem_optin;
 }
 
-enum PmKernel { PM_WS, PM_TC, PM_POINTS, PM_MASKED };
+enum PmKernel { PM_WS, PM_TC, PM_POINTS, PM_MASKED, PM_UNCERT };
+// What a launch is for: the correlation of a border class, the masked pass of SID_MASKED, the uncertainty pass of
+// SID_UNCERT
+enum PmPass { PASS_MATCH, PASS_MASKED, PASS_UNCERT };
 
 // Everything a matching launch needs that does not depend on which points it takes: the kernel and its variant, its
 // configuration and tensor maps, the geometry fields of PmArgs, the CTA shape and that of the split tail
@@ -286,9 +298,11 @@ struct PmPlan {
 };
 
 // Kernel, variant and shape of a launch over points with borders up to max_border (typ_border: the typical point, which
-// sizes the CTA and pads pm_ws_kernel's layout).  `masked`: the masked pass of SID_MASKED (pm_masked_kernel, any border,
-// its own tail).  Host queries only: nothing is allocated or enqueued.
-int plan_pm(sid_ctx *ctx, int s, int n_angles, unsigned flags, int max_border, int typ_border, PmPlan &p, bool masked = false) {
+// sizes the CTA and pads pm_ws_kernel's layout).  PASS_MASKED: the masked pass of SID_MASKED (pm_masked_kernel, any
+// border, its own tail); PASS_UNCERT: the uncertainty pass of SID_UNCERT (uncert_kernel, every row of the call, after
+// every other launch).  Host queries only: nothing is allocated or enqueued.
+int plan_pm(sid_ctx *ctx, int s, int n_angles, unsigned flags, int max_border, int typ_border, PmPlan &p,
+            PmPass pass = PASS_MATCH) {
     p = PmPlan{};
     const int hws = s / 2;
     const int Wmax = 2 * hws + 2 * max_border + 1;
@@ -302,7 +316,17 @@ int plan_pm(sid_ctx *ctx, int s, int n_angles, unsigned flags, int max_border, i
     gaussian_weights(a.gw);
     a.max_rr = Rmax * Rmax;
     a.max_hrw = Wmax * Rmax;
-    if (masked) {
+    if (pass == PASS_UNCERT) {
+        p.kernel = PM_UNCERT;
+        p.kfn = (const void *)uncert_kernel;
+        p.name = "sid::uncert_kernel";
+        p.threads = UNC_THREADS;
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&p.occ, p.kfn, p.threads, 0));
+        if (p.occ < 1) return fail(ctx, SID_ECUDA, "uncert_kernel does not fit on an SM");
+        p.occ_api = p.occ;
+        return SID_OK;
+    }
+    if (pass == PASS_MASKED) {
         p.kernel = PM_MASKED;
         p.kfn = (flags & SID_PEAKS) ? (const void *)pm_masked_kernel<true> : (const void *)pm_masked_kernel<false>;
         p.name = "sid::pm_masked_kernel";
@@ -520,6 +544,7 @@ struct PmCall {
     size_t tail_stride;              // floats per point of the tail hand-off regions
     size_t scratch_slot;             // bytes of global scratch per band stream
     double *peaks = nullptr;         // SID_PEAKS only, see PmArgs::peaks
+    double *uncert = nullptr;        // set by reserve_call for an uncertainty pass: n x 3 doubles (uncert_kernel)
 };
 
 // The buffers the launches of a call share, reserved once before the first launch, so that none of them is reallocated
@@ -528,9 +553,10 @@ struct PmCall {
 int reserve_call(sid_ctx *ctx, PmCall &call, const PmPlan *plans, int nplans) {
     call.tail_stride = 0;
     call.scratch_slot = 0;
-    bool masked = false;
+    bool masked = false, uncert = false;
     for (int i = 0; i < nplans; ++i) {
         const PmPlan &p = plans[i];
+        if (p.kernel == PM_UNCERT) uncert = true;
         // a work item of pm_ws_kernel hands over three integer arrays (PmTailRec::mode 1), the others a float map
         if (p.args.split_tail) call.tail_stride = std::max(call.tail_stride, tail_item_words(p.args.tail_stride, p.kernel == PM_WS));
         if (p.kernel == PM_MASKED) masked = true;
@@ -547,14 +573,21 @@ int reserve_call(sid_ctx *ctx, PmCall &call, const PmPlan *plans, int nplans) {
         if ((rc = reserve(ctx, ctx->tail_maps, (size_t)call.n * call.tail_stride * sizeof(float)))) return rc;
         if ((rc = reserve(ctx, ctx->tail_recs, (size_t)call.n * sizeof(PmTailRec)))) return rc;
     }
-    if (masked) {
-        // the masked pass finds its rows by their status: a call without a status array gets the context's
+    if (masked || uncert) {
+        // the masked and uncertainty passes find their rows by their status: a call without a status array gets the
+        // context's
         if (!call.status) {
             if ((rc = reserve(ctx, ctx->status, (size_t)call.n * sizeof(int)))) return rc;
             call.status = (int *)ctx->status.p;
         }
+    }
+    if (masked) {
         if ((rc = reserve(ctx, ctx->cand, (size_t)call.n * sizeof(int)))) return rc;
         call.cand = (int *)ctx->cand.p;
+    }
+    if (uncert) {                    // the pass writes every row's record: no fill needed
+        if ((rc = reserve(ctx, ctx->uncert, (size_t)call.n * 3 * sizeof(double)))) return rc;
+        call.uncert = (double *)ctx->uncert.p;
     }
     return SID_OK;
 }
@@ -563,7 +596,8 @@ int reserve_call(sid_ctx *ctx, PmCall &call, const PmPlan *plans, int nplans) {
 // points 0 .. n - 1), their tail hand-off at point offset tail_off of the call's regions; `slot` picks the counter and
 // scratch of one of the two band streams.  `continues`: the second class of a two-class call, or the masked pass, so the
 // kernel-time events bracket every launch of the call.  The masked pass (PM_MASKED) runs after every other launch of the
-// call: it gathers the rows they left with status 0 on the device (masked_candidates_kernel) and takes those.
+// call: it gathers the rows they left with status 0 on the device (masked_candidates_kernel) and takes those.  The
+// uncertainty pass (PM_UNCERT) runs after the masked pass, over all n rows of the call.
 int enqueue_pm(sid_ctx *ctx, const PmCall &call, const PmPlan &p, long long n, const int *order, cudaStream_t st, int slot,
                long long tail_off, bool continues) {
     PmArgs a = p.args;
@@ -594,7 +628,9 @@ int enqueue_pm(sid_ctx *ctx, const PmCall &call, const PmPlan &p, long long n, c
     const bool debug = getenv("SID_DEBUG") != nullptr;
     const PmWsCfg &wg = p.wg;
     const PmTcCfg &tg = p.tg;
-    if (debug && p.kernel == PM_MASKED)
+    if (debug && p.kernel == PM_UNCERT)
+        fprintf(stderr, "[sid] launch: uncert threads=%d occ=%d grid=%lld\n", p.threads, p.occ, grid);
+    else if (debug && p.kernel == PM_MASKED)
         fprintf(stderr, "[sid] launch: masked threads=%d occ=%d scratch=%llu grid=%lld\n", p.threads, p.occ, a.scratch_per_cta, grid);
     else if (debug && p.kernel == PM_WS)
         fprintf(stderr, "[sid] launch: ws smem=%d nstat=%d nab=%d ks=%d npairs=%d nslots=%d slot_bytes=%d npanels=%d wrows=%d n16max=%d grid=%lld\n",
@@ -610,14 +646,16 @@ int enqueue_pm(sid_ctx *ctx, const PmCall &call, const PmPlan &p, long long n, c
     void *params_tc[] = {(void *)&a, (void *)&p.tg, (void *)&p.tmap};
     void *params_points[] = {(void *)&a, (void *)&p.tmap};
     void *params_masked[] = {(void *)&a, (void *)&n_cand};
-    void **params = p.kernel == PM_WS ? params_ws : p.kernel == PM_TC ? params_tc : p.kernel == PM_MASKED ? params_masked : params_points;
+    void *params_uncert[] = {(void *)&a, (void *)&call.uncert};
+    void **params = p.kernel == PM_WS ? params_ws : p.kernel == PM_TC ? params_tc : p.kernel == PM_MASKED ? params_masked
+                    : p.kernel == PM_UNCERT ? params_uncert : params_points;
     if (!ctx->k_ev[0]) { CU(cudaEventCreate(&ctx->k_ev[0])); CU(cudaEventCreate(&ctx->k_ev[1])); }
     if (!continues) CU(cudaEventRecord(ctx->k_ev[0], st));
     CU(cudaLaunchKernel(p.kfn, dim3((unsigned)grid), dim3((unsigned)p.threads), params, p.smem, st));
     CU(cudaEventRecord(ctx->k_ev[1], st));
     ctx->k_ev_valid = true;
-    // the masked pass keeps the name of the correlation kernel of the call
-    ctx->k_name = p.kernel == PM_MASKED ? ctx->k_name
+    // the masked and uncertainty passes keep the name of the correlation kernel of the call
+    ctx->k_name = p.kernel == PM_MASKED || p.kernel == PM_UNCERT ? ctx->k_name
                   : p.kernel != PM_WS || !continues ? p.name
                   : strstr(ctx->k_name, "pm_tc_kernel") ? "sid::pm_tc_kernel + sid::pm_ws_kernel"
                   : strstr(ctx->k_name, "pm_points_kernel") ? "sid::pm_points_kernel + sid::pm_ws_kernel" : p.name;
@@ -683,7 +721,7 @@ void sid_destroy(sid_ctx *ctx) {
     cudaStreamSynchronize(ctx->stream);
     DevBuf *bufs[] = {&ctx->img1, &ctx->img2, &ctx->pts, &ctx->order, &ctx->out, &ctx->status,
                       &ctx->angles, &ctx->scratch, &ctx->counter, &ctx->misc, &ctx->tail_maps, &ctx->tail_recs, &ctx->epi, &ctx->fg,
-                      &ctx->maps, &ctx->map_off, &ctx->tpl, &ctx->cand};
+                      &ctx->maps, &ctx->map_off, &ctx->tpl, &ctx->cand, &ctx->peaks, &ctx->filt, &ctx->uncert};
     for (DevBuf *b : bufs) if (b->p && b->owned) cudaFree(b->p);
     if (ctx->pin) cudaFreeHost(ctx->pin);
     if (ctx->stage) cudaFreeHost(ctx->stage);
@@ -962,6 +1000,8 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
     if (rc) return rc;
     ctx->peaks_n = -1;
     ctx->peaks_of_table = false;
+    ctx->uncert_n = -1;
+    if ((rc = check_uncert(ctx, flags))) return rc;
     if (!pair && !ctx->have_pair) return fail(ctx, SID_ENOPAIR, "sid_set_pair has not been called");
     if (n < 0 || (n > 0 && (!c1 || !r1 || !c2fg || !r2fg || !border)) || !angles)
         return fail(ctx, SID_EINVAL, "null point array");
@@ -976,11 +1016,13 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
                                    pair->cols2, pair->pitch2)))
                 return rc;
             ctx->peaks_n = (flags & SID_PEAKS) ? 0 : -1;
+            ctx->uncert_n = (flags & SID_UNCERT) ? 0 : -1;
             return SID_OK;
         }
     }
     if (n == 0) {
         ctx->peaks_n = (flags & SID_PEAKS) ? 0 : -1;
+        ctx->uncert_n = (flags & SID_UNCERT) ? 0 : -1;
         return SID_OK;
     }
 
@@ -1192,14 +1234,16 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
     PmCall call{dp, dp + n, dp + 2 * n, dp + 3 * n, dp + 4 * n, d_angles, d_tab, rot_order, (double *)ctx->out.p,
                 (int *)ctx->status.p, maps_out, map_off, tpl_out, n, 0, 0};
     if (flags & SID_PEAKS) call.peaks = (double *)ctx->peaks.p;
-    // the larger borders (all points when the call is not split into classes), the class of pm_ws_kernel, the masked pass
-    PmPlan plans[3];
-    const bool masked = (flags & SID_MASKED) != 0;
-    const int nplans = two_class ? 2 : 1;
+    // the larger borders (all points when the call is not split into classes), the class of pm_ws_kernel, the masked pass,
+    // the uncertainty pass
+    PmPlan plans[4];
+    const bool masked = (flags & SID_MASKED) != 0, uncert = (flags & SID_UNCERT) != 0;
+    const int nplans = two_class ? 2 : 1, p_unc = nplans + (masked ? 1 : 0);
     if ((rc = plan_pm(ctx, img_size, n_angles, flags, max_border, two_class ? typ_big : typ_border, plans[0]))) return rc;
     if (two_class && (rc = plan_pm(ctx, img_size, n_angles, flags, small_max, typ_small, plans[1]))) return rc;
-    if (masked && (rc = plan_pm(ctx, img_size, n_angles, flags, max_border, typ_border, plans[nplans], true))) return rc;
-    if ((rc = reserve_call(ctx, call, plans, nplans + (masked ? 1 : 0)))) return rc;
+    if (masked && (rc = plan_pm(ctx, img_size, n_angles, flags, max_border, typ_border, plans[nplans], PASS_MASKED))) return rc;
+    if (uncert && (rc = plan_pm(ctx, img_size, n_angles, flags, max_border, typ_border, plans[p_unc], PASS_UNCERT))) return rc;
+    if ((rc = reserve_call(ctx, call, plans, p_unc + (uncert ? 1 : 0)))) return rc;
     const bool two_streams = pair && nbands > 1;
     if (two_streams) {
         if (!ctx->band_stream[0])
@@ -1228,6 +1272,8 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
     }
     // every band has arrived and every row has its status
     if (masked && (rc = enqueue_pm(ctx, call, plans[nplans], n, nullptr, ctx->stream, 0, 0, true))) return rc;
+    // ... and every row has its final table entry and status
+    if (uncert && (rc = enqueue_pm(ctx, call, plans[p_unc], n, nullptr, ctx->stream, 0, 0, true))) return rc;
     if (pair) ctx->have_pair = true;
     double *hout = (double *)((char *)ctx->pin + pts_bytes + ord_bytes);
     int *hst = (int *)((char *)hout + out_bytes);
@@ -1239,6 +1285,7 @@ int run_host(sid_ctx *ctx, const HostPair *pair, int64_t n, const double *c1, co
     if (out) memcpy(out, hout, out_bytes);
     if (status) memcpy(status, hst, st_bytes);
     if (flags & SID_PEAKS) { ctx->peaks_n = n; ctx->peaks_of_table = true; }
+    if (uncert) ctx->uncert_n = n;
     return SID_OK;
 }
 
@@ -1270,11 +1317,14 @@ int sid_run_device(sid_ctx *ctx, int64_t n, const double *d_c1, const double *d_
     if (rc) return rc;
     ctx->peaks_n = -1;
     ctx->peaks_of_table = false;
+    ctx->uncert_n = -1;
+    if ((rc = check_uncert(ctx, flags))) return rc;
     if (!ctx->have_pair) return fail(ctx, SID_ENOPAIR, "sid_set_pair has not been called");
     if (n < 0 || (n > 0 && (!d_c1 || !d_r1 || !d_c2fg || !d_r2fg || !d_border || !d_out)) || !angles)
         return fail(ctx, SID_EINVAL, "null point array");
     if (n == 0) {
         ctx->peaks_n = (flags & SID_PEAKS) ? 0 : -1;
+        ctx->uncert_n = (flags & SID_UNCERT) ? 0 : -1;
         return SID_OK;
     }
     CU(cudaSetDevice(ctx->device));
@@ -1294,8 +1344,8 @@ int sid_run_device(sid_ctx *ctx, int64_t n, const double *d_c1, const double *d_
         CU(cudaMemsetAsync(ctx->peaks.p, 0xff, b, ctx->stream));
         call.peaks = (double *)ctx->peaks.p;
     }
-    PmPlan plans[3];                 // [0], [1]: the border classes; the masked pass behind them
-    const bool masked = (flags & SID_MASKED) != 0;
+    PmPlan plans[4];                 // [0], [1]: the border classes; the masked and uncertainty passes behind them
+    const bool masked = (flags & SID_MASKED) != 0, uncert = (flags & SID_UNCERT) != 0;
     // border classes as in sid_run (see run_host): the indices are split on the device, one 8-byte read-back sizes the launches
     const int limit = n < 512 ? -1 : small_class_limit(ctx, img_size, n_angles, flags, max_border);
     if (limit >= 0) {
@@ -1313,22 +1363,30 @@ int sid_run_device(sid_ctx *ctx, int64_t n, const double *d_c1, const double *d_
         if (n_small >= 256 && n_big > 0) {
             if ((rc = plan_pm(ctx, img_size, n_angles, flags, max_border, max_border, plans[0]))) return rc;
             if ((rc = plan_pm(ctx, img_size, n_angles, flags, limit, limit, plans[1]))) return rc;
-            if (masked && (rc = plan_pm(ctx, img_size, n_angles, flags, max_border, max_border, plans[2], true))) return rc;
-            if ((rc = reserve_call(ctx, call, plans, masked ? 3 : 2))) return rc;
+            const int p_unc = masked ? 3 : 2;
+            if (masked && (rc = plan_pm(ctx, img_size, n_angles, flags, max_border, max_border, plans[2], PASS_MASKED))) return rc;
+            if (uncert && (rc = plan_pm(ctx, img_size, n_angles, flags, max_border, max_border, plans[p_unc], PASS_UNCERT))) return rc;
+            if ((rc = reserve_call(ctx, call, plans, p_unc + (uncert ? 1 : 0)))) return rc;
             if ((rc = enqueue_pm(ctx, call, plans[0], n_big, d_big, ctx->stream, 0, 0, false))) return rc;
             if ((rc = enqueue_pm(ctx, call, plans[1], n_small, d_small, ctx->stream, 0, n_big, true))) return rc;
             if (masked && (rc = enqueue_pm(ctx, call, plans[2], n, nullptr, ctx->stream, 0, 0, true))) return rc;
+            if (uncert && (rc = enqueue_pm(ctx, call, plans[p_unc], n, nullptr, ctx->stream, 0, 0, true))) return rc;
             if (flags & SID_PEAKS) ctx->peaks_n = n;
+            if (uncert) ctx->uncert_n = n;
             return SID_OK;
         }
         if (n_big == 0) max_border = limit;              // every point fits the pipeline kernel
     }
     if ((rc = plan_pm(ctx, img_size, n_angles, flags, max_border, max_border, plans[0]))) return rc;
-    if (masked && (rc = plan_pm(ctx, img_size, n_angles, flags, max_border, max_border, plans[1], true))) return rc;
-    if ((rc = reserve_call(ctx, call, plans, masked ? 2 : 1))) return rc;
+    const int p_unc = masked ? 2 : 1;
+    if (masked && (rc = plan_pm(ctx, img_size, n_angles, flags, max_border, max_border, plans[1], PASS_MASKED))) return rc;
+    if (uncert && (rc = plan_pm(ctx, img_size, n_angles, flags, max_border, max_border, plans[p_unc], PASS_UNCERT))) return rc;
+    if ((rc = reserve_call(ctx, call, plans, p_unc + (uncert ? 1 : 0)))) return rc;
     if ((rc = enqueue_pm(ctx, call, plans[0], n, nullptr, ctx->stream, 0, 0, false))) return rc;
     if (masked && (rc = enqueue_pm(ctx, call, plans[1], n, nullptr, ctx->stream, 0, 0, true))) return rc;
+    if (uncert && (rc = enqueue_pm(ctx, call, plans[p_unc], n, nullptr, ctx->stream, 0, 0, true))) return rc;
     if (flags & SID_PEAKS) ctx->peaks_n = n;
+    if (uncert) ctx->uncert_n = n;
     return SID_OK;
 }
 
@@ -1372,6 +1430,8 @@ int sid_run_maps(sid_ctx *ctx, int64_t n, const double *c1, const double *r1, co
     if (rc) return rc;
     ctx->peaks_n = -1;
     ctx->peaks_of_table = false;
+    ctx->uncert_n = -1;
+    if ((rc = check_uncert(ctx, flags))) return rc;
     if (!angles) return fail(ctx, SID_EINVAL, "null point array");
     if (n > 0x7fffffffLL) return fail(ctx, SID_EINVAL, "too many points");
     std::vector<long long> off;
@@ -1381,6 +1441,7 @@ int sid_run_maps(sid_ctx *ctx, int64_t n, const double *c1, const double *r1, co
     if (total > 0 && !maps) return fail(ctx, SID_EINVAL, "null maps buffer");
     if (n == 0) {
         ctx->peaks_n = (flags & SID_PEAKS) ? 0 : -1;
+        ctx->uncert_n = (flags & SID_UNCERT) ? 0 : -1;
         return SID_OK;
     }
     CU(cudaSetDevice(ctx->device));
@@ -1459,6 +1520,17 @@ int sid_pm_epilogue_affine(sid_ctx *ctx, int64_t n_valid, const int32_t *grid_in
     ctx->launches += n_valid ? 2 : 1;
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(out, d_out, b_out, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    return SID_OK;
+}
+
+int sid_get_uncertainty(sid_ctx *ctx, int64_t n, double *out) {
+    if (!ctx) return SID_EINVAL;
+    if (n < 0 || ctx->uncert_n != n) return fail(ctx, SID_EINVAL, "the previous sid_run* call did not set SID_UNCERT for n points");
+    if (n > 0 && !out) return fail(ctx, SID_EINVAL, "null output pointer");
+    if (n == 0) return SID_OK;
+    CU(cudaSetDevice(ctx->device));
+    CU(cudaMemcpyAsync(out, ctx->uncert.p, (size_t)n * 3 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
     return SID_OK;
 }
@@ -1921,6 +1993,7 @@ int sid_rotate_and_match(sid_ctx *ctx, const uint8_t *img1, int rows1, int cols1
     if (rc) return rc;
     if (!valid || !dc || !dr || !best_angle_idx || !best_r || !best_h) return fail(ctx, SID_EINVAL, "null output pointer");
     if (flags & SID_PEAKS) return fail(ctx, SID_EUNSUPPORTED, "SID_PEAKS is for the batched sid_run* calls");
+    if (flags & SID_UNCERT) return fail(ctx, SID_EUNSUPPORTED, "SID_UNCERT is for the batched sid_run* calls");
     const int s = img_size;
     if (!img1 || !image2 || H < s + 1 || W < s + 1)
         return fail(ctx, SID_EINVAL, "search window must exceed the template by at least one pixel in each axis");

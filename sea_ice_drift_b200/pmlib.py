@@ -144,11 +144,17 @@ def use_mcc_batch(c1, r1, c2fg, r2fg, border, img1, img2, img_size, alpha0, **kw
     ``peaks=True`` (extension): also return the three next-best peaks of every row's winning map (``SID_PEAKS``,
     include/sid_b200.h) as an (N, 3, 4) float64 array of c2, r2, r, h per peak, NaN where missing, appended to what the
     call returns: ``(table, peaks)`` or ``(table, maps, templates, peaks)``.  The table is unchanged.  Needs the
-    built-in matcher."""
+    built-in matcher.
+
+    ``uncertainty=True`` (extension, needs ``subpixel=True``): also return the covariance of every row's sub-pixel
+    offsets by correlation statistics (``SID_UNCERT``, include/sid_b200.h) as an (N, 3) float64 array of var_c, var_r,
+    cov_cr in image-2 pixels^2, NaN where undefined, appended last (after the peaks when both are asked for).  The
+    table is unchanged.  Needs the built-in matcher."""
     matcher = kwargs.get('template_matcher')
     return_maps = kwargs.get('return_maps', False)
     want_peaks = kwargs.get('peaks', False)
-    for option in ('return_maps', 'subpixel', 'masked', 'peaks'):
+    want_unc = kwargs.get('uncertainty', False)
+    for option in ('return_maps', 'subpixel', 'masked', 'peaks', 'uncertainty'):
         if kwargs.get(option) and not _is_builtin_matcher(matcher):
             raise ValueError("%s=True needs the built-in matcher (template_matcher None, match_template or "
                              "cv2.matchTemplate)" % option)
@@ -156,8 +162,8 @@ def use_mcc_batch(c1, r1, c2fg, r2fg, border, img1, img2, img_size, alpha0, **kw
         rows = [use_mcc(a, b, c, d, e, img1, img2, img_size, alpha0, **kwargs)
                 for a, b, c, d, e in zip(c1, r1, c2fg, r2fg, border)]
         return np.array(rows, dtype=np.float64).reshape(-1, 5)
-    ctx = _ctx(kwargs)
     flags = flags_from_options(kwargs) | (_lib.SID_PEAKS if want_peaks else 0)
+    ctx = _ctx(kwargs)
     args = (c1, r1, c2fg, r2fg, border, img_size, list(kwargs.get('angles', [-3, 0, 3])), alpha0,
             kwargs.get('rot_order', 0), flags, kwargs.get('mtype', TM_CCOEFF_NORMED))
     # The pair is uploaded on EVERY call (overlapped with the matching, so it costs ~1.5 ms per EW pair) unless
@@ -174,11 +180,15 @@ def use_mcc_batch(c1, r1, c2fg, r2fg, border, img1, img2, img_size, alpha0, **kw
     else:
         out = ctx.run_pair(img1, img2, *args)
         ctx._pair_key = (np.shape(img1), np.shape(img2))
-    if not want_peaks:
+    if not (want_peaks or want_unc):
         return out
-    if return_maps:
-        return out + (ctx.peaks(len(out[0])),)
-    return out, ctx.peaks(len(out))
+    extra = ()
+    n = len(out[0]) if return_maps else len(out)
+    if want_peaks:
+        extra += (ctx.peaks(n),)
+    if want_unc:
+        extra += (ctx.uncertainty(n),)
+    return (out if return_maps else (out,)) + extra
 
 
 def use_mcc(c1, r1, c2fg, r2fg, border, img1, img2, img_size, alpha0, **kwargs):
@@ -524,14 +534,25 @@ def pattern_matching(lon_pm1, lat_pm1, n1, c1, r1, n2, c2, r2,
     1.0 px, ``outlier_threshold`` default 2.0): replaced vectors come back in place, rejected ones as NaN.  Needs the
     built-in matcher and one GPU (no process group of more than one rank).  With ``return_flags=True`` an eighth grid
     (int32) holds every point's flag of :func:`filter_outliers`, and -4 where the point was not matched (outside the
-    image or its search window)."""
+    image or its search window).
+    ``uncertainty=True`` (extension, needs ``subpixel=True``): two more grids ``su``, ``sv``, appended last (after the
+    flags grid with ``return_flags=True``): the standard deviations of u and v, in their units, from the covariance of
+    every vector's sub-pixel offsets by correlation statistics (see :func:`use_mcc_batch`), propagated through the
+    Jacobian of image-2 pixel -> destination x/y at the vector's end point (the affine map's linear part on the device
+    path, central differences of ``n2.transform_points`` at +-0.5 px on the host path).  NaN where u is NaN, where the
+    peak lies on its map's edge, and, with ``outliers=True``, where a vector was replaced or rejected (its record
+    describes the primary peak).  Needs the built-in matcher and one GPU."""
     from .sharding import use_mcc_batch_sharded, _dist
     outliers = kwargs.get('outliers', False)
-    if outliers and not _is_builtin_matcher(kwargs.get('template_matcher')):
-        raise ValueError("outliers=True needs the built-in matcher (template_matcher None, match_template or "
-                         "cv2.matchTemplate)")
-    if outliers and _dist() is not None:
-        raise ValueError("outliers=True runs on one GPU: it is not supported under a process group of more than one rank")
+    uncertainty = kwargs.get('uncertainty', False)
+    for option in ('outliers', 'uncertainty'):
+        if kwargs.get(option) and not _is_builtin_matcher(kwargs.get('template_matcher')):
+            raise ValueError("%s=True needs the built-in matcher (template_matcher None, match_template or "
+                             "cv2.matchTemplate)" % option)
+        if kwargs.get(option) and _dist() is not None:
+            raise ValueError("%s=True runs on one GPU: it is not supported under a process group of more than one "
+                             "rank" % option)
+    flags_from_options(kwargs)                  # uncertainty without subpixel: ValueError before any device work
     eps, threshold = kwargs.get('outlier_eps', OUTLIER_EPS), kwargs.get('outlier_threshold', OUTLIER_THRESHOLD)
     return_flags = kwargs.get('return_flags', False)
     if return_flags and not outliers:
@@ -562,12 +583,29 @@ def pattern_matching(lon_pm1, lat_pm1, n1, c1, r1, n2, c2, r2,
     grid_shape = _grid_shape(dst_shape)
     flag_grid = np.full(dst_shape, -4, np.int32)
 
-    def finish(grids, flags=None):
+    def finish(grids, flags=None, sigma=None):
+        out = tuple(grids)
         if return_flags:
             if flags is not None:
                 flag_grid.ravel()[np.flatnonzero(gpi)] = flags
-            return tuple(grids) + (flag_grid,)
-        return tuple(grids)
+            out += (flag_grid,)
+        if uncertainty:
+            if sigma is None:
+                sigma = (np.full(dst_shape, np.nan), np.full(dst_shape, np.nan))
+            out += tuple(sigma)
+        return out
+
+    def sigma_grids(unc, jac, flags):
+        """su, sv grids from the (N, 3) records and the (N, 2, 2) Jacobians pixel -> x/y of the valid points"""
+        vc, vr, cv = unc[:, 0], unc[:, 1], unc[:, 2]
+        sig = []
+        for k in range(2):
+            j0, j1 = jac[:, k, 0], jac[:, k, 1]
+            s = np.sqrt(j0 * j0 * vc + 2.0 * j0 * j1 * cv + j1 * j1 * vr)
+            if flags is not None:
+                s[(flags != 0) & (flags != -2)] = np.nan    # replaced / rejected: the record is the primary peak's
+            sig.append(_fill_gpi(dst_shape, gpi, s))
+        return sig
 
     # Affine geolocation (an object exposing ``affine_maps(srs) -> (pixel->x/y, pixel->lon/lat)`` 2 x 3 matrices, e.g.
     # synthetic.ArrayDomain): the post-processing below (reference pmlib.py:462-497) runs on the device too, on the
@@ -579,21 +617,30 @@ def pattern_matching(lon_pm1, lat_pm1, n1, c1, r1, n2, c2, r2,
         xy, ll = affine(srs)
         ctx = _ctx(kwargs)
         flags = flags_from_options(kwargs) | (_lib.SID_PEAKS if outliers else 0)
+        n_valid = int(np.count_nonzero(gpi))
         ctx.run_pair(img1, img2, c1pm1i[gpi], r1pm1i[gpi], c2fg[gpi], r2fg[gpi], brd2[gpi], img_size,
                      list(kwargs.get('angles', [-3, 0, 3])), alpha0, kwargs.get('rot_order', 0), flags,
                      kwargs.get('mtype', TM_CCOEFF_NORMED), keep_on_device=True)
+        unc = ctx.uncertainty(n_valid) if uncertainty else None
         out_flags = None
         if outliers:
             out_flags = ctx.filter_outliers(grid_shape, gpi, c2pm1, r2pm1, eps=eps, threshold=threshold, in_place=True)[1]
         grids = ctx.pm_epilogue_affine(gpi, c2pm1, r2pm1, xy, ll)
+        sigma = None
+        if uncertainty:
+            jac = np.broadcast_to(np.asarray(xy, dtype=np.float64).reshape(2, 3)[:, :2], (n_valid, 2, 2))
+            sigma = sigma_grids(unc, jac, out_flags)
         print('\n', 'Pattern matching - OK! (%3.0f sec)' % (time.time() - t0))
-        return finish((grid.reshape(dst_shape) for grid in grids), out_flags)
+        return finish((grid.reshape(dst_shape) for grid in grids), out_flags, sigma)
     out_flags = None
-    if outliers:
-        results, peaks = use_mcc_batch(c1pm1i[gpi], r1pm1i[gpi], c2fg[gpi], r2fg[gpi], brd2[gpi],
-                                       img1, img2, img_size, alpha0, **dict(kwargs, peaks=True))
-        if len(results):
-            results, out_flags = _ctx(kwargs).filter_outliers(grid_shape, gpi, c2pm1, r2pm1, results, peaks, eps,
+    unc = None
+    if outliers or uncertainty:
+        extra = use_mcc_batch(c1pm1i[gpi], r1pm1i[gpi], c2fg[gpi], r2fg[gpi], brd2[gpi],
+                              img1, img2, img_size, alpha0, **dict(kwargs, peaks=outliers))
+        results = extra[0]
+        unc = extra[-1] if uncertainty else None
+        if outliers and len(results):
+            results, out_flags = _ctx(kwargs).filter_outliers(grid_shape, gpi, c2pm1, r2pm1, results, extra[1], eps,
                                                               threshold)
     else:
         results = use_mcc_batch_sharded(c1pm1i[gpi], r1pm1i[gpi], c2fg[gpi], r2fg[gpi], brd2[gpi],
@@ -615,4 +662,15 @@ def pattern_matching(lon_pm1, lat_pm1, n1, c1, r1, n2, c2, r2,
     a = _fill_gpi(dst_shape, gpi, results[:, 2])
     r = _fill_gpi(dst_shape, gpi, results[:, 3])
     h = _fill_gpi(dst_shape, gpi, results[:, 4])
-    return finish((u, v, a, r, h, _fill_gpi(dst_shape, gpi, lon_pm2), _fill_gpi(dst_shape, gpi, lat_pm2)), out_flags)
+    sigma = None
+    if uncertainty:
+        # Jacobian of pixel -> x/y at the end point (c2pm2, r2pm2) by central differences at +-0.5 px
+        jac = np.empty((len(results), 2, 2))
+        for k, (dc, dr) in enumerate(((0.5, 0.0), (0.0, 0.5))):
+            xp, yp = n2.transform_points(c2pm2 + dc, r2pm2 + dr, 0, nsr)
+            xm, ym = n2.transform_points(c2pm2 - dc, r2pm2 - dr, 0, nsr)
+            jac[:, 0, k] = np.asarray(xp) - np.asarray(xm)
+            jac[:, 1, k] = np.asarray(yp) - np.asarray(ym)
+        sigma = sigma_grids(unc, jac, out_flags)
+    return finish((u, v, a, r, h, _fill_gpi(dst_shape, gpi, lon_pm2), _fill_gpi(dst_shape, gpi, lat_pm2)), out_flags,
+                  sigma)

@@ -57,11 +57,17 @@ def _collective_device(dist, device=None):
     return torch.device('cuda', _lib.default_context(device).device)
 
 
+def _refuse_uncertainty(kwargs, name):
+    if kwargs.get('uncertainty'):
+        raise ValueError("uncertainty=True runs on one GPU: it is not supported by %s (use pmlib.use_mcc_batch)" % name)
+
+
 def use_mcc_batch_sharded(c1, r1, c2fg, r2fg, border, img1, img2, img_size, alpha0, compute=None, **kwargs):
     """``use_mcc_batch`` over all ranks of an initialised process group (falls back to
     a plain single-GPU call when there is none).  Every rank passes the same inputs
     and receives the full table.  ``compute`` is the per-shard function (the GPU
     batch by default; the CPU tests inject a stand-in)."""
+    _refuse_uncertainty(kwargs, 'use_mcc_batch_sharded')
     if compute is None:
         from .pmlib import use_mcc_batch as compute
     dist = _dist()
@@ -165,6 +171,7 @@ def use_mcc_batch_split(c1, r1, c2fg, r2fg, border, img1, img2, img_size, alpha0
     stream (slab copies, collectives, kernels), so the only host synchronisation is the final read-back.  Every rank
     passes the same arguments.  Falls back to :func:`use_mcc_batch_sharded` (each rank uploads the whole pair)
     without NCCL."""
+    _refuse_uncertainty(kwargs, 'use_mcc_batch_split')
     dist = _dist()
     n = len(c1)
     if dist is None or dist.get_backend() != 'nccl' or n == 0:
@@ -233,6 +240,7 @@ def use_mcc_series(pairs, img_size, alpha0=0.0, n_contexts=1, compute=None, gath
     ``Context.run_pair`` by default; the CPU tests inject a stand-in)."""
     import queue
     import threading
+    _refuse_uncertainty(kwargs, 'use_mcc_series')
     dist = _dist()
     rank, world = (dist.get_rank(), dist.get_world_size()) if dist is not None else (0, 1)
     mine = shard_pairs(len(pairs), world, rank)
